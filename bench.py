@@ -2,6 +2,7 @@
 """bench.py -- descriptor pairs/sec and match wall-time of the keypoint-matching hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c4|c3|c2|c1|dense]
+                    [--dump-outputs DIR]
 
 A step = one pass of the hot path (match.cpp:638-652: every image pair of a group through ComputeMatches)
 over ONE synthetic keypoint group.  Default workload: BASELINE.json configs[3], the configuration the
@@ -351,6 +352,25 @@ def producer_line(device, size=256, steps=5, warmup=3, points=20000):
     return out
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, lists):
+    """The match lists of the last timed step, as fm_match returns them: counts.npy [image pairs] and pairs.npy
+    [matches, 2] ((first, second) keypoint indices, image pairs in (i, j) order, i < j), float64.  Above DUMP_BYTES
+    pairs.npy holds a fixed seeded sample of the rows, whose indices are in pairs_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    counts = np.array([m.shape[0] for m in lists], np.float64)
+    pairs = np.concatenate([np.zeros((0, 2), np.uint32)] + list(lists)).astype(np.float64)
+    np.save(os.path.join(out_dir, "counts.npy"), counts)
+    cap = (DUMP_BYTES - counts.nbytes) // 24  # 16 bytes per sampled row + 8 for its index
+    if pairs.shape[0] > cap:
+        rows = np.sort(np.random.default_rng(0).choice(pairs.shape[0], cap, replace=False))
+        np.save(os.path.join(out_dir, "pairs_rows.npy"), rows.astype(np.float64))
+        pairs = pairs[rows]
+    np.save(os.path.join(out_dir, "pairs.npy"), pairs)
+
+
 def bench_ours(args):
     import torch
     import torch.distributed as dist
@@ -497,13 +517,15 @@ def bench_ours(args):
         def __exit__(self, *a):
             host_ms[self.name] += (time.perf_counter() - self.t) * 1e3
 
-    def finish_resident(res):
+    def finish_resident(res, keep=False):
         with phase("wait_kernels"):
             res.wait()  # this step's kernels are done; the next step's are already queued behind them
         if world > 1:
             with phase("gather"):
                 hand_off(res, to_host=False)
         retired.append((res.stats(), int(res.total)))
+        if keep:
+            return res
         res.free()
 
     def timed_resident(steps, warmup):
@@ -526,7 +548,7 @@ def bench_ours(args):
             if prev is not None:
                 finish_resident(prev)
             prev = res
-        finish_resident(prev)
+        last = finish_resident(prev, keep=bool(args.dump_outputs))  # with --dump-outputs: freed once it is written
         stream.wait_stream(comm)
         e1.record(stream)
         barrier()
@@ -534,11 +556,20 @@ def bench_ours(args):
         t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        return float(t.item()), t0, t1
+        return float(t.item()), t0, t1, last
 
     sampler = ClockSampler(local) if rank == 0 else None
-    ms_res, t0, t1 = timed_resident(args.steps, args.warmup)
+    ms_res, t0, t1, last = timed_resident(args.steps, args.warmup)
     clocks = sampler.stop(t0, t1) if sampler else None
+    if args.dump_outputs:
+        cptr, pptr = last.device_pointers()
+        counts = fdist.as_torch_u32(cptr, last.n_pairs, dev)
+        pairs = fdist.as_torch_u32(pptr, 2 * int(last.total), dev)
+        got = fdist.gather_match_lists(counts, pairs, 0) if world > 1 else ([counts], [pairs])
+        torch.cuda.synchronize()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, fdist.assemble(shards, *got, len(pf_all)))
+        last.free()
     stats = [o[0] for o in retired]
     matches_rank = retired[-1][1]
     res_host_ms = {k: round(v / args.steps, 4) for k, v in host_ms.items()}
@@ -714,6 +745,7 @@ def main():
     ap.add_argument("--no-wall-gz", action="store_true")
     ap.add_argument("--debug-opt", action="append", default=[], metavar="NAME=VALUE",
                     help="kernel-study switch (include/frogmatch_debug.h), e.g. variant=1; not for reported numbers")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the match lists of the last timed step to DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":

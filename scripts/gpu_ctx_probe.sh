@@ -3,6 +3,7 @@
 mkdir -p gpurun_out
 N=${1:-2}
 P=scripts/probe/ctx_probe
+[ -x $P ] || nvcc -gencode arch=compute_100a,code=sm_100a -O2 -std=c++17 -o $P $P.cu -lcuda || exit 1
 nproc; nvidia-smi --query-gpu=persistence_mode --format=csv,noheader | head -1
 {
 echo "== single process, one device (x3)"; for i in 1 2 3; do CUDA_VISIBLE_DEVICES=0 $P -tag single; done

@@ -2,7 +2,9 @@
 written by the verbatim reference build, the verbatim build itself where its .so travelled, and the numpy
 restatement.  Integer work (cast, integral volume, flags, keypoint order) and FP32 / FP64 arithmetic replayed op for
 op (responses, descriptors) are compared BIT FOR BIT; the sub-voxel interpolation (OpenCV SVD in the reference, absent
-here) within 1 float ulp with the number of differing values reported (0 on every case so far)."""
+here) within 1 float ulp with the number of differing values reported (0 on every case so far).  The volumes no
+fixture holds are compared with the verbatim build where oracle/_ref is built, else with its outputs as recorded in
+tests/golden/ref."""
 import json
 import os
 import subprocess
@@ -12,9 +14,10 @@ import numpy as np
 import pytest
 
 from conftest import ROOT
-from frog_b200 import build, surf, synth
+from frog_b200 import build, surf
 
 sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import make_ref_golden as rg  # noqa: E402
 import make_surf_golden as mg  # noqa: E402
 from oracle import surf_numpy as sn, surf_oracle as so  # noqa: E402
 
@@ -117,34 +120,35 @@ def test_voxel_types_and_device_pointer(producer):
     assert np.array_equal(producer.integral(), sn.integral(sn.cast_shift(wide)))
 
 
-@pytest.mark.skipif(not so.available(), reason="oracle/_ref/libsurf_ref.so did not travel")
+def reference_surf(name, vol, n_points):
+    """(hashes, keypoint arrays) of the verbatim build on `vol`: computed where oracle/_ref is built, else as recorded
+    from it (tests/golden/ref, make_ref_golden.py)."""
+    return rg.surf_outputs(True, vol, n_points) if so.available() else rg.load(name)
+
+
 def test_fresh_volume_against_the_reference_build(producer):
-    """A volume no fixture holds (four octaves: 400 voxels wide) straight against the reference's compiled code."""
-    vol = synth.make_volume((100, 120, 400), 17, blobs_per_mvox=2500.0)
-    vol = np.pad(vol, ((150, 150), (140, 140), (0, 0)), mode="reflect")  # 400 x 400 x 400
-    ref = so.RefSurf(vol)
-    rx, rlap, rdesc = ref.update(threshold=0.0, number_of_points=3000)
+    """A volume no fixture holds (four octaves: 400 voxels wide) against the reference's compiled code."""
+    vol = rg.fresh_volume()
+    want, ref = reference_surf("surf_fresh", vol, 3000)
     p = producer
     p.set_volume(vol)
-    assert np.array_equal(p.integral(), ref.integral_volume())
+    assert mg.sha(p.integral()) == want["integral"]
     n = p.detect(0.0)
     assert p.stats()["n_layers"] == 10
-    gl, rl = p.layers(), ref.response_layers(0.0)
-    assert mg.layer_hashes(gl) == mg.layer_hashes(rl)
-    det, det_lap = ref.detect(0.0)
-    assert n == len(det)
+    assert mg.layer_hashes(p.layers()) == want["layers"]
+    assert n == want["n_detected"]
     pts, _ = p.points(with_descriptors=False)
-    differing = assert_points_close(pts_matrix(pts), det)
+    differing = assert_points_close(pts_matrix(pts), ref["det_xyzsr"])
     p.select(3000)
     p.describe(0, 5, True)
     pts, desc = p.points()
-    differing += assert_points_close(pts_matrix(pts), rx)
-    assert len(pts) == 3000 and np.array_equal(pts["laplacian"], rlap)
+    differing += assert_points_close(pts_matrix(pts), ref["xyzsr"])
+    assert len(pts) == 3000 and np.array_equal(pts["laplacian"], ref["lap"])
     if differing == 0:
-        assert np.array_equal(bits(desc), bits(rdesc))
-    p.set_points(rx[:, :4])
+        assert mg.sha(desc) == want["desc"]
+    p.set_points(ref["xyzsr"][:, :4])
     p.describe(0, 5, True)
-    assert np.array_equal(bits(p.points()[1]), bits(rdesc))
+    assert mg.sha(p.points()[1]) == want["desc"]
 
 
 def test_cli_writes_the_reference_files(built, tmp_path):
@@ -168,35 +172,43 @@ def test_cli_writes_the_reference_files(built, tmp_path):
     assert open(base + "9.csv.gz", "rb").read() == open(os.path.join(GOLD, "small_points_l9p4.csv.gz"), "rb").read()
 
 
-@pytest.mark.skipif(not so.available() or not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "match_ref")),
-                    reason="reference builds did not travel")
 def test_producer_feeds_matcher_like_run_sh(built, tmp_path):
     """run.sh:80-93 with both stages on the GPU: surf3d per volume -> list file -> match, against the same chain run
-    by the reference's compiled code (its producer writes the .csv.gz files, its matcher pairs them): pairs.bin cmp."""
-    vols = [synth.make_volume((136, 128, 144), 30, blobs_per_mvox=3000.0)]
-    vols.append(np.roll(vols[0], (3, -2, 4), (0, 1, 2)) + np.random.default_rng(1).integers(-6, 7, vols[0].shape).astype(np.int16))
-    vols.append(synth.make_volume((136, 128, 144), 31, blobs_per_mvox=3000.0))
+    by the reference's compiled code (its producer writes the .csv.gz files, its matcher pairs them): pairs.bin cmp.
+    Where oracle/_ref is not built, against that chain's files as recorded (tests/golden/ref)."""
+    import hashlib
+    live = so.available() and os.path.exists(os.path.join(ROOT, "oracle", "_ref", "match_ref"))
+    want = rg.load("surf_run_sh")[0]
+    vols = rg.run_sh_volumes()
     gdir, rdir = tmp_path / "gpu", tmp_path / "ref"
     gdir.mkdir()
     rdir.mkdir()
     for i, v in enumerate(vols):
         mha = str(tmp_path / f"v{i}.mha")
-        surf.write_metaimage(mha, v, (0.75, 0.75, 0.75), (-50.0, -40.0, 10.0 * i))
+        surf.write_metaimage(mha, v, rg.RUN_SH_SPACING, rg.RUN_SH_ORIGIN(i))
         r = subprocess.run([build.SURF_BIN, mha, "-o", str(gdir / f"points{i}"), "-t", "0", "-n", "20000"], capture_output=True, text=True)
         assert r.returncode == 0, r.stderr
-        ref = so.RefSurf(v, (0.75, 0.75, 0.75), (-50.0, -40.0, 10.0 * i))
-        ref.update(threshold=0.0, number_of_points=20000)
-        ref.write(str(rdir / f"points{i}.csv.gz"), "csv.gz")
-        assert open(gdir / f"points{i}.csv.gz", "rb").read() == open(rdir / f"points{i}.csv.gz", "rb").read()
+        got = open(gdir / f"points{i}.csv.gz", "rb").read()
+        if live:
+            ref = so.RefSurf(v, rg.RUN_SH_SPACING, rg.RUN_SH_ORIGIN(i))
+            ref.update(threshold=0.0, number_of_points=20000)
+            ref.write(str(rdir / f"points{i}.csv.gz"), "csv.gz")
+            assert got == open(rdir / f"points{i}.csv.gz", "rb").read()
+        else:
+            assert hashlib.sha256(got).hexdigest() == want["files"][i]
     for d in (gdir, rdir):
         open(d / "points.txt", "w").write("".join(f"{d}/points{i}.csv.gz\n" for i in range(len(vols))))
     r = subprocess.run([build.BIN, str(gdir / "points.txt"), "-o", str(gdir / "pairs.bin"), "-d", "1"], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
-    from oracle import oracle
-    rr = oracle.run_ref_binary([str(rdir / "points.txt"), "-o", str(rdir / "pairs.bin"), "-d", "1"])
-    assert rr.returncode == 0
-    got, want = open(gdir / "pairs.bin", "rb").read(), open(rdir / "pairs.bin", "rb").read()
-    assert len(got) > 1000 and got == want
+    got = open(gdir / "pairs.bin", "rb").read()
+    if live:
+        from oracle import oracle
+        rr = oracle.run_ref_binary([str(rdir / "points.txt"), "-o", str(rdir / "pairs.bin"), "-d", "1"])
+        assert rr.returncode == 0
+        assert got == open(rdir / "pairs.bin", "rb").read()
+    else:
+        assert rg.pairs_digest(got) == want["pairs"]
+    assert len(got) > 1000
 
 
 def test_cli_point_file(built, tmp_path):
@@ -218,26 +230,23 @@ def test_cli_point_file(built, tmp_path):
     assert open(base + "30.csv.gz", "rb").read() == open(os.path.join(GOLD, "pfile_points_n30.csv.gz"), "rb").read()
 
 
-@pytest.mark.skipif(not so.available(), reason="oracle/_ref/libsurf_ref.so did not travel")
 def test_odd_dimensions_against_the_reference_build(producer):
     """Odd sizes on every axis (131 x 103 x 117 voxels, z y x): the parity-split layout's half rows differ in length,
     the layers drop the last voxel of each axis."""
-    vol = synth.make_volume((131, 103, 117), 5)
-    ref = so.RefSurf(vol)
-    rx, rlap, rdesc = ref.update(threshold=0.0, number_of_points=20000)
+    vol = rg.odd_volume()
+    want, ref = reference_surf("surf_odd", vol, 20000)
     p = producer
     p.set_volume(vol)
-    assert np.array_equal(p.integral(), ref.integral_volume())
+    assert mg.sha(p.integral()) == want["integral"]
     n = p.detect(0.0)
-    assert mg.layer_hashes(p.layers()) == mg.layer_hashes(ref.response_layers(0.0))
-    det, det_lap = ref.detect(0.0)
-    assert n == len(det) and n > 20
+    assert mg.layer_hashes(p.layers()) == want["layers"]
+    assert n == want["n_detected"] and n > 20
     pts, _ = p.points(with_descriptors=False)
-    differing = assert_points_close(pts_matrix(pts), det)
+    differing = assert_points_close(pts_matrix(pts), ref["det_xyzsr"])
     p.select(20000)
     p.describe(0, 5, True)
     pts, desc = p.points()
-    differing += assert_points_close(pts_matrix(pts), rx)
-    assert np.array_equal(pts["laplacian"], rlap)
+    differing += assert_points_close(pts_matrix(pts), ref["xyzsr"])
+    assert np.array_equal(pts["laplacian"], ref["lap"])
     if differing == 0:
-        assert np.array_equal(bits(desc), bits(rdesc))
+        assert mg.sha(desc) == want["desc"]

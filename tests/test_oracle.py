@@ -2,6 +2,7 @@
 files written by the unmodified reference binary pin all of them (oracle parity = PINNED)."""
 import json
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -9,6 +10,9 @@ import pytest
 import helpers
 from frog_b200 import pairsbin, synth
 from oracle import oracle as O
+
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+import make_ref_golden as rg  # noqa: E402
 
 CASES = sorted(json.load(open(os.path.join(os.path.dirname(__file__), "golden", "manifest.json"))).items())
 
@@ -86,17 +90,13 @@ def test_known_answers(libs):
 
 def test_match_all_port_equals_reference(libs):
     """`-all` (matchAll, match.cpp:295-300): the C port against the verbatim reference in-process, including the
-    stale `match` carried across rows and the -sym orientation."""
+    stale `match` carried across rows and the -sym orientation.  Where oracle/_ref is not built, the reference's lists
+    as recorded in tests/golden/ref."""
     port, ref = libs
-    if ref is None:
-        pytest.skip("oracle/_ref/libmatch_ref.so not built here")
-    from frog_b200 import synth
-    for seed in range(3):
-        a, b = synth.make("bank", 300, seed), synth.make("bank", 260, seed + 5)
-        A, B = (a.desc, a.scale, a.lap), (b.desc, b.scale, b.lap)
-        for thr in (0.22, 0.6, 5.0):
-            for sym in (False, True):
-                assert np.array_equal(ref.compute_matches_all(A, B, thr, sym), port.compute_matches_all(A, B, thr, sym))
+    recorded = rg.load("match_all")[1]
+    for key, A, B, thr, sym in rg.match_all_cases():
+        want = ref.compute_matches_all(A, B, thr, sym) if ref is not None else recorded[key]
+        assert np.array_equal(want, port.compute_matches_all(A, B, thr, sym)), key
     # known answer: rows 0 and 1 both lie within the threshold of column 1 only; column 0 is far.  Row 0 meets the far
     # column first (match = 0), row 1 has its own far column 0 as well -> both emit (0, row); a third row that sees NO
     # far column before its near one inherits the previous row's value.
