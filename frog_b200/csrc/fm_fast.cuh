@@ -4,6 +4,7 @@
 
 #include "fm_host.h"
 #include "fm_prep.cuh"
+#include "fm_reject.cuh"
 #include "fm_rescore.cuh"
 #include "fm_score.cuh"
 
@@ -157,11 +158,12 @@ inline cudaError_t fast_match_batch(fm_ctx* c, const FastBatchArgs& a) {
       return cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     };
     if ((e = prep(score_kernel<false, 0, 0>)) != cudaSuccess) return e;
-    if ((e = prep(score_kernel<false, 0, 1>)) != cudaSuccess) return e;
     if ((e = prep(score_kernel<false, 0, 2>)) != cudaSuccess) return e;
     if ((e = prep(score_kernel<false, 1, 0>)) != cudaSuccess) return e;
     if ((e = prep(score_kernel<false, 2, 0>)) != cudaSuccess) return e;
     if ((e = prep(score_kernel<true, 0, 0>)) != cudaSuccess) return e;
+    // the reject pass: one CTA per SM
+    if ((e = cudaFuncSetAttribute(reject_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRjSmemBytes)) != cudaSuccess) return e;
     c->score_attr_set = true;
   }
   bool two_phase_ran = false;
@@ -184,9 +186,10 @@ inline cudaError_t fast_match_batch(fm_ctx* c, const FastBatchArgs& a) {
       uint32_t* surv_off = surv_count + a.n_tasks;
       uint32_t* surv_rows = surv_off + a.n_tasks + 1;
       if ((e = cudaMemsetAsync(surv_count, 0, (size_t)a.n_tasks * sizeof(uint32_t), c->stream)) != cudaSuccess) return e;
-      score_kernel<false, 0, 1><<<a.units, kScoreThreads, kScoreSmemBytes, c->stream>>>(
-          a.images, a.tasks, a.unit_off, a.n_tasks, a.segs, c->d_bands.as<uint2>(), c->d_cands.as<Cand>(),
-          &a.counters->scored_cols, nullptr, 0, 0, 0, a.thr, a.ratio, rowstat, surv_count, surv_rows);
+      // persistent: one CTA per SM walks the units
+      reject_kernel<<<std::min<uint32_t>(a.units, (uint32_t)c->sm_count), kRjThreads, kRjSmemBytes, c->stream>>>(
+          a.images, a.tasks, a.unit_off, a.n_tasks, a.units, c->d_bands.as<uint2>(), &a.counters->scored_cols, a.thr,
+          a.ratio, rowstat, surv_count, surv_rows);
       surv_plan_kernel<<<1, 1024, 0, c->stream>>>(surv_count, a.n_tasks, surv_off, cap_units, a.tasks, surv_rows, rowstat,
                                                   c->d_redo.as<uint2>(), &a.counters->rescore.redo_rows);
       score_kernel<false, 0, 2><<<cap_units, kScoreThreads, kScoreSmemBytes, c->stream>>>(

@@ -118,6 +118,26 @@ __device__ __forceinline__ void tmem_ld_wait(uint32_t (&r)[16]) {
                : "memory");
 }
 
+// 32 lanes x 32 consecutive 32-bit columns.
+__device__ __forceinline__ void tmem_ld32(uint32_t (&r)[32], uint32_t taddr) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
+      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
+        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
+        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
+      : "r"(taddr)
+      : "memory");
+}
+// Wait for this thread's outstanding tcgen05.ld into four 32-register arrays; each register is passed through an
+// empty asm after the wait so that no consumer can be scheduled above it.
+__device__ __forceinline__ void tmem_ld_wait(uint32_t (&a)[32], uint32_t (&b)[32], uint32_t (&c)[32], uint32_t (&d)[32]) {
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+  for (int i = 0; i < 32; i++) asm volatile("" : "+r"(a[i]), "+r"(b[i]), "+r"(c[i]), "+r"(d[i]));
+}
+
 // Shared-memory matrix descriptor for a K-major, SWIZZLE_128B operand tile whose rows are 128 B
 // (64 FP16): 8-row atoms 1024 B apart (SBO), LBO unused (=1), descriptor version 1 (sm_100),
 // layout type 2 = SWIZZLE_128B.  Field layout: cute::UMMA::SmemDescriptor.

@@ -1,0 +1,328 @@
+// fm_reject.cuh -- reject pass of two-phase scoring (fm_fast.cuh): for every row of a 256-row unit, the row's best
+// approximate score g1 and the second largest 16-column chunk maximum g2 over its gated-in columns, then the certified
+// rejection test (certified_reject, fm_score.cuh) and the survivor list the capture pass works on.
+//
+// One persistent CTA per SM walks units blockIdx.x, blockIdx.x + gridDim.x, ...  Per 256-column step the unit's two
+// row halves each take one tcgen05.mma M=128 x N=256 x K=16 chain (4 K-steps) into their own 256-column TMEM buffer.
+// Against the single pass's N=64 this reads the row operand once per 256 columns instead of once per 64: 12 KB of
+// shared-memory operand reads per 128 cycles of MMA math instead of 6 KB per 32, which is what kept the tensor pipe
+// below half its rate.  The accumulator shape (M=128, FP32, K=64 in four steps) is the single pass's, so every score,
+// and therefore g1, g2 and the set of rejected rows, is the same.
+//   warp 0      scheduler  : task lookup, the unit's 256 bands and its column-step range -> a 4-slot ring in shared
+//                            memory, so unit prologues (dependent global loads) run ahead of the pipeline
+//   warp 1      TMA        : the unit's two 16 KB row-operand tiles (double-buffered across units) and 32 KB column
+//                            steps into a 4-stage ring
+//   warp 2      MMA        : buffer h <- row half h, alternating, so one half's MMAs run while the other is drained
+//   warps 3..10 epilogue   : (TMEM lane quadrant = warp % 4) x (row half): one row per thread.  Each warp loads a
+//                            step's 256 columns in two rounds of 128, releases the buffer after the second load, and
+//                            reduces 32-column groups with 3-input max trees; masking is decided per group, warp-
+//                            uniformly.  (Eight warps, not sixteen: eleven warps leave 168 registers per thread for the
+//                            128-column rounds, nineteen would leave 96.)
+// Scores never leave the SM.
+#pragma once
+#include "fm_score.cuh"
+
+namespace fm {
+
+// N of one MMA: columns per step, 128 or 256 (FM_REJECT_COLS overrides it to time the other one).  TMEM holds
+// 512 / (2 N) accumulator stages of both row halves; the epilogue loads a stage in rounds of 128 columns.
+#ifndef FM_REJECT_COLS
+#define FM_REJECT_COLS 256
+#endif
+constexpr int kRjCols = FM_REJECT_COLS;
+static_assert(kRjCols == 128 || kRjCols == 256, "reject pass: N = 128 or 256");
+constexpr int kRjAccStages = 512 / (2 * kRjCols);
+constexpr int kRjRounds = kRjCols / 128;
+constexpr int kRjStepBytes = kRjCols * 128;  // one step of the column operand: N / 128 stored operand tiles
+constexpr int kRjStages = 4 * 256 / kRjCols; // 128 KB of column-operand ring
+constexpr int kRjSlots = 4;                  // units the scheduler warp may run ahead
+constexpr int kRjEpiWarps = 8;
+constexpr int kRjThreads = (3 + kRjEpiWarps) * 32;
+
+struct RjUnit {
+  const uint8_t* rowop;  // the unit's two row-operand tiles (row halves 0 and 1)
+  const uint8_t* colop;
+  const float* norm2;
+  uint32_t task, n_rows, row_off, s0;  // s0: sorted position of the unit's first row
+  uint32_t step0, n_steps;             // column steps [step0, step0 + n_steps) of kRjCols columns
+  uint32_t halves;                     // row halves holding rows of the image (1: the image ends in row half 0)
+  float eps;
+  uint32_t skip;                       // task takes the exact kernel: nothing to write
+};
+
+struct alignas(1024) RejectSmem {
+  uint8_t a[2][2][kOpTileBytes];        // [unit buffer][row half]
+  uint8_t b[kRjStages][kRjStepBytes];
+  uint2 band[kRjSlots][kUnitRows];      // the unit's bands, (0, 0) for rows past the image
+  RjUnit unit[kRjSlots];
+  uint64_t bar_afull[2], bar_aempty[2];
+  uint64_t bar_bfull[kRjStages], bar_bempty[kRjStages];
+  uint64_t bar_accfull[kRjAccStages][2], bar_accempty[kRjAccStages][2];  // [stage][row half]
+  uint64_t bar_ufull[kRjSlots], bar_uempty[kRjSlots];
+  uint32_t tmem_base;
+};
+constexpr size_t kRjSmemBytes = sizeof(RejectSmem) + 1024;
+
+// Maximum of 16 consecutive columns (index O of r); kMasked: columns outside [lo, lo + width) count as -inf.
+template <bool kMasked, int O>
+__device__ __forceinline__ float rj_chunk(const uint32_t (&r)[32], uint32_t col0, uint32_t lo, uint32_t width) {
+  float f[16];
+#pragma unroll
+  for (int e = 0; e < 16; e++) {
+    f[e] = __uint_as_float(r[O + e]);
+    if (kMasked) f[e] = ((col0 + e) - lo < width) ? f[e] : -INFINITY;
+  }
+  const float ga = max3(max3(f[0], f[1], f[2]), max3(f[3], f[4], f[5]), max3(f[6], f[7], f[8]));
+  const float gb = max3(max3(f[9], f[10], f[11]), max3(f[12], f[13], f[14]), f[15]);
+  return fmaxf(ga, gb);
+}
+
+struct RjWarpRange {
+  uint32_t cmin, cmax;  // columns some row of the warp accepts lie in [cmin, cmax)
+  uint32_t imin, imax;  // every row of the warp accepts [imin, imax)
+};
+
+// 32 columns starting at gc (a multiple of 32, so the two 16-column chunks are the single pass's chunks): fold both
+// chunk maxima into the row's top two (g1 >= g2).
+__device__ __forceinline__ void rj_group(const uint32_t (&r)[32], uint32_t gc, const RjWarpRange& w, uint32_t lo,
+                                         uint32_t width, float& g1, float& g2) {
+  if (gc >= w.cmax || gc + 32 <= w.cmin) return;  // warp-uniform: no row of the warp accepts these columns
+  float a, b;
+  if (gc >= w.imin && gc + 32 <= w.imax) {
+    a = rj_chunk<false, 0>(r, gc, lo, width);
+    b = rj_chunk<false, 16>(r, gc + 16, lo, width);
+  } else {
+    a = rj_chunk<true, 0>(r, gc, lo, width);
+    b = rj_chunk<true, 16>(r, gc + 16, lo, width);
+  }
+  const float hi = fmaxf(a, b), lw = fminf(a, b);
+  g2 = max3(g2, lw, fminf(g1, hi));
+  g1 = fmaxf(g1, hi);
+}
+
+// units = unit_off[n_tasks] (segs = 1).  scored_cols += (row, column) scores the tensor cores computed: 128 x kRjCols
+// per MMA chain issued, band-edge and past-the-band columns of a step included.  Writes rowstat[row] (1 = rejected) for every row of every fast task and
+// appends the sorted position of each surviving row to its task's survivor list (surv_count / surv_rows, any order).
+__global__ void __launch_bounds__(kRjThreads, 1)
+reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ tasks, const uint32_t* __restrict__ unit_off,
+              uint32_t n_tasks, uint32_t units, const uint2* __restrict__ bands, unsigned long long* __restrict__ scored_cols,
+              float thr, float ratio, uint8_t* __restrict__ rowstat, uint32_t* __restrict__ surv_count,
+              uint32_t* __restrict__ surv_rows) {
+  extern __shared__ uint8_t smem_raw[];
+  RejectSmem& sm = *reinterpret_cast<RejectSmem*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
+  const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+
+  if (warp == 2 && lane == 0) {
+    for (int i = 0; i < 2; i++) {
+      ptx::mbar_init(&sm.bar_afull[i], 1);
+      ptx::mbar_init(&sm.bar_aempty[i], 1);
+    }
+    for (int i = 0; i < kRjAccStages; i++)
+      for (int h = 0; h < 2; h++) {
+        ptx::mbar_init(&sm.bar_accfull[i][h], 1);
+        ptx::mbar_init(&sm.bar_accempty[i][h], kRjEpiWarps / 2);
+      }
+    for (int i = 0; i < kRjStages; i++) { ptx::mbar_init(&sm.bar_bfull[i], 1); ptx::mbar_init(&sm.bar_bempty[i], 1); }
+    for (int i = 0; i < kRjSlots; i++) {
+      ptx::mbar_init(&sm.bar_ufull[i], 32);                // every lane of the scheduler warp
+      ptx::mbar_init(&sm.bar_uempty[i], 2 + kRjEpiWarps);  // TMA thread, MMA thread, one arrival per epilogue warp
+    }
+    ptx::fence_mbar_init();
+  }
+  if (warp == 0) ptx::tmem_alloc<512>(&sm.tmem_base);
+  ptx::tc_fence_before();
+  __syncthreads();
+  ptx::tc_fence_after();
+  const uint32_t tmem = sm.tmem_base;
+
+  if (warp == 0) {
+    // ---- scheduler --------------------------------------------------------------------------------------------
+    uint32_t k = 0;
+    for (uint32_t unit = blockIdx.x; unit < units; unit += gridDim.x, k++) {
+      const uint32_t slot = k % kRjSlots;
+      if (k >= (uint32_t)kRjSlots) ptx::mbar_wait(&sm.bar_uempty[slot], (k / kRjSlots - 1) & 1);
+      const uint32_t t = find_segment_near(unit_off, n_tasks, unit, units);
+      const Task task = tasks[t];
+      const ImageDev A = images[task.col_img];
+      const ImageDev B = images[task.row_img];
+      const uint32_t s0 = (unit - unit_off[t]) * kUnitRows;
+      const bool skip = (task.flags & kTaskExact) != 0;
+      uint32_t cmin = 0xFFFFFFFFu, cmax = 0u;
+#pragma unroll
+      for (int j = 0; j < kUnitRows / 32; j++) {
+        const uint32_t r = j * 32 + lane, s = s0 + r;
+        uint2 bd = make_uint2(0u, 0u);
+        if (!skip && s < B.n) bd = bands[task.row_off + s];
+        if (bd.y > bd.x) { cmin = min(cmin, bd.x); cmax = max(cmax, bd.y); }
+        sm.band[slot][r] = bd;
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        cmin = min(cmin, __shfl_xor_sync(0xffffffffu, cmin, o));
+        cmax = max(cmax, __shfl_xor_sync(0xffffffffu, cmax, o));
+      }
+      if (lane == 0) {
+        RjUnit u;
+        u.rowop = reinterpret_cast<const uint8_t*>(B.rowop) + (size_t)s0 / 128 * kOpTileBytes;
+        u.colop = reinterpret_cast<const uint8_t*>(A.colop);
+        u.norm2 = B.norm2_sorted;
+        u.task = t;
+        u.n_rows = B.n;
+        u.row_off = task.row_off;
+        u.s0 = s0;
+        u.step0 = cmax > cmin ? cmin / kRjCols : 0u;
+        u.n_steps = cmax > cmin ? (cmax + kRjCols - 1) / kRjCols - u.step0 : 0u;
+        u.eps = skip ? 0.f : task_eps(A.meta, B.meta);
+        u.skip = skip ? 1u : 0u;
+        u.halves = B.n - s0 > 128 ? 2u : 1u;
+        sm.unit[slot] = u;
+      }
+      ptx::mbar_arrive(&sm.bar_ufull[slot]);
+    }
+  } else if (warp == 1) {
+    // ---- TMA ----------------------------------------------------------------------------------------------------
+    if (lane == 0) {
+      uint32_t k = 0, a_use = 0, bq = 0;
+      for (uint32_t unit = blockIdx.x; unit < units; unit += gridDim.x, k++) {
+        const uint32_t slot = k % kRjSlots;
+        ptx::mbar_wait(&sm.bar_ufull[slot], (k / kRjSlots) & 1);
+        const RjUnit& us = sm.unit[slot];
+        const uint8_t* rowop = us.rowop;
+        const uint8_t* colop = us.colop;
+        const uint32_t step0 = us.step0, n_steps = us.n_steps;
+        ptx::mbar_arrive(&sm.bar_uempty[slot]);
+        if (n_steps == 0) continue;
+        const uint32_t ab = a_use & 1;
+        if (a_use >= 2) ptx::mbar_wait(&sm.bar_aempty[ab], (a_use / 2 - 1) & 1);
+        a_use++;
+        ptx::mbar_expect_tx(&sm.bar_afull[ab], 2 * kOpTileBytes);
+        ptx::bulk_g2s(sm.a[ab][0], rowop, kOpTileBytes, &sm.bar_afull[ab]);
+        ptx::bulk_g2s(sm.a[ab][1], rowop + kOpTileBytes, kOpTileBytes, &sm.bar_afull[ab]);
+        for (uint32_t i = 0; i < n_steps; i++, bq++) {
+          const uint32_t stg = bq % kRjStages, use = bq / kRjStages;
+          if (use > 0) ptx::mbar_wait(&sm.bar_bempty[stg], (use - 1) & 1);
+          const uint8_t* src = colop + (size_t)(step0 + i) * kRjStepBytes;  // n_pad is a multiple of 256: in bounds
+          ptx::mbar_expect_tx(&sm.bar_bfull[stg], kRjStepBytes);
+          ptx::bulk_g2s(sm.b[stg], src, kRjStepBytes / 2, &sm.bar_bfull[stg]);
+          ptx::bulk_g2s(sm.b[stg] + kRjStepBytes / 2, src + kRjStepBytes / 2, kRjStepBytes / 2, &sm.bar_bfull[stg]);
+        }
+      }
+    }
+  } else if (warp == 2) {
+    // ---- MMA ----------------------------------------------------------------------------------------------------
+    if (lane == 0) {
+      constexpr uint32_t idesc = ptx::umma_idesc_f16_f32(128, kRjCols);
+      uint32_t k = 0, a_use = 0, bq = 0, g = 0;
+      unsigned long long issued = 0;
+      for (uint32_t unit = blockIdx.x; unit < units; unit += gridDim.x, k++) {
+        const uint32_t slot = k % kRjSlots;
+        ptx::mbar_wait(&sm.bar_ufull[slot], (k / kRjSlots) & 1);
+        const uint32_t n_steps = sm.unit[slot].n_steps, halves = sm.unit[slot].halves;
+        ptx::mbar_arrive(&sm.bar_uempty[slot]);
+        if (n_steps == 0) continue;
+        const uint32_t ab = a_use & 1;
+        ptx::mbar_wait(&sm.bar_afull[ab], (a_use / 2) & 1);
+        a_use++;
+        const uint64_t adesc[2] = {ptx::umma_desc_sw128(ptx::smem_u32(sm.a[ab][0])), ptx::umma_desc_sw128(ptx::smem_u32(sm.a[ab][1]))};
+        for (uint32_t i = 0; i < n_steps; i++, bq++, g++) {
+          const uint32_t stg = bq % kRjStages;
+          ptx::mbar_wait(&sm.bar_bfull[stg], (bq / kRjStages) & 1);
+          const uint64_t bdesc = ptx::umma_desc_sw128(ptx::smem_u32(sm.b[stg]));
+#pragma unroll
+          for (int h = 0; h < 2; h++) {
+            const uint32_t as = g % kRjAccStages, use = g / kRjAccStages;
+            if (use > 0) ptx::mbar_wait(&sm.bar_accempty[as][h], (use - 1) & 1);
+            ptx::tc_fence_after();
+            if ((uint32_t)h < halves) {  // (a half without rows is still handed to its epilogue warps, unscored)
+#pragma unroll
+              for (int kk = 0; kk < kKPad / 16; kk++)  // +32 B per K step inside the 128 B swizzle row
+                ptx::mma_f16_ss(tmem + (as * 2 + h) * kRjCols, adesc[h] + 2 * kk, bdesc + 2 * kk, idesc, kk > 0);
+              issued += 128 * kRjCols;
+            }
+            ptx::mma_commit(&sm.bar_accfull[as][h]);
+          }
+          ptx::mma_commit(&sm.bar_bempty[stg]);
+        }
+        ptx::mma_commit(&sm.bar_aempty[ab]);
+      }
+      if (scored_cols != nullptr) atomicAdd(scored_cols, issued);
+    }
+  } else {
+    // ---- epilogue -----------------------------------------------------------------------------------------------
+    const uint32_t h = (warp - 3) >> 2, q = warp & 3;  // row half, TMEM lane quadrant
+    const uint32_t row = h * 128 + q * 32 + lane;
+    uint32_t taddr = tmem + ((q * 32) << 16) + h * kRjCols;
+    asm volatile("" : "+r"(taddr));
+    uint32_t g = 0, k = 0;
+    for (uint32_t unit = blockIdx.x; unit < units; unit += gridDim.x, k++) {
+      const uint32_t slot = k % kRjSlots;
+      ptx::mbar_wait(&sm.bar_ufull[slot], (k / kRjSlots) & 1);
+      // (the slot is released at unit end, after the rejection tail has read the rest of it)
+      const RjUnit& us = sm.unit[slot];
+      const uint32_t step0 = us.step0, n_steps = us.n_steps;
+      const uint2 bd = sm.band[slot][row];
+      const uint32_t s = us.s0 + row;
+      const bool valid = bd.y > bd.x;
+      const uint32_t lo = bd.x, width = bd.y - bd.x;
+      const float na = valid ? us.norm2[s] : 0.f;  // used at unit end (valid: s is a row of the image)
+      RjWarpRange w{valid ? lo : 0xFFFFFFFFu, valid ? bd.y : 0u, valid ? lo : 0u, valid ? bd.y : 0xFFFFFFFFu};
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        w.cmin = min(w.cmin, __shfl_xor_sync(0xffffffffu, w.cmin, o));
+        w.cmax = max(w.cmax, __shfl_xor_sync(0xffffffffu, w.cmax, o));
+        w.imin = max(w.imin, __shfl_xor_sync(0xffffffffu, w.imin, o));
+        w.imax = min(w.imax, __shfl_xor_sync(0xffffffffu, w.imax, o));
+      }
+      float g1 = -INFINITY, g2 = -INFINITY;
+      for (uint32_t i = 0; i < n_steps; i++, g++) {
+        const uint32_t as = g % kRjAccStages;
+        const uint32_t tstage = taddr + as * 2 * kRjCols;
+        ptx::mbar_wait(&sm.bar_accfull[as][h], (g / kRjAccStages) & 1);
+        ptx::tc_fence_after();
+        uint32_t r0[32], r1[32], r2[32], r3[32];
+#pragma unroll
+        for (int rd = 0; rd < kRjRounds; rd++) {
+          const uint32_t c0 = (step0 + i) * kRjCols + rd * 128;
+          const bool need = c0 < w.cmax && c0 + 128 > w.cmin;  // warp-uniform
+          if (need) {
+            ptx::tmem_ld32(r0, tstage + rd * 128);
+            ptx::tmem_ld32(r1, tstage + rd * 128 + 32);
+            ptx::tmem_ld32(r2, tstage + rd * 128 + 64);
+            ptx::tmem_ld32(r3, tstage + rd * 128 + 96);
+            ptx::tmem_ld_wait(r0, r1, r2, r3);
+          }
+          if (rd == kRjRounds - 1) {
+            // every column this warp needs is in registers: hand the stage back to the MMA warp
+            ptx::tc_fence_before();
+            __syncwarp();
+            if (lane == 0) ptx::mbar_arrive(&sm.bar_accempty[as][h]);
+          }
+          if (need) {
+            rj_group(r0, c0, w, lo, width, g1, g2);
+            rj_group(r1, c0 + 32, w, lo, width, g1, g2);
+            rj_group(r2, c0 + 64, w, lo, width, g1, g2);
+            rj_group(r3, c0 + 96, w, lo, width, g1, g2);
+          }
+        }
+      }
+      if (!us.skip && s < us.n_rows) {
+        // a row with no gated-in column has nothing to emit; otherwise the certified test (g1 = a1, g2 <= a2)
+        bool rejected = true;
+        if (valid && g1 > -INFINITY) rejected = certified_reject(na, g1, g2, us.eps, thr, ratio);
+        const uint32_t row_off = us.row_off;
+        rowstat[row_off + s] = rejected ? 1 : 0;
+        if (!rejected) surv_rows[row_off + atomicAdd(surv_count + us.task, 1u)] = s;  // at most n_rows survivors
+      }
+      __syncwarp();
+      if (lane == 0) ptx::mbar_arrive(&sm.bar_uempty[slot]);
+    }
+  }
+  ptx::tc_fence_before();
+  __syncthreads();
+  if (warp == 0) {
+    ptx::tc_fence_after();
+    ptx::tmem_dealloc<512>(tmem);
+  }
+}
+
+}  // namespace fm

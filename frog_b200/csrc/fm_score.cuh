@@ -396,18 +396,6 @@ __device__ __forceinline__ void score_pair(const uint32_t (&ra)[16], const uint3
   }
 }
 
-// Reject pass (kMode 1): the two largest 16-column chunk maxima only -- no threshold, no capture, no vote.
-template <bool kMasked>
-__device__ __forceinline__ void max_pair(const uint32_t (&ra)[16], const uint32_t (&rb)[16], uint32_t col0, uint32_t lo,
-                                         uint32_t width, RowScan& st) {
-  float fa[16], fb[16];
-  const ChunkMax a = chunk_max<kMasked>(ra, col0, lo, width, fa);
-  const ChunkMax b = chunk_max<kMasked>(rb, col0 + 16, lo, width, fb);
-  const float hi = fmaxf(a.m, b.m), lw = fminf(a.m, b.m);
-  st.g2 = max3(st.g2, lw, fminf(st.g1, hi));
-  st.g1 = fmaxf(st.g1, hi);
-}
-
 // One 64-column accumulator tile of one row: two pairs of TMEM loads.
 template <bool kMasked, bool kDump, int kProbe, int kVar>
 __device__ __forceinline__ void score_tile(uint32_t taddr, uint32_t cb, uint32_t lo, uint32_t width, RowScan& st,
@@ -433,8 +421,7 @@ __device__ __forceinline__ void score_tile(uint32_t taddr, uint32_t cb, uint32_t
         dump_row[cb + (c + 1) * 16 + e] = __uint_as_float(rb[e]);
       }
     }
-    if (kVar == 1) max_pair<kMasked>(ra, rb, cb + c * 16, lo, width, st);
-    else score_pair<kMasked, kProbe, kVar>(ra, rb, cb + c * 16, lo, width, st, two_eps, upd, cap);
+    score_pair<kMasked, kProbe, kVar>(ra, rb, cb + c * 16, lo, width, st, two_eps, upd, cap);
   }
 }
 
@@ -447,12 +434,8 @@ __device__ __forceinline__ void score_tile(uint32_t taddr, uint32_t cb, uint32_t
 // dump (kDump only): [256][dump_ld] raw t of the unit.
 // kProbe (performance attribution only, results are garbage): 1 = capture threshold pinned at +inf,
 // i.e. the max-tree fast path alone; 2 = epilogue skips the TMEM loads too (TMA + MMA pipeline alone).
-// kVar = mode of the TWO-PHASE path (fm_fast.cuh decides when to use it; 0 = the ordinary single pass):
-//   1  reject pass: every tile is scored but the epilogue only keeps each row's two largest chunk maxima g1 >= g2
-//      (a third of the single pass's instructions, no look-ahead revisit).  g1 is the row's best approximate score
-//      a1 and g2 <= a2, so the certified rejection test of the rescoring kernel (certified_reject below: the
-//      reference's ratio / threshold test must fail) can be made from them alone.  Writes rowstat[row] = 1 for
-//      rejected rows; the sorted position of every SURVIVING row is appended to its task's survivor list.
+// kVar = mode of the TWO-PHASE path (fm_fast.cuh decides when to use it; 0 = the ordinary single pass).  Its first
+// pass, the reject pass, is reject_kernel (fm_reject.cuh): it writes rowstat and the survivor lists.
 //   2  capture pass on the survivors: surv_plan_kernel cuts every task's survivor list into units of 256 rows and
 //      `unit_off` is the prefix of THOSE units; a unit's row operand tiles are gathered row by row from the image's
 //      operand tiles (generic-proxy stores into the swizzled shared-memory image, then a proxy fence), everything
@@ -530,7 +513,7 @@ score_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ tasks
   // ONE row costs its whole warp the slow path.  Visiting the first tiles once without capturing establishes
   // the threshold of a 64 * n_pre column prefix before the first column is captured: a few tiles of extra
   // MMA work (the tensor pipe has slack) for about a third fewer slow-path entries and no list overflow handling.
-  const uint32_t n_pre = kVar == 1 ? 0u : min(pre_tiles, n_tiles / 4);  // (the single-unit debug launch passes pre_tiles = 0)
+  const uint32_t n_pre = min(pre_tiles, n_tiles / 4);  // (the single-unit debug launch passes pre_tiles = 0)
   const uint32_t n_sched = n_tiles + n_pre;
 
   RowScan st;
@@ -664,22 +647,6 @@ score_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ tasks
     }
   }
 
-  if (kVar == 1) {
-    // Reject pass: certified rejection from (g1, g2) -- the same test rescore_kernel applies to (a1, a2); g1 = a1 and
-    // g2 <= a2, so d2_hi only gets larger (harder to reject).  A row with no gated-in column has nothing to emit.
-    if (is_epi) {
-      bool rejected = true;
-      if (s < B.n && st.g1 > -INFINITY) {
-        const float eps = task_eps(A.meta, B.meta);
-        rejected = certified_reject(B.norm2_sorted[s], st.g1, st.g2, eps, thr, ratio);
-      }
-      if (s < B.n) {
-        rowstat[task.row_off + s] = rejected ? 1 : 0;
-        if (!rejected) surv_rows[task.row_off + atomicAdd(surv_count + t, 1u)] = s;  // at most B.n survivors: the list fits
-      }
-    }
-    return;
-  }
   if (is_epi && s < B.n) {
     // Final list: the entries above the final threshold.
     uint32_t cnt = st.ovf ? 0u : cap_compress(st.cap, min((st.capw - st.cap) / kCapStride, (uint32_t)kCapSlots), st.thr);
