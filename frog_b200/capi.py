@@ -30,7 +30,7 @@ PUBLIC_SYMBOLS = [
     "fm_links_build", "fm_links_total", "fm_links_fetch", "fm_links_offsets", "fm_links_data", "fm_links_device_offsets",
     "fm_links_device_data", "fm_links_build_ms", "fm_links_free",
 ]
-DEBUG_SYMBOLS = ["fm_debug_image", "fm_debug_score_unit", "fm_debug_set_option"]
+DEBUG_SYMBOLS = ["fm_debug_image", "fm_debug_image_norms", "fm_debug_score_unit", "fm_debug_set_option"]
 
 
 class Stats(C.Structure):
@@ -96,6 +96,7 @@ def load():
     L.fm_get_stats.argtypes = [vp, C.POINTER(Stats)]
     L.fm_version.restype = C.c_char_p
     L.fm_debug_image.argtypes = [vp, C.c_uint32, u32p, u32p, f32p, u32p, f32p, vp, vp, vp, vp]
+    L.fm_debug_image_norms.argtypes = [vp, C.c_uint32, f32p, f32p, f32p]
     L.fm_debug_score_unit.argtypes = [vp, C.c_uint32, C.c_uint32, C.c_uint32, vp, C.c_uint32, vp, vp, vp]
     L.fm_debug_set_option.argtypes = [C.c_char_p, C.c_int]
     L.fm_links_build.argtypes = [vp, vp, vp, vp, C.POINTER(vp)]
@@ -312,6 +313,11 @@ class Matcher:
                     class_lap=np.array(class_lap[:ncls.value], np.float32),
                     class_begin=np.array(class_begin[:ncls.value + 1], np.uint32),
                     perm=perm[:n], scale_sorted=ss[:n], rowop=rowop, colop=colop)
+
+    def debug_image_norms(self, img: int) -> dict:
+        mn, mx, md = C.c_float(), C.c_float(), C.c_float()
+        self._check(self._L.fm_debug_image_norms(self._h, img, C.byref(mn), C.byref(mx), C.byref(md)))
+        return dict(min_norm2=mn.value, max_norm2=mx.value, max_delta2=md.value)
 
     def debug_score_unit(self, first_img: int, second_img: int, row_block: int, n_first: int, n_second: int) -> dict:
         ld = (n_first + 255) & ~255

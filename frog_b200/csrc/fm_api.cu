@@ -970,6 +970,18 @@ int fm_debug_image(fm_ctx* c, uint32_t img, uint32_t* flags, uint32_t* n_classes
   return FM_OK;
 }
 
+int fm_debug_image_norms(fm_ctx* c, uint32_t img, float* min_norm2_out, float* max_norm2, float* max_delta2) {
+  if (!c || img >= c->images.size() || !c->images[img].valid) return FM_ERR_INVALID;
+  FM_CUDA(c, cudaSetDevice(c->device));
+  int rc = sync_images(c);
+  if (rc != FM_OK) return rc;
+  const ImageMeta& m = c->h_metas[img];
+  if (min_norm2_out) *min_norm2_out = min_norm2(m);
+  if (max_norm2) *max_norm2 = m.max_norm2;
+  if (max_delta2) *max_delta2 = m.max_delta2;
+  return FM_OK;
+}
+
 int fm_debug_score_unit(fm_ctx* c, uint32_t first_img, uint32_t second_img, uint32_t row_block, float* t_out,
                         uint32_t ld, uint32_t* bands_out, float* cand_t, uint32_t* cand_col) {
   if (!c || first_img >= c->images.size() || second_img >= c->images.size() || !c->images[first_img].valid ||

@@ -4,6 +4,7 @@
 #include <cuda_fp16.h>
 #include <cfloat>
 #include <cstdint>
+#include <cstring>
 
 namespace fm {
 
@@ -29,7 +30,16 @@ struct ImageMeta {
   float max_delta2;                   // max squared L2 norm of (fp16(desc) - desc): actual FP16 rounding residual
   float class_lap[kMaxClasses];       // laplacian value of each class, ascending bit pattern order
   uint32_t class_begin[kMaxClasses + 1];  // class c occupies sorted positions [begin[c], begin[c+1])
+  uint32_t min_norm2_inv;             // ~(bit pattern) of the min squared L2 norm, kept by atomicMax so that the zeroed
+                                      // word means "no keypoint yet" (min_norm2() then reads NaN)
 };
+
+__host__ __device__ __forceinline__ float min_norm2(const ImageMeta& m) {
+  const uint32_t u = ~m.min_norm2_inv;
+  float f;
+  memcpy(&f, &u, 4);
+  return f;
+}
 
 // Device view of one image.  Arrays marked (orig) are in upload order -- the ids pairs.bin carries;
 // arrays marked (sorted) are ordered by (laplacian class, scale) for the tensor-core path.

@@ -9,7 +9,8 @@
 //     tile layout tcgen05.mma reads, so one 16 KB cp.async.bulk lands a ready tile in shared memory.
 //     K is padded 48 -> 64: slots 48,49 carry (1, 1) on the row side and the hi/lo FP16 halves of
 //     -|b|^2/2 on the column side, so the MMA itself yields  t = a.b - |b|^2/2  = (|a|^2 - d^2)/2.
-//   * per-image flags + max squared norm (certification inputs for the FP32 rescoring).
+//   * per-image flags + max squared norm (certification inputs for the FP32 rescoring) and min squared
+//     norm (the reject pass drops the norm slots for column images whose norms barely vary, fm_reject.cuh).
 #pragma once
 #include <cub/device/device_radix_sort.cuh>
 
@@ -88,16 +89,20 @@ prep_keys_kernel(const ImageDev* __restrict__ images, const PrepSeg* __restrict_
   // warp-aggregate then one atomic per warp
   float m = isfinite(n2) ? n2 : 0.f;
   float md = isfinite(dl2) ? dl2 : 0.f;
+  // the min: complemented patterns, 0 (contributes nothing to the atomicMax) past the image and for non-finite norms
+  uint32_t mn_inv = (i < seg.n && isfinite(n2)) ? ~__float_as_uint(n2) : 0u;
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
     md = fmaxf(md, __shfl_xor_sync(0xffffffffu, md, o));
+    mn_inv = max(mn_inv, __shfl_xor_sync(0xffffffffu, mn_inv, o));
     flags |= __shfl_xor_sync(0xffffffffu, flags, o);
   }
   if ((threadIdx.x & 31) == 0) {
     if (flags) atomicOr(&meta->flags, flags);
     atomicMax(reinterpret_cast<unsigned int*>(&meta->max_norm2), __float_as_uint(m));   // non-negative floats
     atomicMax(reinterpret_cast<unsigned int*>(&meta->max_delta2), __float_as_uint(md));  // order like uints
+    if (mn_inv) atomicMax(&meta->min_norm2_inv, mn_inv);
   }
 }
 

@@ -3,11 +3,15 @@
 // rejection test (certified_reject, fm_score.cuh) and the survivor list the capture pass works on.
 //
 // One persistent CTA per SM walks units blockIdx.x, blockIdx.x + gridDim.x, ...  Per 256-column step the unit's two
-// row halves each take one tcgen05.mma M=128 x N=256 x K=16 chain (4 K-steps) into their own 256-column TMEM buffer.
+// row halves each take one tcgen05.mma M=128 x N<=256 x K=16 chain into their own 256-column TMEM buffer.
 // Against the single pass's N=64 this reads the row operand once per 256 columns instead of once per 64: 12 KB of
 // shared-memory operand reads per 128 cycles of MMA math instead of 6 KB per 32, which is what kept the tensor pipe
-// below half its rate.  The accumulator shape (M=128, FP32, K=64 in four steps) is the single pass's, so every score,
-// and therefore g1, g2 and the set of rejected rows, is the same.
+// below half its rate.  Two cuts keep the MMAs to the work the result needs:
+//   * a half's chain covers only the step's columns inside that half's own band union, rounded out to 16 columns;
+//   * for column images whose squared norms barely vary (normalised descriptors) the chain is 3 K-steps, not 4: the
+//     norm term moves out of the MMA into the rejection test as the image's norm range (rj_ksteps).
+// Any other image keeps the single pass's accumulator (M=128, FP32, K=64 in four steps), so its scores, and therefore
+// its g1, g2 and rejected rows, are the single pass's.
 //   warp 0      scheduler  : task lookup, the unit's 256 bands and its column-step range -> a 4-slot ring in shared
 //                            memory, so unit prologues (dependent global loads) run ahead of the pipeline
 //   warp 1      TMA        : the unit's two 16 KB row-operand tiles (double-buffered across units) and 32 KB column
@@ -45,10 +49,28 @@ struct RjUnit {
   const float* norm2;
   uint32_t task, n_rows, row_off, s0;  // s0: sorted position of the unit's first row
   uint32_t step0, n_steps;             // column steps [step0, step0 + n_steps) of kRjCols columns
-  uint32_t halves;                     // row halves holding rows of the image (1: the image ends in row half 0)
+  uint2 span[2];                       // row half h's bands lie in columns [span[h].x, span[h].y) (empty: y <= x)
+  uint32_t ksteps;                     // K-steps per MMA chain: 4, or 3 without the norm slots (see rj_ksteps)
+  float noff1, noff2;                  // ksteps == 3: n_min / 2 and n_max / 2 of the column image; else 0
   float eps;
   uint32_t skip;                       // task takes the exact kernel: nothing to write
 };
+
+// K = 48 instead of 64 for a column image whose squared norms barely vary (SURF3D descriptors are L2-normalised).
+// The fourth K-step (slots 48..63) only adds the column's -|b|^2/2 through slots 48 and 49.  Without it the MMA yields
+// t' = fp16(a).fp16(b) in FP32, and the K = 64 score is t = t' - n_b/2 with n_b in [n_min, n_max] (FP32 norms, the values
+// the operand carries).  The unit end then tests, instead of the row's g1 and g2 of t,
+//   a1 = g1' - n_min/2  (rounded up)    >= best t       (every column's t <= t' - n_min/2 <= g1' - n_min/2)
+//   a2 = g2' - n_max/2  (rounded down)  <= second t     (two columns of different chunks reach t' >= g2')
+// so certified_reject keeps its meaning: rounding toward +-inf makes the FP32 subtractions one-sided, with no slack
+// term.  The existing eps still bounds |t' - n_b/2 - (a.b - |b|^2/2)|: of its additive part, the hi/lo split of
+// -|b|^2/2 is gone, and the FP32 accumulation inside the tensor core now sums 48 products without the norm term,
+// less than the 64-term bound it was given; the operand rounding terms are the same.  What the rows lose is
+// (n_max - n_min)/2 of certification margin, hence the rule: K = 48 when that is at most eps, so that normalised inputs
+// reject as before (differences only at the certification edge), while any other image keeps its exact K = 64 chain.
+__device__ __forceinline__ uint32_t rj_ksteps(const ImageMeta& col, float eps) {
+  return 0.5f * (col.max_norm2 - min_norm2(col)) <= eps ? 3u : 4u;  // (no keypoint: min_norm2 is NaN, 4)
+}
 
 struct alignas(1024) RejectSmem {
   uint8_t a[2][2][kOpTileBytes];        // [unit buffer][row half]
@@ -100,8 +122,8 @@ __device__ __forceinline__ void rj_group(const uint32_t (&r)[32], uint32_t gc, c
   g1 = fmaxf(g1, hi);
 }
 
-// units = unit_off[n_tasks] (segs = 1).  scored_cols += (row, column) scores the tensor cores computed: 128 x kRjCols
-// per MMA chain issued, band-edge and past-the-band columns of a step included.  Writes rowstat[row] (1 = rejected) for every row of every fast task and
+// units = unit_off[n_tasks] (segs = 1).  scored_cols += (row, column) scores the tensor cores computed: 128 x N per
+// MMA chain issued, band-edge and 16-column round-out columns included.  Writes rowstat[row] (1 = rejected) for every row of every fast task and
 // appends the sorted position of each surviving row to its task's survivor list (surv_count / surv_rows, any order).
 __global__ void __launch_bounds__(kRjThreads, 1)
 reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ tasks, const uint32_t* __restrict__ unit_off,
@@ -147,21 +169,25 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
       const ImageDev B = images[task.row_img];
       const uint32_t s0 = (unit - unit_off[t]) * kUnitRows;
       const bool skip = (task.flags & kTaskExact) != 0;
-      uint32_t cmin = 0xFFFFFFFFu, cmax = 0u;
+      uint32_t cmin[2] = {0xFFFFFFFFu, 0xFFFFFFFFu}, cmax[2] = {0u, 0u};  // per row half
 #pragma unroll
       for (int j = 0; j < kUnitRows / 32; j++) {
         const uint32_t r = j * 32 + lane, s = s0 + r;
+        const int h = j / (kUnitRows / 64);
         uint2 bd = make_uint2(0u, 0u);
         if (!skip && s < B.n) bd = bands[task.row_off + s];
-        if (bd.y > bd.x) { cmin = min(cmin, bd.x); cmax = max(cmax, bd.y); }
+        if (bd.y > bd.x) { cmin[h] = min(cmin[h], bd.x); cmax[h] = max(cmax[h], bd.y); }
         sm.band[slot][r] = bd;
       }
 #pragma unroll
-      for (int o = 16; o > 0; o >>= 1) {
-        cmin = min(cmin, __shfl_xor_sync(0xffffffffu, cmin, o));
-        cmax = max(cmax, __shfl_xor_sync(0xffffffffu, cmax, o));
-      }
+      for (int o = 16; o > 0; o >>= 1)
+#pragma unroll
+        for (int h = 0; h < 2; h++) {
+          cmin[h] = min(cmin[h], __shfl_xor_sync(0xffffffffu, cmin[h], o));
+          cmax[h] = max(cmax[h], __shfl_xor_sync(0xffffffffu, cmax[h], o));
+        }
       if (lane == 0) {
+        const uint32_t umin = min(cmin[0], cmin[1]), umax = max(cmax[0], cmax[1]);
         RjUnit u;
         u.rowop = reinterpret_cast<const uint8_t*>(B.rowop) + (size_t)s0 / 128 * kOpTileBytes;
         u.colop = reinterpret_cast<const uint8_t*>(A.colop);
@@ -170,11 +196,15 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
         u.n_rows = B.n;
         u.row_off = task.row_off;
         u.s0 = s0;
-        u.step0 = cmax > cmin ? cmin / kRjCols : 0u;
-        u.n_steps = cmax > cmin ? (cmax + kRjCols - 1) / kRjCols - u.step0 : 0u;
+        u.step0 = umax > umin ? umin / kRjCols : 0u;
+        u.n_steps = umax > umin ? (umax + kRjCols - 1) / kRjCols - u.step0 : 0u;
+        u.span[0] = make_uint2(cmin[0], cmax[0]);
+        u.span[1] = make_uint2(cmin[1], cmax[1]);
         u.eps = skip ? 0.f : task_eps(A.meta, B.meta);
+        u.ksteps = skip ? 4u : rj_ksteps(*A.meta, u.eps);
+        u.noff1 = u.ksteps == 3 ? 0.5f * min_norm2(*A.meta) : 0.f;
+        u.noff2 = u.ksteps == 3 ? 0.5f * A.meta->max_norm2 : 0.f;
         u.skip = skip ? 1u : 0u;
-        u.halves = B.n - s0 > 128 ? 2u : 1u;
         sm.unit[slot] = u;
       }
       ptx::mbar_arrive(&sm.bar_ufull[slot]);
@@ -211,13 +241,14 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
   } else if (warp == 2) {
     // ---- MMA ----------------------------------------------------------------------------------------------------
     if (lane == 0) {
-      constexpr uint32_t idesc = ptx::umma_idesc_f16_f32(128, kRjCols);
       uint32_t k = 0, a_use = 0, bq = 0, g = 0;
       unsigned long long issued = 0;
       for (uint32_t unit = blockIdx.x; unit < units; unit += gridDim.x, k++) {
         const uint32_t slot = k % kRjSlots;
         ptx::mbar_wait(&sm.bar_ufull[slot], (k / kRjSlots) & 1);
-        const uint32_t n_steps = sm.unit[slot].n_steps, halves = sm.unit[slot].halves;
+        const RjUnit& us = sm.unit[slot];
+        const uint32_t step0 = us.step0, n_steps = us.n_steps, ksteps = us.ksteps;
+        const uint2 span[2] = {us.span[0], us.span[1]};
         ptx::mbar_arrive(&sm.bar_uempty[slot]);
         if (n_steps == 0) continue;
         const uint32_t ab = a_use & 1;
@@ -225,19 +256,27 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
         a_use++;
         const uint64_t adesc[2] = {ptx::umma_desc_sw128(ptx::smem_u32(sm.a[ab][0])), ptx::umma_desc_sw128(ptx::smem_u32(sm.a[ab][1]))};
         for (uint32_t i = 0; i < n_steps; i++, bq++, g++) {
-          const uint32_t stg = bq % kRjStages;
+          const uint32_t stg = bq % kRjStages, c0 = (step0 + i) * kRjCols;
           ptx::mbar_wait(&sm.bar_bfull[stg], (bq / kRjStages) & 1);
-          const uint64_t bdesc = ptx::umma_desc_sw128(ptx::smem_u32(sm.b[stg]));
 #pragma unroll
           for (int h = 0; h < 2; h++) {
             const uint32_t as = g % kRjAccStages, use = g / kRjAccStages;
             if (use > 0) ptx::mbar_wait(&sm.bar_accempty[as][h], (use - 1) & 1);
             ptx::tc_fence_after();
-            if ((uint32_t)h < halves) {  // (a half without rows is still handed to its epilogue warps, unscored)
+            // Only the step's columns inside this half's span, in whole 16-column pieces (N = 16 .. 256; a B operand
+            // starting 16 j rows into the step starts on a 1024 B swizzle atom).  The buffer's other columns keep
+            // stale values: they lie outside every band of the half, so the epilogue masks or skips them.  A half
+            // whose span misses the step (or that has no rows) is still handed to its epilogue warps, unscored.
+            const uint32_t lo = max(span[h].x, c0), hi = min(span[h].y, c0 + kRjCols);
+            if (hi > lo) {
+              const uint32_t off = (lo - c0) & ~15u, n = ((hi - c0 + 15) & ~15u) - off;
+              const uint32_t idesc = ptx::umma_idesc_f16_f32(128, (int)n);
+              const uint64_t bdesc = ptx::umma_desc_sw128(ptx::smem_u32(sm.b[stg]) + off * 128);
 #pragma unroll
-              for (int kk = 0; kk < kKPad / 16; kk++)  // +32 B per K step inside the 128 B swizzle row
-                ptx::mma_f16_ss(tmem + (as * 2 + h) * kRjCols, adesc[h] + 2 * kk, bdesc + 2 * kk, idesc, kk > 0);
-              issued += 128 * kRjCols;
+              for (uint32_t kk = 0; kk < kKPad / 16; kk++)  // +32 B per K step inside the 128 B swizzle row
+                if (kk < ksteps)
+                  ptx::mma_f16_ss(tmem + (as * 2 + h) * kRjCols + off, adesc[h] + 2 * kk, bdesc + 2 * kk, idesc, kk > 0);
+              issued += 128 * n;
             }
             ptx::mma_commit(&sm.bar_accfull[as][h]);
           }
@@ -308,7 +347,9 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
       if (!us.skip && s < us.n_rows) {
         // a row with no gated-in column has nothing to emit; otherwise the certified test (g1 = a1, g2 <= a2)
         bool rejected = true;
-        if (valid && g1 > -INFINITY) rejected = certified_reject(na, g1, g2, us.eps, thr, ratio);
+        // (K = 48: the bounds of rj_ksteps; K = 64: the offsets are 0 and a1, a2 are g1, g2)
+        if (valid && g1 > -INFINITY)
+          rejected = certified_reject(na, __fsub_ru(g1, us.noff1), __fsub_rd(g2, us.noff2), us.eps, thr, ratio);
         const uint32_t row_off = us.row_off;
         rowstat[row_off + s] = rejected ? 1 : 0;
         if (!rejected) surv_rows[row_off + atomicAdd(surv_count + us.task, 1u)] = s;  // at most n_rows survivors

@@ -23,6 +23,13 @@ int fm_debug_image(fm_ctx* ctx, uint32_t img, uint32_t* flags, uint32_t* n_class
                    uint16_t* rowop, uint16_t* colop);
 
 /*
+ * Squared-norm statistics of an uploaded image's descriptors (FP32), as the certified bounds use them:
+ * min_norm2 / max_norm2 over its keypoints (min_norm2 is NaN for an image without keypoints) and max_delta2, the
+ * largest squared norm of the FP16 rounding residual.  Any output pointer may be NULL.
+ */
+int fm_debug_image_norms(fm_ctx* ctx, uint32_t img, float* min_norm2, float* max_norm2, float* max_delta2);
+
+/*
  * Run the band kernel and ONE unit (256 sorted rows starting at row_block * 256 of image
  * `second` against the band of image `first`) of the tensor-core scoring kernel in dump mode.
  *   t_out    : 256 x ld floats, t_out[r * ld + col] = raw score of (unit row r, sorted column col);
