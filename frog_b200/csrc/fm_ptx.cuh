@@ -61,6 +61,11 @@ __device__ __forceinline__ void mbar_wait_u32(uint32_t bar, uint32_t parity) {
   } while (!ok);
 }
 
+// Named barrier `id` (1 .. 15; 0 is __syncthreads) over `count` threads, a multiple of 32.
+__device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t count) {
+  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory");
+}
+
 // ---- TMA engine, 1-D bulk copy global -> shared, completion on an mbarrier (SASS: UBLKCP) -------
 __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(

@@ -17,28 +17,27 @@
 //   warp 1      TMA        : the unit's two 16 KB row-operand tiles (double-buffered across units) and 32 KB column
 //                            steps into a 4-stage ring
 //   warp 2      MMA        : buffer h <- row half h, alternating, so one half's MMAs run while the other is drained
-//   warps 3..10 epilogue   : (TMEM lane quadrant = warp % 4) x (row half): one row per thread.  Each warp loads a
-//                            step's 256 columns in two rounds of 128, releases the buffer after the second load, and
-//                            reduces 32-column groups with 3-input max trees; masking is decided per group, warp-
-//                            uniformly.  (Eight warps, not sixteen: eleven warps leave 168 registers per thread for the
-//                            128-column rounds, nineteen would leave 96.)
+//   warps 3..10 epilogue   : (TMEM lane quadrant = warp % 4) x (column round c): every warp drains every buffer, in
+//                            the order the MMA warp fills them, loading its 128 columns [128 c, 128 c + 128) and
+//                            releasing the buffer before it reduces them, so a buffer goes back to the MMA warp one
+//                            TMEM load after it was published.  Whether a round is skipped, interior (straight-line
+//                            max trees) or masked is decided once per round, warp-uniformly.  Each thread keeps a
+//                            partial (g1, g2) for its row in both halves; at unit end the quadrant's two warps merge
+//                            them (exactly: max and min) and warp (q, c) tests the rows of half c.  (Eight warps, not
+//                            sixteen: eleven warps leave 168 registers per thread for the 128-column rounds, nineteen
+//                            would leave 96.)
 // Scores never leave the SM.
 #pragma once
 #include "fm_score.cuh"
 
 namespace fm {
 
-// N of one MMA: columns per step, 128 or 256 (FM_REJECT_COLS overrides it to time the other one).  TMEM holds
-// 512 / (2 N) accumulator stages of both row halves; the epilogue loads a stage in rounds of 128 columns.
-#ifndef FM_REJECT_COLS
-#define FM_REJECT_COLS 256
-#endif
-constexpr int kRjCols = FM_REJECT_COLS;
-static_assert(kRjCols == 128 || kRjCols == 256, "reject pass: N = 128 or 256");
-constexpr int kRjAccStages = 512 / (2 * kRjCols);
-constexpr int kRjRounds = kRjCols / 128;
-constexpr int kRjStepBytes = kRjCols * 128;  // one step of the column operand: N / 128 stored operand tiles
-constexpr int kRjStages = 4 * 256 / kRjCols; // 128 KB of column-operand ring
+// One step is 256 columns (N = 256): TMEM's 512 columns hold one accumulator buffer per row half, and each epilogue
+// warp drains one 128-column round of every buffer.  (N = 128 with two stages per half measured 1.3x slower: the row
+// operand is re-read from shared memory for every 128 columns.)
+constexpr int kRjCols = 256;
+constexpr int kRjStepBytes = kRjCols * 128;  // one step of the column operand: two stored operand tiles
+constexpr int kRjStages = 4;                 // 128 KB of column-operand ring
 constexpr int kRjSlots = 4;                  // units the scheduler warp may run ahead
 constexpr int kRjEpiWarps = 8;
 constexpr int kRjThreads = (3 + kRjEpiWarps) * 32;
@@ -46,7 +45,6 @@ constexpr int kRjThreads = (3 + kRjEpiWarps) * 32;
 struct RjUnit {
   const uint8_t* rowop;  // the unit's two row-operand tiles (row halves 0 and 1)
   const uint8_t* colop;
-  const float* norm2;
   uint32_t task, n_rows, row_off, s0;  // s0: sorted position of the unit's first row
   uint32_t step0, n_steps;             // column steps [step0, step0 + n_steps) of kRjCols columns
   uint2 span[2];                       // row half h's bands lie in columns [span[h].x, span[h].y) (empty: y <= x)
@@ -72,54 +70,76 @@ __device__ __forceinline__ uint32_t rj_ksteps(const ImageMeta& col, float eps) {
   return 0.5f * (col.max_norm2 - min_norm2(col)) <= eps ? 3u : 4u;  // (no keypoint: min_norm2 is NaN, 4)
 }
 
+struct RjWarpRange {
+  uint32_t cmin, cmax;  // columns some row of the warp accepts lie in [cmin, cmax)
+  uint32_t imin, imax;  // every row of the warp accepts [imin, imax)
+};
+
 struct alignas(1024) RejectSmem {
   uint8_t a[2][2][kOpTileBytes];        // [unit buffer][row half]
   uint8_t b[kRjStages][kRjStepBytes];
   uint2 band[kRjSlots][kUnitRows];      // the unit's bands, (0, 0) for rows past the image
+  float norm2[kRjSlots][kUnitRows];     // the rows' squared norms (rows with a band only)
   RjUnit unit[kRjSlots];
   uint64_t bar_afull[2], bar_aempty[2];
   uint64_t bar_bfull[kRjStages], bar_bempty[kRjStages];
-  uint64_t bar_accfull[kRjAccStages][2], bar_accempty[kRjAccStages][2];  // [stage][row half]
+  uint64_t bar_accfull[2], bar_accempty[2];  // [row half]
   uint64_t bar_ufull[kRjSlots], bar_uempty[kRjSlots];
+  float2 part[2][kUnitRows];                 // [unit parity][row]: (g1, g2) of one column round, passed at unit end
+  RjWarpRange wrange[kRjEpiWarps][2];        // [epilogue warp][row half], warp-uniform (kept out of registers)
   uint32_t tmem_base;
 };
 constexpr size_t kRjSmemBytes = sizeof(RejectSmem) + 1024;
 
-// Maximum of 16 consecutive columns (index O of r); kMasked: columns outside [lo, lo + width) count as -inf.
+// Maximum of the 16 columns r[O .. O + 16) of a 32-column group; kMasked: column O + e counts only if bit O + e of
+// the group's mask m is set (a bit test and a select per score), otherwise as -inf.
 template <bool kMasked, int O>
-__device__ __forceinline__ float rj_chunk(const uint32_t (&r)[32], uint32_t col0, uint32_t lo, uint32_t width) {
+__device__ __forceinline__ float rj_chunk(const uint32_t (&r)[32], uint32_t m) {
   float f[16];
 #pragma unroll
   for (int e = 0; e < 16; e++) {
     f[e] = __uint_as_float(r[O + e]);
-    if (kMasked) f[e] = ((col0 + e) - lo < width) ? f[e] : -INFINITY;
+    if (kMasked) f[e] = (m & (1u << (O + e))) ? f[e] : -INFINITY;
   }
   const float ga = max3(max3(f[0], f[1], f[2]), max3(f[3], f[4], f[5]), max3(f[6], f[7], f[8]));
   const float gb = max3(max3(f[9], f[10], f[11]), max3(f[12], f[13], f[14]), f[15]);
   return fmaxf(ga, gb);
 }
 
-struct RjWarpRange {
-  uint32_t cmin, cmax;  // columns some row of the warp accepts lie in [cmin, cmax)
-  uint32_t imin, imax;  // every row of the warp accepts [imin, imax)
-};
+// (a1 >= a2) and (b1 >= b2) are the two largest values of two multisets: make (a1, a2) those of their union.  Max and
+// min are exact, so the result does not depend on how a row's chunk maxima are grouped.
+__device__ __forceinline__ void rj_top2(float& a1, float& a2, float b1, float b2) {
+  a2 = max3(a2, b2, fminf(a1, b1));
+  a1 = fmaxf(a1, b1);
+}
 
-// 32 columns starting at gc (a multiple of 32, so the two 16-column chunks are the single pass's chunks): fold both
-// chunk maxima into the row's top two (g1 >= g2).
-__device__ __forceinline__ void rj_group(const uint32_t (&r)[32], uint32_t gc, const RjWarpRange& w, uint32_t lo,
-                                         uint32_t width, float& g1, float& g2) {
-  if (gc >= w.cmax || gc + 32 <= w.cmin) return;  // warp-uniform: no row of the warp accepts these columns
-  float a, b;
-  if (gc >= w.imin && gc + 32 <= w.imax) {
-    a = rj_chunk<false, 0>(r, gc, lo, width);
-    b = rj_chunk<false, 16>(r, gc + 16, lo, width);
-  } else {
-    a = rj_chunk<true, 0>(r, gc, lo, width);
-    b = rj_chunk<true, 16>(r, gc + 16, lo, width);
+// Bits [0, n) set, n clamped to [0, 32].
+__device__ __forceinline__ uint32_t rj_bits_below(int n) { return __funnelshift_lc(0xFFFFFFFFu, 0u, (uint32_t)max(n, 0)); }
+
+// One 128-column round (r0 .. r3, 32 columns each, starting at a multiple of 128, so its eight 16-column chunks are the
+// single pass's chunks): fold the chunk maxima into the row's top two (g1 >= g2).  kMasked: only columns
+// [a, a + width) of the round count (a relative to the round's first column, may be negative).
+template <bool kMasked>
+__device__ __forceinline__ void rj_round(const uint32_t (&r0)[32], const uint32_t (&r1)[32], const uint32_t (&r2)[32],
+                                         const uint32_t (&r3)[32], int a, int width, float& g1, float& g2) {
+  uint32_t m[4] = {0u, 0u, 0u, 0u};  // group j's columns [a - 32 j, a + width - 32 j) as bits
+  if (kMasked)
+#pragma unroll
+    for (int j = 0; j < 4; j++) m[j] = rj_bits_below(a + width - 32 * j) & ~rj_bits_below(a - 32 * j);
+  const float c[8] = {rj_chunk<kMasked, 0>(r0, m[0]), rj_chunk<kMasked, 16>(r0, m[0]),
+                      rj_chunk<kMasked, 0>(r1, m[1]), rj_chunk<kMasked, 16>(r1, m[1]),
+                      rj_chunk<kMasked, 0>(r2, m[2]), rj_chunk<kMasked, 16>(r2, m[2]),
+                      rj_chunk<kMasked, 0>(r3, m[3]), rj_chunk<kMasked, 16>(r3, m[3])};
+  float t1[4], t2[4];
+#pragma unroll
+  for (int p = 0; p < 4; p++) {
+    t1[p] = fmaxf(c[2 * p], c[2 * p + 1]);
+    t2[p] = fminf(c[2 * p], c[2 * p + 1]);
   }
-  const float hi = fmaxf(a, b), lw = fminf(a, b);
-  g2 = max3(g2, lw, fminf(g1, hi));
-  g1 = fmaxf(g1, hi);
+  rj_top2(t1[0], t2[0], t1[1], t2[1]);
+  rj_top2(t1[2], t2[2], t1[3], t2[3]);
+  rj_top2(t1[0], t2[0], t1[2], t2[2]);
+  rj_top2(g1, g2, t1[0], t2[0]);
 }
 
 // units = unit_off[n_tasks] (segs = 1).  scored_cols += (row, column) scores the tensor cores computed: 128 x N per
@@ -139,11 +159,10 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
       ptx::mbar_init(&sm.bar_afull[i], 1);
       ptx::mbar_init(&sm.bar_aempty[i], 1);
     }
-    for (int i = 0; i < kRjAccStages; i++)
-      for (int h = 0; h < 2; h++) {
-        ptx::mbar_init(&sm.bar_accfull[i][h], 1);
-        ptx::mbar_init(&sm.bar_accempty[i][h], kRjEpiWarps / 2);
-      }
+    for (int h = 0; h < 2; h++) {
+      ptx::mbar_init(&sm.bar_accfull[h], 1);
+      ptx::mbar_init(&sm.bar_accempty[h], kRjEpiWarps);  // every epilogue warp drains every buffer
+    }
     for (int i = 0; i < kRjStages; i++) { ptx::mbar_init(&sm.bar_bfull[i], 1); ptx::mbar_init(&sm.bar_bempty[i], 1); }
     for (int i = 0; i < kRjSlots; i++) {
       ptx::mbar_init(&sm.bar_ufull[i], 32);                // every lane of the scheduler warp
@@ -178,6 +197,7 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
         if (!skip && s < B.n) bd = bands[task.row_off + s];
         if (bd.y > bd.x) { cmin[h] = min(cmin[h], bd.x); cmax[h] = max(cmax[h], bd.y); }
         sm.band[slot][r] = bd;
+        if (bd.y > bd.x) sm.norm2[slot][r] = B.norm2_sorted[s];
       }
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1)
@@ -191,7 +211,6 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
         RjUnit u;
         u.rowop = reinterpret_cast<const uint8_t*>(B.rowop) + (size_t)s0 / 128 * kOpTileBytes;
         u.colop = reinterpret_cast<const uint8_t*>(A.colop);
-        u.norm2 = B.norm2_sorted;
         u.task = t;
         u.n_rows = B.n;
         u.row_off = task.row_off;
@@ -260,8 +279,7 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
           ptx::mbar_wait(&sm.bar_bfull[stg], (bq / kRjStages) & 1);
 #pragma unroll
           for (int h = 0; h < 2; h++) {
-            const uint32_t as = g % kRjAccStages, use = g / kRjAccStages;
-            if (use > 0) ptx::mbar_wait(&sm.bar_accempty[as][h], (use - 1) & 1);
+            if (g > 0) ptx::mbar_wait(&sm.bar_accempty[h], (g - 1) & 1);
             ptx::tc_fence_after();
             // Only the step's columns inside this half's span, in whole 16-column pieces (N = 16 .. 256; a B operand
             // starting 16 j rows into the step starts on a 1024 B swizzle atom).  The buffer's other columns keep
@@ -275,10 +293,10 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
 #pragma unroll
               for (uint32_t kk = 0; kk < kKPad / 16; kk++)  // +32 B per K step inside the 128 B swizzle row
                 if (kk < ksteps)
-                  ptx::mma_f16_ss(tmem + (as * 2 + h) * kRjCols + off, adesc[h] + 2 * kk, bdesc + 2 * kk, idesc, kk > 0);
+                  ptx::mma_f16_ss(tmem + h * kRjCols + off, adesc[h] + 2 * kk, bdesc + 2 * kk, idesc, kk > 0);
               issued += 128 * n;
             }
-            ptx::mma_commit(&sm.bar_accfull[as][h]);
+            ptx::mma_commit(&sm.bar_accfull[h]);
           }
           ptx::mma_commit(&sm.bar_bempty[stg]);
         }
@@ -288,9 +306,12 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
     }
   } else {
     // ---- epilogue -----------------------------------------------------------------------------------------------
-    const uint32_t h = (warp - 3) >> 2, q = warp & 3;  // row half, TMEM lane quadrant
-    const uint32_t row = h * 128 + q * 32 + lane;
-    uint32_t taddr = tmem + ((q * 32) << 16) + h * kRjCols;
+    // Warp (q, c): TMEM lane quadrant q = warp % 4 (the lanes the warp may access) and column round c: columns
+    // [128 c, 128 c + 128) of every step, in both row halves' buffers.  Per row half h, thread `lane` keeps row
+    // 128 h + 32 q + lane: its band and the (g1, g2) of the chunks in the warp's rounds.  At unit end the quadrant's two
+    // warps exchange their partial pairs through shared memory, and warp (q, c) tests the rows of half c.
+    const uint32_t c = (warp - 3) >> 2, q = warp & 3;
+    uint32_t taddr = tmem + ((q * 32) << 16) + c * 128;
     asm volatile("" : "+r"(taddr));
     uint32_t g = 0, k = 0;
     for (uint32_t unit = blockIdx.x; unit < units; unit += gridDim.x, k++) {
@@ -299,57 +320,73 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
       // (the slot is released at unit end, after the rejection tail has read the rest of it)
       const RjUnit& us = sm.unit[slot];
       const uint32_t step0 = us.step0, n_steps = us.n_steps;
-      const uint2 bd = sm.band[slot][row];
-      const uint32_t s = us.s0 + row;
-      const bool valid = bd.y > bd.x;
-      const uint32_t lo = bd.x, width = bd.y - bd.x;
-      const float na = valid ? us.norm2[s] : 0.f;  // used at unit end (valid: s is a row of the image)
-      RjWarpRange w{valid ? lo : 0xFFFFFFFFu, valid ? bd.y : 0u, valid ? lo : 0u, valid ? bd.y : 0xFFFFFFFFu};
+      const uint2* band = sm.band[slot] + q * 32 + lane;  // + 128 h: this thread's row of half h
+      RjWarpRange* wr = sm.wrange[warp - 3];
 #pragma unroll
-      for (int o = 16; o > 0; o >>= 1) {
-        w.cmin = min(w.cmin, __shfl_xor_sync(0xffffffffu, w.cmin, o));
-        w.cmax = max(w.cmax, __shfl_xor_sync(0xffffffffu, w.cmax, o));
-        w.imin = max(w.imin, __shfl_xor_sync(0xffffffffu, w.imin, o));
-        w.imax = min(w.imax, __shfl_xor_sync(0xffffffffu, w.imax, o));
+      for (int h = 0; h < 2; h++) {
+        const uint2 bd = band[h * 128];
+        const bool valid = bd.y > bd.x;
+        RjWarpRange w{valid ? bd.x : 0xFFFFFFFFu, valid ? bd.y : 0u, valid ? bd.x : 0u, valid ? bd.y : 0xFFFFFFFFu};
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+          w.cmin = min(w.cmin, __shfl_xor_sync(0xffffffffu, w.cmin, o));
+          w.cmax = max(w.cmax, __shfl_xor_sync(0xffffffffu, w.cmax, o));
+          w.imin = max(w.imin, __shfl_xor_sync(0xffffffffu, w.imin, o));
+          w.imax = min(w.imax, __shfl_xor_sync(0xffffffffu, w.imax, o));
+        }
+        if (lane == 0) wr[h] = w;
       }
-      float g1 = -INFINITY, g2 = -INFINITY;
+      __syncwarp();
+      float g1[2] = {-INFINITY, -INFINITY}, g2[2] = {-INFINITY, -INFINITY};
       for (uint32_t i = 0; i < n_steps; i++, g++) {
-        const uint32_t as = g % kRjAccStages;
-        const uint32_t tstage = taddr + as * 2 * kRjCols;
-        ptx::mbar_wait(&sm.bar_accfull[as][h], (g / kRjAccStages) & 1);
-        ptx::tc_fence_after();
-        uint32_t r0[32], r1[32], r2[32], r3[32];
+        const uint32_t c0 = (step0 + i) * kRjCols + c * 128;
 #pragma unroll
-        for (int rd = 0; rd < kRjRounds; rd++) {
-          const uint32_t c0 = (step0 + i) * kRjCols + rd * 128;
-          const bool need = c0 < w.cmax && c0 + 128 > w.cmin;  // warp-uniform
+        for (int h = 0; h < 2; h++) {  // in the order the MMA warp fills the buffers
+          ptx::mbar_wait(&sm.bar_accfull[h], g & 1);
+          ptx::tc_fence_after();
+          const RjWarpRange w = wr[h];
+          const bool need = c0 < w.cmax && c0 + 128 > w.cmin;        // warp-uniform
+          const bool interior = c0 >= w.imin && c0 + 128 <= w.imax;  // warp-uniform: every row accepts the round
+          uint32_t r0[32], r1[32], r2[32], r3[32];
           if (need) {
-            ptx::tmem_ld32(r0, tstage + rd * 128);
-            ptx::tmem_ld32(r1, tstage + rd * 128 + 32);
-            ptx::tmem_ld32(r2, tstage + rd * 128 + 64);
-            ptx::tmem_ld32(r3, tstage + rd * 128 + 96);
+            const uint32_t t = taddr + h * kRjCols;
+            ptx::tmem_ld32(r0, t);
+            ptx::tmem_ld32(r1, t + 32);
+            ptx::tmem_ld32(r2, t + 64);
+            ptx::tmem_ld32(r3, t + 96);
             ptx::tmem_ld_wait(r0, r1, r2, r3);
           }
-          if (rd == kRjRounds - 1) {
-            // every column this warp needs is in registers: hand the stage back to the MMA warp
-            ptx::tc_fence_before();
-            __syncwarp();
-            if (lane == 0) ptx::mbar_arrive(&sm.bar_accempty[as][h]);
-          }
+          // every column this warp needs is in registers: hand the buffer back to the MMA warp before reducing
+          ptx::tc_fence_before();
+          __syncwarp();
+          if (lane == 0) ptx::mbar_arrive(&sm.bar_accempty[h]);
           if (need) {
-            rj_group(r0, c0, w, lo, width, g1, g2);
-            rj_group(r1, c0 + 32, w, lo, width, g1, g2);
-            rj_group(r2, c0 + 64, w, lo, width, g1, g2);
-            rj_group(r3, c0 + 96, w, lo, width, g1, g2);
+            if (interior) {
+              rj_round<false>(r0, r1, r2, r3, 0, 0, g1[h], g2[h]);
+            } else {
+              const uint2 bd = band[h * 128];
+              rj_round<true>(r0, r1, r2, r3, (int)(bd.x - c0), bd.y > bd.x ? (int)(bd.y - bd.x) : 0, g1[h], g2[h]);
+            }
           }
         }
       }
+      // the partner warp (q, 1 - c) has the other round of every step: pass it this warp's pairs for half 1 - c and
+      // take its pairs for half c (double-buffered by unit, so a partner already at the next unit end cannot
+      // overwrite a pair before it has been read)
+      const uint32_t row = c * 128 + q * 32 + lane, s = us.s0 + row;  // the row this thread tests
+      float2* part = sm.part[k & 1];
+      part[(c ^ 1) * 128 + q * 32 + lane] = c ? make_float2(g1[0], g2[0]) : make_float2(g1[1], g2[1]);
+      ptx::named_bar_sync(1 + q, 64);
+      const float2 o = part[row];
+      float t1 = c ? g1[1] : g1[0], t2 = c ? g2[1] : g2[0];
+      rj_top2(t1, t2, o.x, o.y);
       if (!us.skip && s < us.n_rows) {
         // a row with no gated-in column has nothing to emit; otherwise the certified test (g1 = a1, g2 <= a2)
         bool rejected = true;
+        const uint2 bd = sm.band[slot][row];
         // (K = 48: the bounds of rj_ksteps; K = 64: the offsets are 0 and a1, a2 are g1, g2)
-        if (valid && g1 > -INFINITY)
-          rejected = certified_reject(na, __fsub_ru(g1, us.noff1), __fsub_rd(g2, us.noff2), us.eps, thr, ratio);
+        if (bd.y > bd.x && t1 > -INFINITY)
+          rejected = certified_reject(sm.norm2[slot][row], __fsub_ru(t1, us.noff1), __fsub_rd(t2, us.noff2), us.eps, thr, ratio);
         const uint32_t row_off = us.row_off;
         rowstat[row_off + s] = rejected ? 1 : 0;
         if (!rejected) surv_rows[row_off + atomicAdd(surv_count + us.task, 1u)] = s;  // at most n_rows survivors
@@ -362,7 +399,7 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
   __syncthreads();
   if (warp == 0) {
     ptx::tc_fence_after();
-    ptx::tmem_dealloc<512>(tmem);
+    ptx::tmem_dealloc<512>(sm.tmem_base);  // (re-read: keeps the address out of the epilogue's registers)
   }
 }
 
