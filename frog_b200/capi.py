@@ -30,7 +30,9 @@ PUBLIC_SYMBOLS = [
     "fm_links_build", "fm_links_total", "fm_links_fetch", "fm_links_offsets", "fm_links_data", "fm_links_device_offsets",
     "fm_links_device_data", "fm_links_build_ms", "fm_links_free",
 ]
-DEBUG_SYMBOLS = ["fm_debug_image", "fm_debug_image_norms", "fm_debug_score_unit", "fm_debug_set_option"]
+DEBUG_SYMBOLS = ["fm_debug_image", "fm_debug_image_norms", "fm_debug_score_unit", "fm_debug_set_option",
+                 "fm_debug_reject_rows"]
+ERR_INVALID = -1  # FM_ERR_INVALID
 
 
 class Stats(C.Structure):
@@ -99,6 +101,7 @@ def load():
     L.fm_debug_image_norms.argtypes = [vp, C.c_uint32, f32p, f32p, f32p]
     L.fm_debug_score_unit.argtypes = [vp, C.c_uint32, C.c_uint32, C.c_uint32, vp, C.c_uint32, vp, vp, vp]
     L.fm_debug_set_option.argtypes = [C.c_char_p, C.c_int]
+    L.fm_debug_reject_rows.argtypes = [vp, C.c_uint32, C.c_uint32, vp, vp, vp, vp, u32p]
     L.fm_links_build.argtypes = [vp, vp, vp, vp, C.POINTER(vp)]
     L.fm_links_total.argtypes = [vp]
     L.fm_links_total.restype = C.c_uint64
@@ -329,6 +332,22 @@ class Matcher:
         self._check(self._L.fm_debug_score_unit(self._h, first_img, second_img, row_block, _ptr(t), ld,
                                                 _ptr(bands), _ptr(ct), _ptr(cc)))
         return dict(t=t, bands=bands, cand_t=ct, cand_col=cc)
+
+    def debug_reject_rows(self, task: int, n_rows: int):
+        """What the reject pass computed for task `task` (n_rows sorted rows) of the last match(), run with the
+        "reject_dump" option set: args [n,4] float32 (a1, a2, |a|^2, eps; NaN rows have no band), rowstat [n] uint8,
+        bands [n,2] uint32 and the ascending survivor list.  None (FM_ERR_INVALID) if the task did not go through
+        the reject pass, or n_rows is not its row count."""
+        args = np.zeros((max(n_rows, 1), 4), np.float32)
+        stat = np.zeros(max(n_rows, 1), np.uint8)
+        bands = np.zeros((max(n_rows, 1), 2), np.uint32)
+        surv = np.zeros(max(n_rows, 1), np.uint32)
+        ns = C.c_uint32()
+        rc = self._L.fm_debug_reject_rows(self._h, task, n_rows, _ptr(args), _ptr(stat), _ptr(bands), _ptr(surv), C.byref(ns))
+        if rc == ERR_INVALID:
+            return None
+        self._check(rc)
+        return dict(args=args[:n_rows], rowstat=stat[:n_rows], bands=bands[:n_rows], survivors=surv[:ns.value])
 
 
 def debug_set_option(name: str, value: int) -> None:

@@ -388,6 +388,8 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
     if (sym) add_task(pair_second[p], pair_first[p], kTaskSwap, p);
   }
   const uint32_t n_tasks = (uint32_t)tasks.size();
+  c->reject_rows.clear();
+  if (g_debug.reject_dump) c->reject_rows.resize(n_tasks);
 
   // ---- batches + prefix arrays (blocks of 128 rows, compaction chunks, score units) ------------
   uint64_t base_units = 0;
@@ -594,6 +596,8 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
         FastBatchArgs fa{};
         fa.images = d_images;
         fa.tasks = d_tasks + b.t0;
+        fa.h_tasks = tasks.data() + b.t0;
+        fa.task0 = b.t0;
         fa.n_tasks = nt;
         fa.rows = b.rows;
         fa.blk_off = blk;
@@ -935,6 +939,7 @@ int fm_debug_set_option(const char* name, int value) {
   else if (!strcmp(name, "two_phase")) g_debug.two_phase = value;
   else if (!strcmp(name, "surv_cap")) g_debug.surv_cap = value;
   else if (!strcmp(name, "compact_v")) g_debug.compact_v = value;
+  else if (!strcmp(name, "reject_dump")) g_debug.reject_dump = value;
   else return FM_ERR_INVALID;
   return FM_OK;
 }
@@ -1022,6 +1027,21 @@ int fm_debug_score_unit(fm_ctx* c, uint32_t first_img, uint32_t second_img, uint
     for (size_t i = 0; i < h.size(); i++) { cand_t[i] = h[i].t; cand_col[i] = h[i].col; }
   }
   d_task.release(); d_meta.release(); d_dump.release();
+  return FM_OK;
+}
+
+int fm_debug_reject_rows(fm_ctx* c, uint32_t task, uint32_t n_rows, float* args, uint8_t* rowstat, uint32_t* bands,
+                         uint32_t* survivors, uint32_t* n_survivors) {
+  if (!c) return FM_ERR_INVALID;
+  if (task >= c->reject_rows.size() || !c->reject_rows[task].valid)
+    return fail(c, FM_ERR_INVALID, "fm_debug_reject_rows: the task did not go through the reject pass of the last fm_match");
+  const fm_ctx::RejectRows& st = c->reject_rows[task];
+  if (n_rows != st.rowstat.size()) return fail(c, FM_ERR_INVALID, "fm_debug_reject_rows: n_rows is not the task's row count");
+  if (args && n_rows) memcpy(args, st.args.data(), (size_t)n_rows * sizeof(float4));
+  if (rowstat && n_rows) memcpy(rowstat, st.rowstat.data(), n_rows);
+  if (bands && n_rows) memcpy(bands, st.bands.data(), (size_t)n_rows * sizeof(uint2));
+  if (survivors && !st.survivors.empty()) memcpy(survivors, st.survivors.data(), st.survivors.size() * sizeof(uint32_t));
+  if (n_survivors) *n_survivors = (uint32_t)st.survivors.size();
   return FM_OK;
 }
 

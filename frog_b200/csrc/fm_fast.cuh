@@ -117,12 +117,15 @@ struct DebugOptions {
   int two_phase = -1;  // two-phase scoring: -1 = the library decides (fm_api.cu), 0 = never, 1 = whenever it is applicable
   int compact_v = 3;   // large-batch compaction (fm_compact.cuh): 3 = warp-autonomous pipelined count, 2 = pipelined count with the
                        // block-wide ranking, 1 = the first version (one CTA per chunk, scan with the per-pair counts)
+  int reject_dump = 0;  // two-phase scoring: 1 = keep every task's reject-pass output on the host (fm_debug_reject_rows)
 };
 inline DebugOptions g_debug;
 
 struct FastBatchArgs {
   const ImageDev* images;
   const Task* tasks;        // device, this batch
+  const Task* h_tasks;      // host copy of `tasks` (row_off set)
+  uint32_t task0;           // index of the batch's first task in the call
   uint32_t n_tasks;
   uint32_t rows;            // rows in the batch
   const uint32_t* blk_off;  // device: 128-row blocks per task (prefix)
@@ -136,6 +139,36 @@ struct FastBatchArgs {
   bool two_phase;  // reject pass + capture pass instead of the single pass (see score_kernel)
   DeviceCounters* counters;
 };
+
+// g_debug.reject_dump: copy what the reject pass left for each task of the batch -- its dump, rowstat, bands and
+// survivor list -- to c->reject_rows, before anything later in the batch changes rowstat.
+inline cudaError_t stash_reject_rows(fm_ctx* c, const FastBatchArgs& a, const float4* dump, const uint8_t* rowstat,
+                                     const uint32_t* surv_count, const uint32_t* surv_rows) {
+  std::vector<float4> h_dump(a.rows);
+  std::vector<uint8_t> h_stat(a.rows);
+  std::vector<uint2> h_bands(a.rows);
+  std::vector<uint32_t> h_count(a.n_tasks), h_surv(a.rows);
+  cudaError_t e;
+  if ((e = cudaStreamSynchronize(c->stream)) != cudaSuccess) return e;
+  if ((e = cudaMemcpy(h_dump.data(), dump, (size_t)a.rows * sizeof(float4), cudaMemcpyDeviceToHost)) != cudaSuccess) return e;
+  if ((e = cudaMemcpy(h_stat.data(), rowstat, a.rows, cudaMemcpyDeviceToHost)) != cudaSuccess) return e;
+  if ((e = cudaMemcpy(h_bands.data(), c->d_bands.p, (size_t)a.rows * sizeof(uint2), cudaMemcpyDeviceToHost)) != cudaSuccess) return e;
+  if ((e = cudaMemcpy(h_count.data(), surv_count, (size_t)a.n_tasks * sizeof(uint32_t), cudaMemcpyDeviceToHost)) != cudaSuccess) return e;
+  if ((e = cudaMemcpy(h_surv.data(), surv_rows, (size_t)a.rows * sizeof(uint32_t), cudaMemcpyDeviceToHost)) != cudaSuccess) return e;
+  for (uint32_t t = 0; t < a.n_tasks; t++) {
+    const Task& task = a.h_tasks[t];
+    if (task.flags & kTaskExact) continue;
+    const uint32_t n = c->images[task.row_img].n, r0 = task.row_off;
+    auto& st = c->reject_rows[a.task0 + t];
+    st.valid = true;
+    st.args.assign(h_dump.begin() + r0, h_dump.begin() + r0 + n);
+    st.rowstat.assign(h_stat.begin() + r0, h_stat.begin() + r0 + n);
+    st.bands.assign(h_bands.begin() + r0, h_bands.begin() + r0 + n);
+    st.survivors.assign(h_surv.begin() + r0, h_surv.begin() + r0 + std::min(h_count[t], n));
+    std::sort(st.survivors.begin(), st.survivors.end());  // the kernel appends in any order
+  }
+  return cudaSuccess;
+}
 
 inline cudaError_t fast_match_batch(fm_ctx* c, const FastBatchArgs& a) {
   cudaError_t e;
@@ -163,7 +196,8 @@ inline cudaError_t fast_match_batch(fm_ctx* c, const FastBatchArgs& a) {
     if ((e = prep(score_kernel<false, 2, 0>)) != cudaSuccess) return e;
     if ((e = prep(score_kernel<true, 0, 0>)) != cudaSuccess) return e;
     // the reject pass: one CTA per SM
-    if ((e = cudaFuncSetAttribute(reject_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRjSmemBytes)) != cudaSuccess) return e;
+    if ((e = cudaFuncSetAttribute(reject_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRjSmemBytes)) != cudaSuccess) return e;
+    if ((e = cudaFuncSetAttribute(reject_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRjSmemBytes)) != cudaSuccess) return e;
     c->score_attr_set = true;
   }
   bool two_phase_ran = false;
@@ -187,9 +221,22 @@ inline cudaError_t fast_match_batch(fm_ctx* c, const FastBatchArgs& a) {
       uint32_t* surv_rows = surv_off + a.n_tasks + 1;
       if ((e = cudaMemsetAsync(surv_count, 0, (size_t)a.n_tasks * sizeof(uint32_t), c->stream)) != cudaSuccess) return e;
       // persistent: one CTA per SM walks the units
-      reject_kernel<<<std::min<uint32_t>(a.units, (uint32_t)c->sm_count), kRjThreads, kRjSmemBytes, c->stream>>>(
-          a.images, a.tasks, a.unit_off, a.n_tasks, a.units, c->d_bands.as<uint2>(), &a.counters->scored_cols, a.thr,
-          a.ratio, rowstat, surv_count, surv_rows);
+      const uint32_t grid = std::min<uint32_t>(a.units, (uint32_t)c->sm_count);
+      if (g_debug.reject_dump) {
+        DevBuf dump;
+        if ((e = dump.ensure((size_t)a.rows * sizeof(float4))) != cudaSuccess) return e;
+        if ((e = cudaMemsetAsync(dump.p, 0xFF, (size_t)a.rows * sizeof(float4), c->stream)) != cudaSuccess) return e;
+        reject_kernel<true><<<grid, kRjThreads, kRjSmemBytes, c->stream>>>(
+            a.images, a.tasks, a.unit_off, a.n_tasks, a.units, c->d_bands.as<uint2>(), &a.counters->scored_cols, a.thr,
+            a.ratio, rowstat, surv_count, surv_rows, dump.as<float4>());
+        if ((e = cudaGetLastError()) == cudaSuccess) e = stash_reject_rows(c, a, dump.as<float4>(), rowstat, surv_count, surv_rows);
+        dump.release();
+        if (e != cudaSuccess) return e;
+      } else {
+        reject_kernel<false><<<grid, kRjThreads, kRjSmemBytes, c->stream>>>(
+            a.images, a.tasks, a.unit_off, a.n_tasks, a.units, c->d_bands.as<uint2>(), &a.counters->scored_cols, a.thr,
+            a.ratio, rowstat, surv_count, surv_rows, nullptr);
+      }
       surv_plan_kernel<<<1, 1024, 0, c->stream>>>(surv_count, a.n_tasks, surv_off, cap_units, a.tasks, surv_rows, rowstat,
                                                   c->d_redo.as<uint2>(), &a.counters->rescore.redo_rows);
       score_kernel<false, 0, 2><<<cap_units, kScoreThreads, kScoreSmemBytes, c->stream>>>(

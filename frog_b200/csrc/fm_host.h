@@ -132,6 +132,16 @@ struct fm_ctx {
   uint32_t compact_epoch = 0;  // tags the look-back status words of a one-pass compaction launch (fm_compact.cuh)
   fm::DevBuf d_bands, d_cands, d_redo, d_taskinfo;
   fm::DevBuf d_rowstat, d_surv;  // two-phase scoring: per-row rejection flags; survivor counts / unit prefix / lists
+  // fm_debug_set_option("reject_dump", 1): per task of the most recent fm_match, what its reject pass computed
+  // (fm_debug_reject_rows); `valid` is false for a task that did not go through the reject pass
+  struct RejectRows {
+    bool valid = false;
+    std::vector<float4> args;        // per sorted row: certified_reject's (a1, a2, |a|^2, eps), NaNs for a row without a band
+    std::vector<uint8_t> rowstat;    // 1 = rejected
+    std::vector<uint2> bands;        // gate band [x, y) of sorted columns
+    std::vector<uint32_t> survivors;  // sorted positions of the surviving rows, ascending
+  };
+  std::vector<RejectRows> reject_rows;
   // Fraction of tensor-path rows the certified rejection test threw out in the most recent finished call with
   // -d2 < 1 (-1: unknown).  At >= kTwoPhaseMin the next such call scores in two phases from its first batch on.
   double reject_hint = -1.0;

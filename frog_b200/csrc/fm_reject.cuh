@@ -145,11 +145,14 @@ __device__ __forceinline__ void rj_round(const uint32_t (&r0)[32], const uint32_
 // units = unit_off[n_tasks] (segs = 1).  scored_cols += (row, column) scores the tensor cores computed: 128 x N per
 // MMA chain issued, band-edge and 16-column round-out columns included.  Writes rowstat[row] (1 = rejected) for every row of every fast task and
 // appends the sorted position of each surviving row to its task's survivor list (surv_count / surv_rows, any order).
+// kDump (test hook fm_debug_reject_rows): also writes dump[row] = (a1, a2, |a|^2, eps), the arguments the row's
+// certified_reject receives, for every row with a non-empty band, and NaNs for every other row of a fast task.
+template <bool kDump>
 __global__ void __launch_bounds__(kRjThreads, 1)
 reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ tasks, const uint32_t* __restrict__ unit_off,
               uint32_t n_tasks, uint32_t units, const uint2* __restrict__ bands, unsigned long long* __restrict__ scored_cols,
               float thr, float ratio, uint8_t* __restrict__ rowstat, uint32_t* __restrict__ surv_count,
-              uint32_t* __restrict__ surv_rows) {
+              uint32_t* __restrict__ surv_rows, float4* __restrict__ dump) {
   extern __shared__ uint8_t smem_raw[];
   RejectSmem& sm = *reinterpret_cast<RejectSmem*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -387,6 +390,9 @@ reject_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ task
         // (K = 48: the bounds of rj_ksteps; K = 64: the offsets are 0 and a1, a2 are g1, g2)
         if (bd.y > bd.x && t1 > -INFINITY)
           rejected = certified_reject(sm.norm2[slot][row], __fsub_ru(t1, us.noff1), __fsub_rd(t2, us.noff2), us.eps, thr, ratio);
+        if constexpr (kDump)
+          dump[us.row_off + s] = bd.y > bd.x ? make_float4(__fsub_ru(t1, us.noff1), __fsub_rd(t2, us.noff2), sm.norm2[slot][row], us.eps)
+                                             : make_float4(NAN, NAN, NAN, NAN);
         const uint32_t row_off = us.row_off;
         rowstat[row_off + s] = rejected ? 1 : 0;
         if (!rejected) surv_rows[row_off + atomicAdd(surv_count + us.task, 1u)] = s;  // at most n_rows survivors

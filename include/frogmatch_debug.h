@@ -1,7 +1,8 @@
 /*
  * frogmatch_debug.h -- test hooks of libfrogmatch.so.  NOT part of the drop-in boundary: these
  * exist so tests/ can check each device stage (sort + class table, FP16 operand packing, the
- * tcgen05 score tile, gate bands, candidate capture) against numpy in isolation.
+ * tcgen05 score tile, gate bands, candidate capture, the reject pass's per-row bounds) against numpy
+ * in isolation.
  */
 #ifndef FROGMATCH_DEBUG_H_
 #define FROGMATCH_DEBUG_H_
@@ -42,6 +43,23 @@ int fm_debug_score_unit(fm_ctx* ctx, uint32_t first_img, uint32_t second_img, ui
                         uint32_t ld, uint32_t* bands_out, float* cand_t, uint32_t* cand_col);
 
 /*
+ * What the reject pass of two-phase scoring computed for one task of the most recent fm_match, which must have run
+ * with the option "reject_dump" set.  Task p is pair p; with FM_FLAG_SYM pair p is tasks 2p and 2p + 1.  Rows are
+ * the sorted positions of the task's row image (image `second`, or `first` for task 2p + 1), n_rows of them.  Any
+ * output pointer may be NULL.
+ *   args       : n_rows x 4 floats, the arguments of the row's certified rejection test -- a1 (>= the best score),
+ *                a2 (<= the second best score), the row's |a|^2 and the task's eps -- or 4 NaNs for a row whose
+ *                gate band is empty
+ *   rowstat    : n_rows bytes, 1 = rejected
+ *   bands      : n_rows x 2 uint32 (lo, hi) interval of gated-in sorted columns
+ *   survivors  : sorted positions of the rows that survived, ascending (room for n_rows); *n_survivors of them
+ * Returns FM_ERR_INVALID for a task that did not go through the reject pass (exact-flagged, or the call scored in
+ * a single pass) and for an n_rows that is not the task's row count.
+ */
+int fm_debug_reject_rows(fm_ctx* ctx, uint32_t task, uint32_t n_rows, float* args, uint8_t* rowstat, uint32_t* bands,
+                         uint32_t* survivors, uint32_t* n_survivors);
+
+/*
  * Experiment switches for kernel studies (process-wide; the defaults are the production configuration):
  *   "probe"     1 | 2   timing-attribution builds of the scoring kernel -- results are GARBAGE
  *   "variant"   n       experiment builds of the scoring kernel -- results stay exact
@@ -50,6 +68,8 @@ int fm_debug_score_unit(fm_ctx* ctx, uint32_t first_img, uint32_t second_img, ui
  *                       -- results are exact either way
  *   "surv_cap"  n       survivor units the capture pass may use per batch (-1 = built-in); a small value forces the
  *                       overflow route (surplus survivors go to the exact row kernel)
+ *   "reject_dump" 0|1   two-phase scoring: keep what the reject pass computed for fm_debug_reject_rows (a dump build
+ *                       of the reject kernel and a synchronisation per batch) -- results stay exact
  * Returns FM_ERR_INVALID for an unknown name.  Nothing reads environment variables.
  */
 int fm_debug_set_option(const char* name, int value);

@@ -90,3 +90,47 @@ def random_group(kind, n_images, n_points, seed0=0):
     from frog_b200 import synth
     kps = [synth.make(kind, n_points, seed0 + i) for i in range(n_images)]
     return [(k.desc, k.scale, k.lap) for k in kps]
+
+
+# ---- the gate replayed in the library's sorted order (tensor-core path, fm_score.cuh bands_kernel) ----------------
+
+def sorted_view(img):
+    """(scale, laplacian) in the library's sorted order: by the laplacian's top 16 pattern bits, then by scale."""
+    _, s, l = img
+    l = np.where(l == 0, np.float32(0), l).astype(np.float32)
+    order = np.lexsort((s.view(np.uint32), l.view(np.uint32) >> 16))
+    return s[order], l[order]
+
+
+def first_true(pred, lo, hi):
+    """Per entry, the first index in [lo, hi) at which the monotone predicate holds (hi if none): binary search."""
+    lo, hi = lo.copy(), hi.copy()
+    while np.any(lo < hi):
+        act = lo < hi
+        m = (lo + hi) >> 1
+        p = pred(np.where(act, m, 0)) & act
+        lo = np.where(act & ~p, m + 1, lo)
+        hi = np.where(p, m, hi)
+    return lo
+
+
+def gate_bands(col, row):
+    """The reference's gates (match.cpp:270-275) as sorted column intervals [lo, hi) per sorted row."""
+    sc, lc = sorted_view(col)
+    sr, lr = sorted_view(row)
+    lo = np.zeros(sr.shape[0], np.int64)
+    hi = np.zeros(sr.shape[0], np.int64)
+    for lap in np.unique(lr):
+        rows = np.nonzero(lr == lap)[0]
+        cls = np.nonzero(lc == lap)[0]
+        if cls.size == 0:
+            continue
+        beg, end = int(cls[0]), int(cls[-1]) + 1
+        x = sr[rows]
+        b = np.full(rows.size, beg, np.int64)
+        e = np.full(rows.size, end, np.int64)
+        # float32 quotients compared with 1.3 (the reference's `float / float > 1.3`)
+        l0 = first_true(lambda m: ~((x / sc[m]).astype(np.float64) > 1.3), b, e)
+        h0 = first_true(lambda m: (sc[m] / x).astype(np.float64) > 1.3, l0, e)
+        lo[rows], hi[rows] = l0, np.maximum(h0, l0)
+    return lo, hi

@@ -7,6 +7,7 @@ checked against the band arithmetic replayed in numpy with the reference's gate 
 import numpy as np
 import pytest
 
+import helpers
 from frog_b200 import capi, synth
 from oracle import oracle as O
 
@@ -144,52 +145,10 @@ def test_reject_trim_edges(kind, rat, oracle_lib):
 
 # ---- issued-work accounting ------------------------------------------------------------------------------------
 
-def _sorted_view(img):
-    """(scale, laplacian) in the library's sorted order: by the laplacian's top 16 pattern bits, then by scale."""
-    _, s, l = img
-    l = np.where(l == 0, np.float32(0), l).astype(np.float32)
-    order = np.lexsort((s.view(np.uint32), l.view(np.uint32) >> 16))
-    return s[order], l[order]
-
-
-def _first_true(pred, lo, hi):
-    """Per entry, the first index in [lo, hi) at which the monotone predicate holds (hi if none): binary search."""
-    lo, hi = lo.copy(), hi.copy()
-    while np.any(lo < hi):
-        act = lo < hi
-        m = (lo + hi) >> 1
-        p = pred(np.where(act, m, 0)) & act
-        lo = np.where(act & ~p, m + 1, lo)
-        hi = np.where(p, m, hi)
-    return lo
-
-
-def _bands(col, row):
-    """The reference's gates (match.cpp:270-275) as sorted column intervals [lo, hi) per sorted row."""
-    sc, lc = _sorted_view(col)
-    sr, lr = _sorted_view(row)
-    lo = np.zeros(sr.shape[0], np.int64)
-    hi = np.zeros(sr.shape[0], np.int64)
-    for lap in np.unique(lr):
-        rows = np.nonzero(lr == lap)[0]
-        cls = np.nonzero(lc == lap)[0]
-        if cls.size == 0:
-            continue
-        beg, end = int(cls[0]), int(cls[-1]) + 1
-        x = sr[rows]
-        b = np.full(rows.size, beg, np.int64)
-        e = np.full(rows.size, end, np.int64)
-        # float32 quotients compared with 1.3 (the reference's `float / float > 1.3`)
-        l0 = _first_true(lambda m: ~((x / sc[m]).astype(np.float64) > 1.3), b, e)
-        h0 = _first_true(lambda m: (sc[m] / x).astype(np.float64) > 1.3, l0, e)
-        lo[rows], hi[rows] = l0, np.maximum(h0, l0)
-    return lo, hi
-
-
 def _issued(col, row):
     """Scores the reject pass issues for one task: per 256-row unit and row half, 128 x N per 256-column step the
     half's band union meets, N = the step's part of the union rounded out to 16 columns."""
-    lo, hi = _bands(col, row)
+    lo, hi = helpers.gate_bands(col, row)
     total = 0
     for s0 in range(0, lo.shape[0], 256):
         for h in range(2):
