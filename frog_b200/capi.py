@@ -31,7 +31,7 @@ PUBLIC_SYMBOLS = [
     "fm_links_device_data", "fm_links_build_ms", "fm_links_free",
 ]
 DEBUG_SYMBOLS = ["fm_debug_image", "fm_debug_image_norms", "fm_debug_score_unit", "fm_debug_set_option",
-                 "fm_debug_reject_rows"]
+                 "fm_debug_reject_rows", "fm_debug_wide_unit"]
 ERR_INVALID = -1  # FM_ERR_INVALID
 
 
@@ -102,6 +102,7 @@ def load():
     L.fm_debug_score_unit.argtypes = [vp, C.c_uint32, C.c_uint32, C.c_uint32, vp, C.c_uint32, vp, vp, vp]
     L.fm_debug_set_option.argtypes = [C.c_char_p, C.c_int]
     L.fm_debug_reject_rows.argtypes = [vp, C.c_uint32, C.c_uint32, vp, vp, vp, vp, u32p]
+    L.fm_debug_wide_unit.argtypes = [vp, C.c_uint32, C.c_uint32, C.c_uint32, vp, C.c_uint32, vp, vp, vp, f32p, u32p]
     L.fm_links_build.argtypes = [vp, vp, vp, vp, C.POINTER(vp)]
     L.fm_links_total.argtypes = [vp]
     L.fm_links_total.restype = C.c_uint64
@@ -332,6 +333,21 @@ class Matcher:
         self._check(self._L.fm_debug_score_unit(self._h, first_img, second_img, row_block, _ptr(t), ld,
                                                 _ptr(bands), _ptr(ct), _ptr(cc)))
         return dict(t=t, bands=bands, cand_t=ct, cand_col=cc)
+
+    def debug_wide_unit(self, first_img: int, second_img: int, row_block: int, n_first: int, n_second: int) -> dict:
+        """One 128-row unit of the wide scoring kernel (d != 48) in dump mode: t [128, n_pad(first)] float32 scores of
+        the columns its MMAs computed (NaN elsewhere), bands [rows, 2], the 8-entry candidate lists cand_t / cand_col
+        [rows, 8], the task's eps and K_pad."""
+        ld = (n_first + 255) & ~255
+        t = np.zeros((128, max(ld, 1)), np.float32)
+        nr = min(128, n_second - row_block * 128)
+        bands = np.zeros((nr, 2), np.uint32)
+        ct = np.zeros((nr, 8), np.float32)
+        cc = np.zeros((nr, 8), np.uint32)
+        eps, kpad = C.c_float(), C.c_uint32()
+        self._check(self._L.fm_debug_wide_unit(self._h, first_img, second_img, row_block, _ptr(t), ld, _ptr(bands),
+                                               _ptr(ct), _ptr(cc), C.byref(eps), C.byref(kpad)))
+        return dict(t=t, bands=bands, cand_t=ct, cand_col=cc, eps=eps.value, k_pad=kpad.value)
 
     def debug_reject_rows(self, task: int, n_rows: int):
         """What the reject pass computed for task `task` (n_rows sorted rows) of the last match(), run with the

@@ -13,6 +13,7 @@
 #include "fm_generic.cuh"
 #include "fm_host.h"
 #include "fm_links.cuh"
+#include "fm_wide.cuh"
 
 using namespace fm;
 
@@ -22,6 +23,7 @@ struct fm_result {
   uint64_t total = 0;
   uint32_t flags = 0;
   float ratio = 1.f;
+  bool d48 = false;  // a d = 48 call: only these feed the two-phase hint (reject_hint)
   std::vector<uint32_t> counts;
   std::vector<uint64_t> offsets;
   DevBuf d_out, d_counts, d_dist;
@@ -158,7 +160,7 @@ int finalize(fm_result* r) {
   r->stats.scored_pairs = hc->scored_cols;
   r->stats.candidates = hc->rescore.candidates;
   r->stats.rows_rejected_early = hc->rescore.rejected_early;
-  if (r->ratio < 1.f && r->stats.rows > r->stats.rows_exact)
+  if (r->ratio < 1.f && r->d48 && r->stats.rows > r->stats.rows_exact)
     c->reject_hint = (double)hc->rescore.rejected_early / (double)(r->stats.rows - r->stats.rows_exact);
   r->stats.rows_exact += hc->redo_total;
   float acc[kNumPhases] = {0};
@@ -303,12 +305,15 @@ int fm_upload_image(fm_ctx* c, uint32_t img, const float* desc, const float* sca
   if (img >= c->images.size()) c->images.resize(img + 1);
   if (img >= c->h_images.size()) c->h_images.resize(img + 1, ImageDev{});
   Image& im = c->images[img];
-  // One slab per image: desc | scale | lap | perm | scale_sorted | norm2_sorted | rowop | colop (1 KB aligned pieces).
+  // One slab per image: desc | scale | lap | perm | scale_sorted | norm2_sorted | rowop | colop | wideop (1 KB aligned pieces).
   auto pad = [](size_t x) { return (x + 1023) & ~(size_t)1023; };
   const uint32_t n_pad = (n + 255u) & ~255u;  // rows are consumed 256 at a time, columns 64
   const size_t b_desc = pad((size_t)n * d * sizeof(float)), b_vec = pad((size_t)std::max(n, 1u) * sizeof(float));
   const size_t b_op = d == (uint32_t)kD ? pad((size_t)n_pad * kKPad * sizeof(__half)) : 0;
-  const size_t need = b_desc + 5 * b_vec + 2 * b_op + 1024;
+  // d != 48: one operand image of wide_kpad(d) halves per keypoint (fm_wide.cuh); longer descriptors have none
+  const bool wide = d != (uint32_t)kD && d <= (uint32_t)kWideMaxD;
+  const size_t b_wide = wide ? pad((size_t)n_pad * wide_kpad(d) * sizeof(__half)) : 0;
+  const size_t need = b_desc + 5 * b_vec + 2 * b_op + b_wide + 1024;
   if (!im.slab || im.slab_bytes < need) {  // a re-upload that fits reuses the image's slab
     void* p = nullptr;
     FM_CUDA(c, c->arena.alloc(need, &p));
@@ -340,6 +345,7 @@ int fm_upload_image(fm_ctx* c, uint32_t img, const float* desc, const float* sca
   v.norm2_sorted = reinterpret_cast<float*>(base + b_desc + 4 * b_vec);
   v.rowop = b_op ? reinterpret_cast<__half*>(base + b_desc + 5 * b_vec) : nullptr;
   v.colop = b_op ? reinterpret_cast<__half*>(base + b_desc + 5 * b_vec + b_op) : nullptr;
+  v.wideop = wide ? reinterpret_cast<__half*>(base + b_desc + 5 * b_vec + 2 * b_op) : nullptr;
   {
     cudaError_t e = ensure_metas(c, (uint32_t)c->h_images.size());
     if (e != cudaSuccess) return cuda_fail(c, e, "fm_upload_image");
@@ -369,7 +375,9 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
   if (rc != FM_OK) return rc;
   const bool sym = flags & FM_FLAG_SYM;
   const bool match_all = flags & FM_FLAG_MATCH_ALL;
-  const bool force_exact = (flags & FM_FLAG_FORCE_EXACT) || c->dim != (uint32_t)kD;
+  const bool force_exact = (flags & FM_FLAG_FORCE_EXACT) != 0;
+  // d != 48: the wide tensor-core path (fm_wide.cuh); images it cannot take (kImgBadDim and the other flags) are exact
+  const bool wide = c->dim != (uint32_t)kD;
 
   // ---- tasks --------------------------------------------------------------------------------
   std::vector<Task> tasks;
@@ -396,7 +404,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
   for (auto& t : tasks)
     if (!(t.flags & kTaskExact)) base_units += (c->images[t.row_img].n + kUnitRows - 1) / kUnitRows;
   uint32_t segs = 1;
-  if (base_units > 0 && base_units < (uint64_t)2 * c->sm_count)
+  if (!wide && base_units > 0 && base_units < (uint64_t)2 * c->sm_count)  // (the wide path scores whole rows: segs = 1)
     segs = (uint32_t)std::min<uint64_t>(8, ((uint64_t)2 * c->sm_count + base_units - 1) / base_units);
   if (match_all && total_rows > 0xFFFFFFF0ull) return fail(c, FM_ERR_UNSUPPORTED, "fm_match: -all supports at most 2^32 outer-loop rows per call");
   const uint32_t kMaxBatchRows = match_all ? 0xFFFFFFF0u : (24u << 20);  // -all: one batch (its scan spans all rows)
@@ -435,6 +443,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
   r->n_pairs = n_pairs;
   r->flags = flags;
   r->ratio = dist2second;
+  r->d48 = !wide;
   r->d_out = take_buf(c->out_free, std::max<uint64_t>(total_rows, 1) * sizeof(uint2));
   r->d_counts = take_buf(c->counts_free, std::max<size_t>(n_pairs, 1) * sizeof(uint32_t));
   const bool want_dist = (flags & FM_FLAG_DISTANCES) && !match_all;
@@ -579,7 +588,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
     // call of this kind on this context rejected >= 99 % of its rows, or, inside a synchronous multi-batch call, once
     // the first batch (single pass) has shown that much.
     constexpr double kTwoPhaseMin = 0.99;
-    const bool two_phase_possible = dist2second < 1.f && segs == 1 && !force_exact;
+    const bool two_phase_possible = dist2second < 1.f && segs == 1 && !force_exact && !wide;  // reject pass: K = 64 only
     bool two_phase = two_phase_possible && c->reject_hint >= kTwoPhaseMin;
     bool probed = false;
     if (g_debug.two_phase >= 0) {  // test hook: force the choice
@@ -611,7 +620,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
         fa.rowdist = d_rowdist;
         fa.two_phase = two_phase;
         fa.counters = d_counters;
-        cudaError_t e = fast_match_batch(c, fa);
+        cudaError_t e = wide ? wide_match_batch(c, fa) : fast_match_batch(c, fa);
         if (e != cudaSuccess) {
           int code = cuda_fail(c, e, "fm_match: tensor-core path");
           fm_result_free(r);
@@ -1027,6 +1036,54 @@ int fm_debug_score_unit(fm_ctx* c, uint32_t first_img, uint32_t second_img, uint
     for (size_t i = 0; i < h.size(); i++) { cand_t[i] = h[i].t; cand_col[i] = h[i].col; }
   }
   d_task.release(); d_meta.release(); d_dump.release();
+  return FM_OK;
+}
+
+int fm_debug_wide_unit(fm_ctx* c, uint32_t first_img, uint32_t second_img, uint32_t row_block, float* t_out, uint32_t ld,
+                       uint32_t* bands_out, float* cand_t, uint32_t* cand_col, float* eps_out, uint32_t* k_pad_out) {
+  if (!c || first_img >= c->images.size() || second_img >= c->images.size() || !c->images[first_img].valid ||
+      !c->images[second_img].valid)
+    return FM_ERR_INVALID;
+  if (c->dim == (uint32_t)kD || c->dim > (uint32_t)kWideMaxD)
+    return fail(c, FM_ERR_INVALID, "fm_debug_wide_unit: the wide path takes descriptor lengths d != 48, d <= 4096");
+  FM_CUDA(c, cudaSetDevice(c->device));
+  int rc = sync_images(c);
+  if (rc != FM_OK) return rc;
+  const uint32_t nB = c->images[second_img].n;
+  const uint32_t n_pad_a = c->h_images[first_img].n_pad;
+  if (row_block * kWdRows >= nB || ld < n_pad_a) return fail(c, FM_ERR_INVALID, "fm_debug_wide_unit: bad row block or ld");
+  Task task{first_img, second_img, 0, 0};
+  const uint32_t blocks = (nB + kWdRows - 1) / kWdRows;
+  uint32_t meta[2] = {0, blocks};
+  DevBuf d_task, d_meta, d_dump, d_eps;
+  FM_CUDA(c, d_task.ensure(sizeof task));
+  FM_CUDA(c, d_meta.ensure(sizeof meta));
+  FM_CUDA(c, d_dump.ensure((size_t)kWdRows * ld * sizeof(float)));
+  FM_CUDA(c, d_eps.ensure(sizeof(float)));
+  FM_CUDA(c, c->d_bands.ensure((size_t)nB * sizeof(uint2)));
+  FM_CUDA(c, c->d_cands.ensure((size_t)nB * kTopK * sizeof(Cand)));
+  FM_CUDA(c, cudaMemcpyAsync(d_task.p, &task, sizeof task, cudaMemcpyHostToDevice, c->stream));
+  FM_CUDA(c, cudaMemcpyAsync(d_meta.p, meta, sizeof meta, cudaMemcpyHostToDevice, c->stream));
+  FM_CUDA(c, cudaMemsetAsync(d_dump.p, 0xFF, (size_t)kWdRows * ld * sizeof(float), c->stream));  // NaN = "not computed"
+  FM_CUDA(c, cudaFuncSetAttribute(wide_score_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWdSmemBytes));
+  bands_kernel<<<blocks, 128, 0, c->stream>>>(c->d_images.as<ImageDev>(), d_task.as<Task>(), d_meta.as<uint32_t>(), 1,
+                                              c->d_bands.as<uint2>());
+  wide_score_kernel<true><<<1, kWdThreads, kWdSmemBytes, c->stream>>>(
+      c->d_images.as<ImageDev>(), d_task.as<Task>(), d_meta.as<uint32_t>(), 1, row_block, row_block + 1, c->d_bands.as<uint2>(),
+      c->d_cands.as<Cand>(), nullptr, d_dump.as<float>(), ld, d_eps.as<float>());
+  FM_CUDA(c, cudaGetLastError());
+  FM_CUDA(c, cudaStreamSynchronize(c->stream));
+  const uint32_t r0 = row_block * kWdRows, nr = std::min<uint32_t>(kWdRows, nB - r0);
+  if (t_out) FM_CUDA(c, cudaMemcpy(t_out, d_dump.p, (size_t)kWdRows * ld * sizeof(float), cudaMemcpyDeviceToHost));
+  if (bands_out) FM_CUDA(c, cudaMemcpy(bands_out, c->d_bands.as<uint2>() + r0, (size_t)nr * sizeof(uint2), cudaMemcpyDeviceToHost));
+  if (cand_t && cand_col) {
+    std::vector<Cand> h((size_t)nr * kTopK);
+    FM_CUDA(c, cudaMemcpy(h.data(), c->d_cands.as<Cand>() + (size_t)r0 * kTopK, h.size() * sizeof(Cand), cudaMemcpyDeviceToHost));
+    for (size_t i = 0; i < h.size(); i++) { cand_t[i] = h[i].t; cand_col[i] = h[i].col; }
+  }
+  if (eps_out) FM_CUDA(c, cudaMemcpy(eps_out, d_eps.p, sizeof(float), cudaMemcpyDeviceToHost));
+  if (k_pad_out) *k_pad_out = wide_kpad(c->dim);
+  d_task.release(); d_meta.release(); d_dump.release(); d_eps.release();
   return FM_OK;
 }
 

@@ -14,13 +14,14 @@ constexpr uint32_t kTaskExact = 2u;      // Task::flags: task must use the exact
 constexpr int kD = 48;                   // SURF3D descriptor length the tensor-core path is built for
 constexpr int kKPad = 64;                // K after augmentation: 48 descriptor + norm/one slots, 4 x UMMA_K
 constexpr int kMaxClasses = 8;           // distinct Laplacian-sign values per image on the fast path
+constexpr int kWideMaxD = 4096;          // longest descriptor the wide tensor-core path (fm_wide.cuh) takes, d != 48
 
 // Image flags (set by the prep kernel; any non-zero value routes the image to the exact kernel).
 constexpr uint32_t kImgNotFinite = 1u;    // NaN/Inf in descriptors, scales or laplacians
 constexpr uint32_t kImgBadScale = 2u;     // scale <= 0: scale gate no longer an interval in sorted order
 constexpr uint32_t kImgBigNorm = 4u;      // |desc| outside the range the FP16 operands are certified for
 constexpr uint32_t kImgManyClasses = 8u;  // more than kMaxClasses distinct laplacian values
-constexpr uint32_t kImgBadDim = 16u;      // d != 48
+constexpr uint32_t kImgBadDim = 16u;      // d > kWideMaxD: no tensor-core path for this length
 
 // Per-image statistics / class table produced on the device by the prep kernels.
 struct ImageMeta {
@@ -58,7 +59,13 @@ struct ImageDev {
                         //          columns 0..47 = fp16(desc), 48,49 = 1, rest 0 (this image as rows)
   const __half* colop;  // same tiling; columns 48,49 = hi/lo halves of -|desc|^2/2 (image as columns)
   const ImageMeta* meta;
+  const __half* wideop;  // (sorted) d != 48, d <= kWideMaxD only: [n_pad/128 tiles][wide_kpad(d)/64 k-blocks] of the
+                         //          same 128 x 64-half SWIZZLE_128B tiles, fp16(desc) in slots 0..d-1, zeros after;
+                         //          one operand for both roles (the norm term is added in the wide epilogue)
 };
+
+// K of the wide path: the descriptor length rounded up to whole 64-value k-blocks.
+__host__ __device__ __forceinline__ uint32_t wide_kpad(uint32_t d) { return (d + 63u) & ~63u; }
 
 // Byte offset of (row r, 16-byte chunk q) inside a 128 x 128 B SWIZZLE_128B K-major tile:
 // 8-row x 128 B atoms, chunk index XORed with (row mod 8)  [cute Swizzle<3,4,3>].

@@ -56,15 +56,20 @@ inline cudaError_t fast_prepare_dirty(fm_ctx* c) {
   c->dirty.erase(std::unique(c->dirty.begin(), c->dirty.end()), c->dirty.end());
   std::vector<PrepSeg> segs;
   uint32_t off = 0, blk_keys = 0, blk_pack = 0;
+  bool wide = false;  // the images carry the wide operand (d != 48): prep_wide_pack_kernel instead of prep_pack_kernel
   for (uint32_t img : c->dirty) {
     if (img >= c->images.size() || !c->images[img].valid) continue;
     const uint32_t n = c->images[img].n;
+    const ImageDev& v = c->h_images[img];
     PrepSeg sg{};
     sg.img = img; sg.n = n; sg.off = off; sg.blk_keys = blk_keys; sg.blk_pack = blk_pack;
     segs.push_back(sg);
     off += n;
     blk_keys += (n + 255) / 256;
-    blk_pack += (c->h_images[img].n_pad * 8 + 255) / 256;
+    if (v.wideop) wide = true;
+    // 16-byte chunks per sorted keypoint: 8 of the K = 64 operands, wide_kpad(d) / 8 of the wide operand
+    const uint64_t chunks = (uint64_t)v.n_pad * (v.wideop ? wide_kpad(v.d) / 8u : 8u);
+    blk_pack += (uint32_t)((chunks + 255) / 256);
   }
   c->dirty.clear();
   if (segs.empty()) return cudaSuccess;
@@ -103,7 +108,8 @@ inline cudaError_t fast_prepare_dirty(fm_ctx* c) {
   }
   prep_finish_kernel<<<n_segs, 1024, 0, c->stream>>>(d_images, d_segs, d_metas, keys_sorted, c->s_idx_sorted.as<uint32_t>(),
                                                      c->s_norm2.as<float>());
-  if (blk_pack) prep_pack_kernel<<<blk_pack, 256, 0, c->stream>>>(d_images, d_segs, n_segs, c->s_norm2.as<float>());
+  if (blk_pack && wide) prep_wide_pack_kernel<<<blk_pack, 256, 0, c->stream>>>(d_images, d_segs, n_segs);
+  else if (blk_pack) prep_pack_kernel<<<blk_pack, 256, 0, c->stream>>>(d_images, d_segs, n_segs, c->s_norm2.as<float>());
   return cudaGetLastError();
 }
 

@@ -158,5 +158,6 @@ struct fm_ctx {
   float ms_prep_acc = 0.f;  // CUDA-event time of the preparation batches since the last fm_clear_images
   fm_stats stats{};
   bool score_attr_set = false;
+  bool wide_attr_set = false;  // shared-memory attribute of wide_score_kernel (fm_wide.cuh) set
   std::string err;
 };

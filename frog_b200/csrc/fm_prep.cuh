@@ -9,6 +9,8 @@
 //     tile layout tcgen05.mma reads, so one 16 KB cp.async.bulk lands a ready tile in shared memory.
 //     K is padded 48 -> 64: slots 48,49 carry (1, 1) on the row side and the hi/lo FP16 halves of
 //     -|b|^2/2 on the column side, so the MMA itself yields  t = a.b - |b|^2/2  = (|a|^2 - d^2)/2.
+//   * for d != 48 (d <= kWideMaxD) instead ONE operand image `wideop` of K_pad = wide_kpad(d) slots, fp16(desc) and
+//     zeros, in k-blocks of the same tiles (fm_wide.cuh adds the norm term in its epilogue).
 //   * per-image flags + max squared norm (certification inputs for the FP32 rescoring) and min squared
 //     norm (the reject pass drops the norm slots for column images whose norms barely vary, fm_reject.cuh).
 #pragma once
@@ -147,7 +149,7 @@ prep_finish_kernel(const ImageDev* __restrict__ images, const PrepSeg* __restric
   if (threadIdx.x == 0) {
     uint32_t cnt = s_cnt;
     uint32_t flags = 0;
-    if (im.d != (uint32_t)kD) flags |= kImgBadDim;
+    if (im.d > (uint32_t)kWideMaxD) flags |= kImgBadDim;
     if (cnt > kMaxClasses || s_collide) { flags |= kImgManyClasses; cnt = min(cnt, (uint32_t)kMaxClasses); }
     for (uint32_t a = 1; a < cnt; a++) {  // insertion sort of <= 8 boundaries
       uint32_t v = s_pos[a];
@@ -211,6 +213,37 @@ prep_pack_kernel(const ImageDev* __restrict__ images, const PrepSeg* __restrict_
   const size_t off = (size_t)(s >> 7) * 16384u + sw128_offset(s & 127u, q);
   *reinterpret_cast<uint4*>(rowop + off) = *reinterpret_cast<const uint4*>(h);
   *reinterpret_cast<uint4*>(colop + off) = *reinterpret_cast<const uint4*>(hc);
+}
+
+// Wide path (d != 48, fm_wide.cuh): one thread per (sorted keypoint, 16-byte chunk of its K_pad halves), the image's
+// single FP16 operand.  Tile (s / 128, k-block kb) is 16 KB at ((s / 128) * kblocks + kb) * 16 KB, so the row tile or
+// one column tile of a k-block is one contiguous cp.async.bulk.  A descriptor row is d floats: unless d is a multiple of
+// 4 its rows are not 16-byte aligned, so the eight values are read with scalar loads (consecutive threads read
+// consecutive chunks of one row: the loads still coalesce).
+__global__ void __launch_bounds__(256)
+prep_wide_pack_kernel(const ImageDev* __restrict__ images, const PrepSeg* __restrict__ segs, uint32_t n_segs) {
+  const uint32_t sg = prep_find(segs, n_segs, blockIdx.x, true);
+  const PrepSeg seg = segs[sg];
+  const ImageDev im = images[seg.img];
+  if (im.wideop == nullptr) return;
+  const uint32_t d = im.d, chunks = wide_kpad(d) / 8u;
+  const uint32_t g = (blockIdx.x - seg.blk_pack) * blockDim.x + threadIdx.x;
+  const uint32_t s = g / chunks, c = g - s * chunks;
+  if (s >= im.n_pad) return;
+  __align__(16) __half h[8];
+#pragma unroll
+  for (int k = 0; k < 8; k++) h[k] = __float2half_rn(0.f);
+  if (s < seg.n) {
+    const float* __restrict__ p = im.desc + (size_t)im.perm[s] * d;
+#pragma unroll
+    for (int k = 0; k < 8; k++) {
+      const uint32_t kk = c * 8u + k;
+      if (kk < d) h[k] = __float2half_rn(__ldg(p + kk));
+    }
+  }
+  uint8_t* op = reinterpret_cast<uint8_t*>(const_cast<__half*>(im.wideop));
+  const size_t off = ((size_t)(s >> 7) * (chunks / 8u) + (c >> 3)) * 16384u + sw128_offset(s & 127u, c & 7u);
+  *reinterpret_cast<uint4*>(op + off) = *reinterpret_cast<const uint4*>(h);
 }
 
 }  // namespace fm

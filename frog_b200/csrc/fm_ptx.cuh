@@ -143,6 +143,13 @@ __device__ __forceinline__ void tmem_ld_wait(uint32_t (&a)[32], uint32_t (&b)[32
   for (int i = 0; i < 32; i++) asm volatile("" : "+r"(a[i]), "+r"(b[i]), "+r"(c[i]), "+r"(d[i]));
 }
 
+// The same for two 32-register arrays.
+__device__ __forceinline__ void tmem_ld_wait(uint32_t (&a)[32], uint32_t (&b)[32]) {
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+  for (int i = 0; i < 32; i++) asm volatile("" : "+r"(a[i]), "+r"(b[i]));
+}
+
 // Shared-memory matrix descriptor for a K-major, SWIZZLE_128B operand tile whose rows are 128 B
 // (64 FP16): 8-row atoms 1024 B apart (SBO), LBO unused (=1), descriptor version 1 (sm_100),
 // layout type 2 = SWIZZLE_128B.  Field layout: cute::UMMA::SmemDescriptor.

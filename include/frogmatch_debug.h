@@ -43,6 +43,23 @@ int fm_debug_score_unit(fm_ctx* ctx, uint32_t first_img, uint32_t second_img, ui
                         uint32_t ld, uint32_t* bands_out, float* cand_t, uint32_t* cand_col);
 
 /*
+ * The wide tensor-core path (descriptor lengths d != 48, d <= 4096): run the band kernel and ONE unit (128 sorted rows
+ * starting at row_block * 128 of image `second` against the band of image `first`) of the wide scoring kernel in dump
+ * mode.  Any output pointer may be NULL.
+ *   t_out    : 128 x ld floats, t_out[r * ld + col] = t~ = fp16(a).fp16(b) - |b|^2/2 of (unit row r, sorted column col)
+ *              for every column the unit's MMAs computed (the steps it visited, trimmed to its band union in
+ *              16-column pieces); NaN elsewhere.  ld >= n_pad(first).
+ *   bands_out: min(128, rows left) x 2 uint32 (lo, hi) sorted-column interval per unit row
+ *   cand_t / cand_col: rows x 8, the row's 8 largest gated scores, descending (-inf padded); columns are sorted
+ *              positions in image `first`, bit 31 of slot 0 set when the row had more than 8 gated columns
+ *   eps_out  : the task's certified bound on |t~ - t_ref|;  k_pad_out: K_pad = d rounded up to 64
+ * Returns FM_ERR_INVALID for d = 48 or d > 4096.
+ */
+int fm_debug_wide_unit(fm_ctx* ctx, uint32_t first_img, uint32_t second_img, uint32_t row_block, float* t_out,
+                       uint32_t ld, uint32_t* bands_out, float* cand_t, uint32_t* cand_col, float* eps_out,
+                       uint32_t* k_pad_out);
+
+/*
  * What the reject pass of two-phase scoring computed for one task of the most recent fm_match, which must have run
  * with the option "reject_dump" set.  Task p is pair p; with FM_FLAG_SYM pair p is tasks 2p and 2p + 1.  Rows are
  * the sorted positions of the task's row image (image `second`, or `first` for task 2p + 1), n_rows of them.  Any
