@@ -184,7 +184,8 @@ int finalize(fm_result* r) {
 
 struct Batch {
   uint32_t t0, t1, rows, blocks, chunks, units;
-  size_t cursor;  // first entry of this batch in the concatenated prefix arrays
+  uint32_t rj_units;  // reject-pass units (kRjUnitRows rows each, fast tasks only)
+  size_t cursor;      // first entry of this batch in the concatenated prefix arrays
   bool any_exact, any_fast;
 };
 
@@ -399,7 +400,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
   c->reject_rows.clear();
   if (g_debug.reject_dump) c->reject_rows.resize(n_tasks);
 
-  // ---- batches + prefix arrays (blocks of 128 rows, compaction chunks, score units) ------------
+  // ---- batches + prefix arrays (blocks of 128 rows, compaction chunks, score units, reject-pass units) ------------
   uint64_t base_units = 0;
   for (auto& t : tasks)
     if (!(t.flags & kTaskExact)) base_units += (c->images[t.row_img].n + kUnitRows - 1) / kUnitRows;
@@ -409,18 +410,19 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
   if (match_all && total_rows > 0xFFFFFFF0ull) return fail(c, FM_ERR_UNSUPPORTED, "fm_match: -all supports at most 2^32 outer-loop rows per call");
   const uint32_t kMaxBatchRows = match_all ? 0xFFFFFFF0u : (24u << 20);  // -all: one batch (its scan spans all rows)
   std::vector<Batch> batches;
-  std::vector<uint32_t> blk_off, unit_off;
+  std::vector<uint32_t> blk_off, unit_off, rj_unit_off;
   std::vector<ChunkDesc> chunk_desc;  // compaction chunks of every batch, batch after batch (fm_compact.cuh)
   std::vector<size_t> chunk_cursor;   // first chunk of each batch in chunk_desc
   for (uint32_t t = 0; t < n_tasks;) {
     chunk_cursor.push_back(chunk_desc.size());
-    Batch b{t, t, 0, 0, 0, 0, blk_off.size(), false, false};
+    Batch b{t, t, 0, 0, 0, 0, 0, blk_off.size(), false, false};
     while (b.t1 < n_tasks) {
       const uint32_t nr = c->images[tasks[b.t1].row_img].n;
       if (b.t1 > b.t0 && (uint64_t)b.rows + nr > kMaxBatchRows) break;
       tasks[b.t1].row_off = b.rows;
       blk_off.push_back(b.blocks);
       unit_off.push_back(b.units);
+      rj_unit_off.push_back(b.rj_units);
       for (uint32_t r0 = 0; r0 < nr; r0 += kCompactChunk)
         chunk_desc.push_back(ChunkDesc{b.rows + r0, std::min<uint32_t>(kCompactChunk, nr - r0) | ((tasks[b.t1].flags & kTaskSwap) ? 0x80000000u : 0u),
                                        r0, pair_of_task[b.t1]});
@@ -428,11 +430,16 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
       b.blocks += (nr + 127) / 128;
       b.chunks += (nr + kCompactChunk - 1) / kCompactChunk;
       if (tasks[b.t1].flags & kTaskExact) b.any_exact = true;
-      else { b.any_fast = true; b.units += ((nr + kUnitRows - 1) / kUnitRows) * segs; }
+      else {
+        b.any_fast = true;
+        b.units += ((nr + kUnitRows - 1) / kUnitRows) * segs;
+        b.rj_units += (nr + kRjUnitRows - 1) / kRjUnitRows;  // (two-phase scoring runs at segs = 1 only)
+      }
       b.t1++;
     }
     blk_off.push_back(b.blocks);
     unit_off.push_back(b.units);
+    rj_unit_off.push_back(b.rj_units);
     batches.push_back(b);
     t = b.t1;
   }
@@ -469,12 +476,13 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
   c->stats.descriptor_pairs = desc_pairs;
   c->stats.rows = total_rows;
 
-  // metadata blob: tasks | chunk descriptors | blk_off | unit_off   (16-byte records first: alignment)
+  // metadata blob: tasks | chunk descriptors | blk_off | unit_off | rj_unit_off   (16-byte records first: alignment)
   const size_t np = blk_off.size();
   const size_t off_chunk = sizeof(Task) * n_tasks;
   const size_t off_blk = off_chunk + sizeof(ChunkDesc) * chunk_desc.size();
   const size_t off_unit = off_blk + sizeof(uint32_t) * np;
-  const size_t blob_bytes = off_unit + sizeof(uint32_t) * np;
+  const size_t off_rj = off_unit + sizeof(uint32_t) * np;
+  const size_t blob_bytes = off_rj + sizeof(uint32_t) * np;
   // The blob is staged in the result's pinned block (behind the counters and per-pair counts the device
   // writes back) so that the copy is asynchronous whatever its size: a pageable source would make
   // cudaMemcpyAsync wait for the stream, i.e. for the previous FM_FLAG_ASYNC call.
@@ -486,6 +494,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
   if (np) {
     memcpy(blob + off_blk, blk_off.data(), sizeof(uint32_t) * np);
     memcpy(blob + off_unit, unit_off.data(), sizeof(uint32_t) * np);
+    memcpy(blob + off_rj, rj_unit_off.data(), sizeof(uint32_t) * np);
   }
   FM_CUDA_R(c->d_meta_blob.ensure(std::max<size_t>(blob_bytes, 16)));
   FM_CUDA_R(cudaMemcpyAsync(c->d_meta_blob.p, blob, std::max<size_t>(blob_bytes, 16), cudaMemcpyHostToDevice, c->stream));
@@ -494,6 +503,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
   const ChunkDesc* d_chunk = reinterpret_cast<const ChunkDesc*>(blob_d + off_chunk);
   const uint32_t* d_blk = reinterpret_cast<const uint32_t*>(blob_d + off_blk);
   const uint32_t* d_unit = reinterpret_cast<const uint32_t*>(blob_d + off_unit);
+  const uint32_t* d_rj_unit = reinterpret_cast<const uint32_t*>(blob_d + off_rj);
 
   uint32_t max_rows = 1, max_chunks = 1;
   for (auto& b : batches) { max_rows = std::max(max_rows, b.rows); max_chunks = std::max(max_chunks, b.chunks); }
@@ -613,6 +623,8 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
         fa.blocks128 = b.blocks;
         fa.unit_off = unt;
         fa.units = b.units;
+        fa.rj_unit_off = d_rj_unit + b.cursor;
+        fa.rj_units = b.rj_units;
         fa.segs = segs;
         fa.thr = dist;
         fa.ratio = dist2second;

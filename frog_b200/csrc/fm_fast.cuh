@@ -138,6 +138,8 @@ struct FastBatchArgs {
   uint32_t blocks128;
   const uint32_t* unit_off;  // device: score units per task (prefix), already multiplied by segs
   uint32_t units;
+  const uint32_t* rj_unit_off;  // device: reject-pass units per task (prefix, kRjUnitRows rows each)
+  uint32_t rj_units;
   uint32_t segs;
   float thr, ratio;
   uint32_t* rowres;
@@ -227,20 +229,20 @@ inline cudaError_t fast_match_batch(fm_ctx* c, const FastBatchArgs& a) {
       uint32_t* surv_rows = surv_off + a.n_tasks + 1;
       if ((e = cudaMemsetAsync(surv_count, 0, (size_t)a.n_tasks * sizeof(uint32_t), c->stream)) != cudaSuccess) return e;
       // persistent: one CTA per SM walks the units
-      const uint32_t grid = std::min<uint32_t>(a.units, (uint32_t)c->sm_count);
+      const uint32_t grid = std::min<uint32_t>(a.rj_units, (uint32_t)c->sm_count);
       if (g_debug.reject_dump) {
         DevBuf dump;
         if ((e = dump.ensure((size_t)a.rows * sizeof(float4))) != cudaSuccess) return e;
         if ((e = cudaMemsetAsync(dump.p, 0xFF, (size_t)a.rows * sizeof(float4), c->stream)) != cudaSuccess) return e;
         reject_kernel<true><<<grid, kRjThreads, kRjSmemBytes, c->stream>>>(
-            a.images, a.tasks, a.unit_off, a.n_tasks, a.units, c->d_bands.as<uint2>(), &a.counters->scored_cols, a.thr,
+            a.images, a.tasks, a.rj_unit_off, a.n_tasks, a.rj_units, c->d_bands.as<uint2>(), &a.counters->scored_cols, a.thr,
             a.ratio, rowstat, surv_count, surv_rows, dump.as<float4>());
         if ((e = cudaGetLastError()) == cudaSuccess) e = stash_reject_rows(c, a, dump.as<float4>(), rowstat, surv_count, surv_rows);
         dump.release();
         if (e != cudaSuccess) return e;
       } else {
         reject_kernel<false><<<grid, kRjThreads, kRjSmemBytes, c->stream>>>(
-            a.images, a.tasks, a.unit_off, a.n_tasks, a.units, c->d_bands.as<uint2>(), &a.counters->scored_cols, a.thr,
+            a.images, a.tasks, a.rj_unit_off, a.n_tasks, a.rj_units, c->d_bands.as<uint2>(), &a.counters->scored_cols, a.thr,
             a.ratio, rowstat, surv_count, surv_rows, nullptr);
       }
       surv_plan_kernel<<<1, 1024, 0, c->stream>>>(surv_count, a.n_tasks, surv_off, cap_units, a.tasks, surv_rows, rowstat,

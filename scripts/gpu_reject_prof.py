@@ -6,10 +6,11 @@
 2 warm-up calls, then 5 calls under torch.profiler with CUDA activities.  Prints and writes one JSON object: µs per
 launch of every kernel, the card, its power limit and SM clocks (nvidia-smi, read right after the profiled calls), and
 from a numpy replay of the reference's gates over the same images:
-  * TMA operand bytes per launch: per unit with a step, its two 16 KB row-operand tiles, plus 32 KB per 256-column step;
-  * the number of steps, and per epilogue warp and step its two 128-column rounds (one per row half) split into
-    skipped (no row of the warp has a column there), interior (every row of the warp accepts all 128 columns) and
-    edge (masked per score).
+  * TMA operand bytes per launch: per 512-row unit with a step, its 16 KB row-operand tiles (one per 128-row quarter
+    with rows: 1 to 4), plus 32 KB per 256-column step;
+  * the number of units and steps, and per epilogue warp and step its four 128-column rounds (one per quarter's fill)
+    split into skipped (no row of the warp has a column there), interior (every row of the warp accepts all 128
+    columns) and edge (masked per score).
 --lib points at another build of libfrogmatch.so, so that two builds can be alternated in one session.
 --counts-only skips the GPU and prints the replay alone.
 """
@@ -29,7 +30,7 @@ sys.path.insert(0, ROOT)
 from frog_b200 import capi, synth  # noqa: E402
 
 N_IMAGES, N_POINTS, THR, RATIO = 24, 20000, 1.0, 0.8
-UNIT, WARP_ROWS, STEP, ROUND = 256, 32, 256, 128
+UNIT, TILE_ROWS, WARP_ROWS, STEP, ROUND = 512, 128, 32, 256, 128  # reject-pass unit = four 128-row quarters
 OP_TILE_BYTES, STEP_BYTES = 16384, 32768
 
 
@@ -95,10 +96,11 @@ def replay(kps, pf, ps):
         nst = np.where(has, (umax + STEP - 1) // STEP - step0, 0)
         tot["units"] += int(has.sum())
         tot["steps"] += int(nst.sum())
-        tot["tma_operand_bytes_per_launch"] += int(has.sum()) * 2 * OP_TILE_BYTES + int(nst.sum()) * STEP_BYTES
+        tiles = np.minimum(UNIT // TILE_ROWS, (n - np.arange(units) * UNIT + TILE_ROWS - 1) // TILE_ROWS)  # quarters with rows
+        tot["tma_operand_bytes_per_launch"] += int((tiles * has).sum()) * OP_TILE_BYTES + int(nst.sum()) * STEP_BYTES
         k = np.arange(int(nst.max()) if nst.size else 0)
         live = k[None, :] < nst[:, None]                       # [unit, step]
-        for c in range(STEP // ROUND):
+        for c in range(STEP // ROUND):  # the 32-row groups are the (quarter, lane quadrant) pairs: one fill each
             c0 = ((step0[:, None] + k[None, :]) * STEP + c * ROUND)[:, :, None]  # [unit, step, 1]
             need = (c0 < cmax[:, None, :]) & (c0 + ROUND > cmin[:, None, :])    # [unit, step, group]
             inter = (c0 >= imin[:, None, :]) & (c0 + ROUND <= imax[:, None, :])
