@@ -58,8 +58,10 @@ def build_cli(force: bool = False) -> str:
     os.makedirs(os.path.dirname(BIN), exist_ok=True)
     cmd = ["g++", "-O2", "-std=c++17", "-fopenmp", "-I", os.path.join(ROOT, "include"),
            os.path.join(CSRC, "match_main.cpp"), os.path.join(CSRC, "keypoint_io.cpp"), os.path.join(CSRC, "fast_inflate.cpp"),
-           "-o", BIN, "-L", os.path.dirname(LIB), "-lfrogmatch", "-lz",
+           os.path.join(CSRC, "surf_io.cpp"),
+           "-o", BIN, "-L", os.path.dirname(LIB), "-lfrogmatch", "-lz", "-ldl",
            "-Wl,-rpath,$ORIGIN/../frog_b200"]
+    # (libfrogsurf.so is not linked: bin/match dlopens it, through the same run path, when a list holds volumes)
     # multi-GPU list gather over NCCL (system libnccl; only the executable links it, never libfrogmatch.so, so a
     # Python process that already carries torch's NCCL is not given a second copy)
     cuda = os.environ.get("CUDA_HOME", "/usr/local/cuda")
@@ -82,7 +84,7 @@ def build_fmio(force: bool = False) -> str:
 
 
 def build_surf_lib(force: bool = False, verbose: bool = False) -> str:
-    srcs = [os.path.join(CSRC, f) for f in ("fs_api.cu", "fs_kernels.cuh")] + [
+    srcs = [os.path.join(CSRC, f) for f in ("fs_api.cu", "fs_kernels.cuh", "fs_as_read.cuh")] + [
         os.path.join(ROOT, "include", f) for f in ("frogsurf.h", "frogsurf_debug.h")]
     if not force and _newer(SURF_LIB, srcs):
         return SURF_LIB
@@ -110,7 +112,7 @@ def build_fsio(force: bool = False) -> str:
     srcs = [os.path.join(CSRC, f) for f in ("surf_io.cpp", "surf_io.h")] + [os.path.join(ROOT, "include", "frogsurf.h")]
     if not force and _newer(FSIO, srcs):
         return FSIO
-    cmd = ["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-I", os.path.join(ROOT, "include"),
+    cmd = ["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-fopenmp", "-I", os.path.join(ROOT, "include"),
            os.path.join(CSRC, "surf_io.cpp"), "-o", FSIO, "-lz"]
     subprocess.run(cmd, check=True, cwd=ROOT)
     return FSIO

@@ -4,12 +4,15 @@
 // interpolation step (fasthessian.cxx:575-661) and the response sort (vtk3DSURF.cxx:209-226).
 #include <algorithm>
 #include <cmath>
+#include <cerrno>
 #include <cstdarg>
+#include <cstdlib>
 #include <cstdio>
 #include <cstring>
 #include <string>
 #include <vector>
 
+#include "fs_as_read.cuh"
 #include "fs_kernels.cuh"
 
 namespace {
@@ -53,6 +56,11 @@ struct fs_ctx {
   float* d_desc = nullptr;
   size_t desc_cap = 0;
   uint32_t desc_size = 0;
+  float* d_as_read = nullptr;  // fs_get_points_as_read: head + descriptors as the .csv.gz reader returns them
+  size_t as_read_cap = 0;
+  fs::AsReadFallback* d_fallback = nullptr;
+  size_t fallback_cap = 0;
+  unsigned long long* d_fallback_count = nullptr;
   bool have_volume = false;
   bool keep_cast = false;  // fs_debug_keep_cast_volume: also store vtk3DSURF::Cast (only the parity tests read it)
   fs_stats stats{};
@@ -255,6 +263,55 @@ int upload_points(fs_ctx* c) {
   return FS_OK;
 }
 
+// format_fixed's snprintf path (surf_io.cpp) followed by the reader's strtof
+float as_read_on_host(double v, int decimals, bool* range_error) {
+  char fmt[16], text[512];
+  std::snprintf(fmt, sizeof fmt, "%%.%df", decimals);
+  std::snprintf(text, sizeof text, fmt, v);
+  errno = 0;
+  const float f = std::strtof(text, nullptr);
+  if (errno == ERANGE) *range_error = true;
+  return f;
+}
+
+// Runs the conversion kernel `launch(list)` until its list of host values holds all of them, then copies `total`
+// results to `out` (split at `split`: out[0 .. split) and out2[0 .. total - split)) and finishes the listed values.
+// `decimals_of(index)` gives a listed value's decimals.
+template <class Launch, class Decimals>
+int as_read_finish(fs_ctx* c, size_t total, size_t split, float* out, float* out2, Launch launch, Decimals decimals_of,
+                   bool* range_error) {
+  unsigned long long listed = 0;
+  for (;;) {
+    FS_CUDA(c, cudaMemsetAsync(c->d_fallback_count, 0, sizeof(unsigned long long), c->stream));
+    launch(fs::AsReadList{c->d_fallback, c->d_fallback_count, (unsigned long long)c->fallback_cap});
+    FS_CUDA(c, cudaGetLastError());
+    FS_CUDA(c, cudaMemcpyAsync(&listed, c->d_fallback_count, sizeof listed, cudaMemcpyDeviceToHost, c->stream));
+    FS_CUDA(c, cudaStreamSynchronize(c->stream));
+    if (listed <= c->fallback_cap) break;
+    if (int rc = ensure(c, c->d_fallback, c->fallback_cap, (size_t)listed)) return rc;
+  }
+  if (split) FS_CUDA(c, cudaMemcpyAsync(out, c->d_as_read, split * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  if (total > split)
+    FS_CUDA(c, cudaMemcpyAsync(out2, c->d_as_read + split, (total - split) * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  std::vector<fs::AsReadFallback> fb((size_t)listed);
+  if (listed) FS_CUDA(c, cudaMemcpyAsync(fb.data(), c->d_fallback, listed * sizeof(fs::AsReadFallback), cudaMemcpyDeviceToHost, c->stream));
+  FS_CUDA(c, cudaStreamSynchronize(c->stream));
+  for (const fs::AsReadFallback& e : fb) {
+    const float f = as_read_on_host(e.value, decimals_of(e.index), range_error);
+    if (e.index < split) out[e.index] = f;
+    else out2[e.index - split] = f;
+  }
+  return FS_OK;
+}
+
+int as_read_buffers(fs_ctx* c, size_t total) {
+  if (int rc = ensure(c, c->d_as_read, c->as_read_cap, total)) return rc;
+  if (!c->d_fallback_count) FS_CUDA(c, cudaMalloc((void**)&c->d_fallback_count, sizeof(unsigned long long)));
+  return ensure(c, c->d_fallback, c->fallback_cap, std::min<size_t>(total, (size_t)1 << 16));
+}
+
+unsigned as_read_blocks(size_t total) { return (unsigned)std::max<size_t>(1, std::min<size_t>((total + 255) / 256, 148 * 16)); }
+
 float elapsed(fs_ctx* c) {
   float ms = 0;
   cudaEventSynchronize(c->ev[1]);
@@ -304,7 +361,7 @@ void fs_destroy(fs_ctx* c) {
   if (c->stream) cudaStreamSynchronize(c->stream);
   cudaFree(c->d_cast); cudaFree(c->d_integral); cudaFree(c->d_split); cudaFree(c->d_in); cudaFree(c->d_blockmin);
   cudaFree(c->d_layer_f); cudaFree(c->d_layer_b); cudaFree(c->d_cand); cudaFree(c->d_interp); cudaFree(c->d_count);
-  cudaFree(c->d_points); cudaFree(c->d_desc);
+  cudaFree(c->d_points); cudaFree(c->d_desc); cudaFree(c->d_as_read); cudaFree(c->d_fallback); cudaFree(c->d_fallback_count);
   if (c->ev[0]) cudaEventDestroy(c->ev[0]);
   if (c->ev[1]) cudaEventDestroy(c->ev[1]);
   if (c->stream) cudaStreamDestroy(c->stream);
@@ -595,6 +652,33 @@ int fs_get_points(fs_ctx* c, fs_point* points, float* desc) {
   return FS_OK;
 }
 
+int fs_get_points_as_read(fs_ctx* c, int precision, const double spacing[3], const double origin[3], float* head, float* desc) {
+  if (!c || !spacing || !origin) return FS_ERR_INVALID;
+  const size_t n = c->points.size(), d = c->desc_size;
+  if (!n) return FS_OK;
+  if (!d) return fail(c, FS_ERR_STATE, "fs_get_points_as_read: no descriptors yet");
+  if (!head || !desc) return fail(c, FS_ERR_INVALID, "fs_get_points_as_read: null output");
+  FS_CUDA(c, cudaSetDevice(c->device));
+  const size_t total = n * (6 + d);
+  if (int rc = as_read_buffers(c, total)) return rc;
+  fs::AsReadGeom g{};
+  for (int i = 0; i < 3; i++) { g.spacing[i] = spacing[i]; g.origin[i] = origin[i]; }
+  g.sspacing = std::pow(spacing[0] * spacing[1] * spacing[2], 1.0 / 3.0);  // the writers' Sspacing (surf_io.cpp)
+  g.decimals = precision >= 0 ? precision : 6;  // "%f" = six decimals
+  bool range_error = false;
+  const int rc = as_read_finish(
+      c, total, n * 6, head, desc,
+      [&](fs::AsReadList list) {
+        fs::as_read_kernel<<<as_read_blocks(total), 256, 0, c->stream>>>(c->d_points, c->d_desc, (unsigned)n, (unsigned)d, g,
+                                                                          c->d_as_read, list);
+      },
+      [&](unsigned long long index) { return index < n * 6 ? 6 : g.decimals; }, &range_error);
+  if (rc) return rc;
+  // the reader's std::stof throws there: the keypoint file could not be read back
+  if (range_error) return fail(c, FS_ERR_INVALID, "fs_get_points_as_read: a value's text is out of float range");
+  return FS_OK;
+}
+
 int fs_get_stats(fs_ctx* c, fs_stats* out) {
   if (!c || !out) return FS_ERR_INVALID;
   *out = c->stats;
@@ -639,6 +723,30 @@ void fs_debug_sort_keys(const uint64_t* keys, uint32_t n, uint32_t* order) {
 }
 
 void fs_debug_keep_cast_volume(fs_ctx* c, int on) { if (c) c->keep_cast = on != 0; }
+
+int fs_debug_as_read(const double* in, size_t n, int precision, float* out) {
+  if (!n) return FS_OK;
+  if (!in || !out) return FS_ERR_INVALID;
+  fs_ctx* c = nullptr;
+  if (int rc = fs_create(0, &c)) return rc;
+  double* d_in = nullptr;
+  size_t in_cap = 0;
+  int rc = as_read_buffers(c, n);
+  if (!rc) rc = ensure(c, d_in, in_cap, n);
+  if (!rc && cudaMemcpy(d_in, in, n * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) rc = FS_ERR_CUDA;
+  const int decimals = precision >= 0 ? precision : 6;
+  bool range_error = false;
+  if (!rc)
+    rc = as_read_finish(
+        c, n, n, out, nullptr,
+        [&](fs::AsReadList list) {
+          fs::as_read_values_kernel<<<as_read_blocks(n), 256, 0, c->stream>>>(d_in, n, decimals, c->d_as_read, list);
+        },
+        [&](unsigned long long) { return decimals; }, &range_error);
+  cudaFree(d_in);
+  fs_destroy(c);
+  return rc;
+}
 
 int fs_get_cast_volume(fs_ctx* c, int32_t* out) {
   if (!c || !out) return FS_ERR_INVALID;

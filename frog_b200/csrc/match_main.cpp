@@ -24,6 +24,17 @@
 //     and leave with _exit; the parent writes pairs.bin in the reference's block order.
 // `-gather nccl` sends the lists GPU-to-GPU over NVLink to worker 0 instead (one communicator rank
 // per worker) -- identical bytes, but communicator start-up costs more than it saves a one-shot run.
+//
+// Volume entries.  A list entry ending in ".mha" is a MetaImage volume: the load loop reads it (in parallel, like the
+// keypoint files) and hands it to the SURF3D producer, which yields exactly the keypoints that
+// `surf3d <volume> <options>` followed by the .csv.gz reader would (`-surf3d "<surf3d options>"`, one token; the
+// conversion to the text's values runs on the device, fs_get_points_as_read).  This removes a process start -- and so
+// a CUDA start-up, ~0.55 s -- and a text round trip per volume.  Producer calls go to ONE fs_ctx on this process's
+// GPU 0, created by the first volume after the workers are forked and used by one loader thread at a time: a 400^3
+// volume takes ~10.5 ms there, so one GPU produces faster than a disk delivers volumes.  libfrogsurf.so is dlopen'ed
+// only when the list holds a volume, so a deployment for keypoint files needs libfrogmatch.so alone.  A resident
+// server keeps its producer context from job to job.
+#include <dlfcn.h>
 #include <omp.h>
 #include <sys/mman.h>
 #include <sys/wait.h>
@@ -40,6 +51,7 @@
 #include <filesystem>
 #include <fstream>
 #include <iostream>
+#include <mutex>
 #include <numeric>
 #include <sstream>
 #include <string>
@@ -47,7 +59,9 @@
 #include <vector>
 
 #include "frogmatch.h"
+#include "frogsurf.h"
 #include "keypoint_io.h"
+#include "surf_io.h"
 
 #ifdef FM_WITH_NCCL
 #include <cuda_runtime.h>
@@ -319,9 +333,95 @@ void worker_run(Control* ctl, int g, int device, fm_ctx* warm) {
   // leave, and destroying one CUDA context per GPU costs more than everything above.
 }
 
-// Contexts a resident server (`match -serve-daemon`) keeps warm: one per visible device.
+// ---- volume entries: the SURF3D producer (libfrogsurf.so, loaded at run time) --------------------------------------
+
+bool is_volume(const string& f) { return f.size() > 4 && f.compare(f.size() - 4, 4, ".mha") == 0; }
+
+struct SurfApi {
+  void* handle = nullptr;
+  // (frogsurf.h's declarations give the types; nothing here links against them)
+  decltype(&fs_create) create = nullptr;
+  decltype(&fs_last_error) last_error = nullptr;
+  decltype(&fs_set_volume) set_volume = nullptr;
+  decltype(&fs_detect) detect = nullptr;
+  decltype(&fs_select) select = nullptr;
+  decltype(&fs_describe) describe = nullptr;
+  decltype(&fs_num_points) num_points = nullptr;
+  decltype(&fs_get_points_as_read) get_points_as_read = nullptr;
+  decltype(&fs_get_stats) get_stats = nullptr;
+
+  // dlopen searches the executable's run path ($ORIGIN/../frog_b200), then the usual places
+  bool load(string& err) {
+    if (handle) return true;
+    void* h = dlopen("libfrogsurf.so", RTLD_NOW | RTLD_LOCAL);
+    if (!h) { err = dlerror(); return false; }
+    bool ok = true;
+    auto sym = [&](auto& fn, const char* name) {
+      fn = reinterpret_cast<std::remove_reference_t<decltype(fn)>>(dlsym(h, name));
+      if (!fn) { ok = false; err = string("libfrogsurf.so lacks ") + name; }
+    };
+    sym(create, "fs_create");
+    sym(last_error, "fs_last_error");
+    sym(set_volume, "fs_set_volume");
+    sym(detect, "fs_detect");
+    sym(select, "fs_select");
+    sym(describe, "fs_describe");
+    sym(num_points, "fs_num_points");
+    sym(get_points_as_read, "fs_get_points_as_read");
+    sym(get_stats, "fs_get_stats");
+    if (!ok) { dlclose(h); return false; }
+    handle = h;
+    return true;
+  }
+};
+
+// One producer context for all volume entries of a job: created by the first volume that needs it, used by one
+// loader thread at a time (an fs_ctx is one-host-thread-at-a-time).
+struct VolumeProducer {
+  SurfApi* api = nullptr;
+  fs_ctx** ctx = nullptr;  // a resident server's, kept across jobs, or this job's
+  std::mutex mu;
+  uint32_t volumes = 0;
+  double busy_s = 0, gpu_ms = 0;
+};
+
+// `surf3d <path> <options>` then fmio::read_keypoints of the .csv.gz it writes, without the file
+bool produce_keypoints(const string& path, const fsio::SurfOptions& o, VolumeProducer& P, fmio::KeypointSet& k, string& err) {
+  fsio::Volume vol;
+  if (!fsio::read_metaimage(path, vol, err, stderr)) return false;
+  fsio::clamp_volume(vol, o);
+  std::lock_guard<std::mutex> lock(P.mu);
+  const double t0 = now_s();
+  const SurfApi& F = *P.api;
+  if (!*P.ctx && F.create(0, P.ctx) != FS_OK) { err = string("SURF3D producer: ") + F.last_error(nullptr); return false; }
+  fs_ctx* c = *P.ctx;
+  uint32_t n = 0, d = 0;
+  auto die = [&](const char* what) { err = string("SURF3D producer, ") + what + ": " + F.last_error(c); return false; };
+  if (F.set_volume(c, vol.data.data(), vol.voxel_type, vol.dims[0], vol.dims[1], vol.dims[2]) != FS_OK) return die("volume");
+  if (F.detect(c, (float)o.threshold, &n) != FS_OK) return die("detector");
+  if (F.select(c, o.numberOfPoints) != FS_OK) return die("select");
+  if (F.describe(c, o.descriptorType, o.subVolumeRadius, o.normalize) != FS_OK) return die("descriptors");
+  F.num_points(c, &n, &d);
+  k = fmio::KeypointSet{};
+  k.n = n;
+  k.d = n ? d : 0;  // an empty file: no row, no length
+  k.head.resize((size_t)n * 6);
+  k.desc.resize((size_t)n * d);
+  if (F.get_points_as_read(c, o.precision, vol.spacing, vol.origin, k.head.data(), k.desc.data()) != FS_OK) return die("read back");
+  fs_stats st{};
+  F.get_stats(c, &st);
+  P.gpu_ms += (double)st.ms_integral + st.ms_response_map + st.ms_extrema + st.ms_describe;
+  P.volumes++;
+  P.busy_s += now_s() - t0;
+  return true;
+}
+
+// Contexts a resident server (`match -serve-daemon`) keeps warm: one per visible device, and the producer's once a
+// job has needed it.
 struct WarmPool {
   std::vector<fm_ctx*> ctx;
+  SurfApi surf_api;
+  fs_ctx* surf = nullptr;
 };
 
 }  // namespace
@@ -356,6 +456,7 @@ int run_job(int argc, char* argv[], std::ostream& cout, std::ostream& cerr, Warm
   // "nccl" = GPU-to-GPU over NVLink to GPU 0, then one device-to-host copy.  Bringing the communicators up costs a
   // one-shot process more than matching a 50 x 50k group, so "host" is the default here.
   const char* gatherMode = "host";
+  const char* surfArgs = "";  // -surf3d "<options>": bin/surf3d's options for the volume entries
 
   // match.cpp:365-431: key = argv[k], value = argv[k+1]; advance by 2, by 1 for -sym.
   for (int k = 2; k < argc;) {
@@ -382,6 +483,7 @@ int run_job(int argc, char* argv[], std::ostream& cout, std::ostream& cerr, Warm
       if (has("-plan")) planOnly = atoi(value) != 0;
       if (has("-mp")) multiProcess = atoi(value) != 0;
       if (has("-serve")) serveMode = atoi(value) != 0;
+      if (has("-surf3d")) surfArgs = value;
     }
     if (has("-all")) matchAll = true;
     if (has("-p")) writePoints = true;
@@ -394,6 +496,25 @@ int run_job(int argc, char* argv[], std::ostream& cout, std::ostream& cerr, Warm
     return 1;
   }
   if (writePoints) cerr << "match: -p (debug CSV dump) is ignored by the B200 build" << endl;
+  // bin/surf3d's own option loop and refusals; the file-output keys (-o -bin -csv -csvgz -gz) and -gpu have nothing
+  // to act on here
+  std::vector<string> surfTokens;
+  {
+    std::istringstream ss(surfArgs);
+    for (string t; ss >> t;) surfTokens.push_back(t);
+  }
+  std::vector<char*> surfArgv;
+  for (string& t : surfTokens) surfArgv.push_back(&t[0]);
+  fsio::SurfOptions surfOpts;
+  fsio::parse_surf_options((int)surfArgv.size(), surfArgv.data(), 0, surfOpts);
+  if (const char* what = fsio::unsupported_surf_option(surfOpts)) {
+    cerr << fsio::unsupported_surf_message(what) << endl;
+    return 7;
+  }
+  if (surfOpts.pointFile) {
+    cerr << "match: -surf3d -p (descriptors at the points of a csv file) is not available for volume entries; terminating." << endl;
+    return 7;
+  }
   const bool want_nccl = strcmp(gatherMode, "nccl") == 0;
   if (distsFile && (matchAll || want_nccl)) {
     cerr << "match: -dists is not available with -all or -gather nccl" << endl;
@@ -454,6 +575,16 @@ int run_job(int argc, char* argv[], std::ostream& cout, std::ostream& cerr, Warm
       const double bytes = (double)fs::file_size(filenames[i], ec);
       if (ec) continue;
       const string& f = filenames[i];
+      if (is_volume(f)) {
+        // At most one extremum per middle response layer position, layers sampled every 2 voxels or more: fewer than
+        // voxels / 3 keypoints, and a voxel takes at least one byte of the file.
+        const double d = surfOpts.descriptorType == 1 ? 24.0 * std::pow((double)surfOpts.subVolumeRadius, 3) : 48.0;
+        const double n_vol = surfOpts.numberOfPoints > 0 ? std::min<double>(surfOpts.numberOfPoints, bytes / 3) : bytes / 3;
+        est_bytes += n_vol * (d + 2) * sizeof(float);
+        pts += n_vol;
+        pts2 += n_vol * n_vol;
+        continue;
+      }
       const bool gz = f.size() > 3 && f.compare(f.size() - 3, 3, ".gz") == 0;
       const bool bin = f.size() > 4 && f.compare(f.size() - 4, 4, ".bin") == 0;
       const double n_est = bytes / (bin ? 216.0 : gz ? 220.0 : 500.0);  // 54 floats; "%f" text; the same gzipped
@@ -495,6 +626,20 @@ int run_job(int argc, char* argv[], std::ostream& cout, std::ostream& cerr, Warm
   if (nt > 0) omp_set_num_threads(nt);
   int nb = (int)n_load;
   if (nb > 65535) { cerr << "match: more than 65535 images cannot be described by pairs.bin (u16 ids)" << endl; return 1; }
+
+  // the producer's library, before any thread or CUDA state exists (its context comes later, see the load loop)
+  SurfApi own_surf_api;
+  fs_ctx* own_surf_ctx = nullptr;
+  VolumeProducer producer;
+  producer.api = warm ? &warm->surf_api : &own_surf_api;
+  producer.ctx = warm ? &warm->surf : &own_surf_ctx;
+  if (std::any_of(filenames.begin(), filenames.begin() + nb, is_volume)) {
+    string err;
+    if (!producer.api->load(err)) {
+      cerr << "match: the list holds MetaImage volumes (.mha), which need libfrogsurf.so: " << err << endl;
+      return 1;
+    }
+  }
 
   Control* ctl = map_arena((size_t)nb, (uint64_t)est_bytes);
   if (!ctl) { cerr << "match: cannot map the shared arena" << endl; return 1; }
@@ -568,7 +713,8 @@ int run_job(int argc, char* argv[], std::ostream& cout, std::ostream& cerr, Warm
     string err;
     fmio::KeypointSet& k = images[it];
     if (ctl->abort.load()) continue;
-    if (!fmio::read_keypoints(filenames[it], k, err)) {
+    if (!(is_volume(filenames[it]) ? produce_keypoints(filenames[it], surfOpts, producer, k, err)
+                                   : fmio::read_keypoints(filenames[it], k, err))) {
 #pragma omp critical
       { cerr << err << " (" << filenames[it] << ")" << endl; load_failed = 1; }
       ctl->abort.store(1);
@@ -790,7 +936,8 @@ int run_job(int argc, char* argv[], std::ostream& cout, std::ostream& cerr, Warm
        << ", \"upload_s\": " << upload_s << ", \"match_call_s\": " << match_s << ", \"gather_s\": " << gather_s
        << ", \"matches\": " << sum
        << ", \"gather\": \"" << (ctl->use_nccl ? "nccl" : (G > 1 ? "host" : "none")) << "\""
-       << ", \"nccl_init_s\": " << nccl_init_s << "}" << endl;
+       << ", \"nccl_init_s\": " << nccl_init_s << ", \"volumes\": " << producer.volumes << ", \"produce_s\": " << producer.busy_s
+       << ", \"produce_gpu_ms\": " << producer.gpu_ms << "}" << endl;
   }
   return leave(0);
 }

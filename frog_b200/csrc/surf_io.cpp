@@ -4,6 +4,7 @@
 
 #include <cmath>
 #include <cstdio>
+#include <cstdlib>
 #include <cstring>
 #include <fstream>
 #include <map>
@@ -92,7 +93,7 @@ inline size_t format_fixed(double v, int decimals, char* out, size_t cap) {
 
 }  // namespace
 
-bool read_metaimage(const std::string& path, Volume& out, std::string& err) {
+bool read_metaimage(const std::string& path, Volume& out, std::string& err, FILE* warnings) {
   std::ifstream f(path, std::ios::binary);
   if (!f) { err = "cannot open " + path; return false; }
   std::map<std::string, std::string> kv;
@@ -145,7 +146,7 @@ bool read_metaimage(const std::string& path, Volume& out, std::string& err) {
     if (!dbls(key, m, 9)) continue;
     for (int i = 0; i < 3; i++) {
       if (!(m[4 * i] < 0)) continue;
-      std::fprintf(stdout, "Warning : RobustReader flipping dimension %d\n", i);
+      if (warnings) std::fprintf(warnings, "Warning : RobustReader flipping dimension %d\n", i);
       switch (type_size(out.voxel_type)) {
         case 1: flip_axis<uint8_t>(out.data, out.dims, i); break;
         case 2: flip_axis<uint16_t>(out.data, out.dims, i); break;
@@ -293,6 +294,71 @@ bool read_points_file(const std::string& path, const double spacing[3], const do
   return true;
 }
 
+void parse_surf_options(int argc, char* const argv[], int first, SurfOptions& o) {
+  for (int k = first; k < argc; k += 2) {
+    const char* key = argv[k];
+    char* value = k + 1 < argc ? argv[k + 1] : (char*)"";
+    if (std::strcmp(key, "-d") == 0) o.maxSize = std::atoi(value);
+    if (std::strcmp(key, "-s") == 0) o.spacing = std::atof(value);
+    if (std::strcmp(key, "-t") == 0) o.threshold = std::atof(value);
+    if (std::strcmp(key, "-cmin") == 0) { o.clampMinValues = true; o.clampMinValue = std::atof(value); }
+    if (std::strcmp(key, "-cmax") == 0) { o.clampMaxValues = true; o.clampMaxValue = std::atof(value); }
+    if (std::strcmp(key, "-m") == 0) o.maskfilename = value;
+    if (std::strcmp(key, "-o") == 0) o.outfilename = value;
+    if (std::strcmp(key, "-json") == 0) o.writeJSON = std::atoi(value);
+    if (std::strcmp(key, "-csv") == 0) o.writeCSV = std::atoi(value);
+    if (std::strcmp(key, "-bin") == 0) o.writeBIN = std::atoi(value);
+    if (std::strcmp(key, "-csvgz") == 0) o.writeCSVGZ = std::atoi(value);
+    if (std::strcmp(key, "-type") == 0) o.descriptorType = std::atoi(value);
+    if (std::strcmp(key, "-n") == 0) o.numberOfPoints = std::atoi(value);
+    if (std::strcmp(key, "-p") == 0) o.pointFile = value;
+    if (std::strcmp(key, "-r") == 0) o.subVolumeRadius = std::atoi(value);
+    if (std::strcmp(key, "-normalize") == 0) o.normalize = std::atoi(value);
+    if (std::strcmp(key, "-pad") == 0) o.pad = std::atoi(value);
+    if (std::strcmp(key, "-gz") == 0) o.gzOpts = value;
+    if (std::strcmp(key, "-precision") == 0) o.precision = std::atoi(value);
+    if (std::strcmp(key, "-gpu") == 0) o.gpu = std::atoi(value);
+  }
+}
+
+const char* unsupported_surf_option(const SurfOptions& o) {
+  if (o.spacing != 0 || o.maxSize > 0) return "-s / -d (vtkImageResample)";
+  if (o.maskfilename) return "-m (mask resampling)";
+  if (o.pad) return "-pad (vtkImageMirrorPad)";
+  if (o.descriptorType == 2) return "-type 2 (vtkImageResize)";
+  if (o.writeJSON) return "-json 1 (picojson point dump)";
+  return nullptr;
+}
+
+std::string unsupported_surf_message(const char* what) {
+  return std::string("surf3d (B200): ") + what + " needs a VTK image filter that this build does not restate; terminating.";
+}
+
+namespace {
+template <typename T>
+void clamp_values(std::vector<unsigned char>& data, bool lo_on, float lo, bool hi_on, float hi) {
+  // values below -cmin become cmin, above -cmax become cmax
+  T* p = reinterpret_cast<T*>(data.data());
+  const size_t n = data.size() / sizeof(T);
+  for (size_t i = 0; i < n; i++) {
+    if (lo_on && (double)p[i] < (double)lo) p[i] = (T)lo;
+    if (hi_on && (double)p[i] > (double)hi) p[i] = (T)hi;
+  }
+}
+}  // namespace
+
+void clamp_volume(Volume& v, const SurfOptions& o) {
+  if (!o.clampMinValues && !o.clampMaxValues) return;
+  const bool lo = o.clampMinValues, hi = o.clampMaxValues;
+  switch (v.voxel_type) {
+    case FS_U8: clamp_values<uint8_t>(v.data, lo, o.clampMinValue, hi, o.clampMaxValue); break;
+    case FS_I16: clamp_values<int16_t>(v.data, lo, o.clampMinValue, hi, o.clampMaxValue); break;
+    case FS_U16: clamp_values<uint16_t>(v.data, lo, o.clampMinValue, hi, o.clampMaxValue); break;
+    case FS_I32: clamp_values<int32_t>(v.data, lo, o.clampMinValue, hi, o.clampMaxValue); break;
+    default: clamp_values<float>(v.data, lo, o.clampMinValue, hi, o.clampMaxValue); break;
+  }
+}
+
 bool write_bounds_json(const std::string& path, const Volume& v) {
   // picojson serialises a std::map (keys sorted) and numbers as "%.f" when integral below 2^53, else "%.17g"
   auto num = [](double x) {
@@ -371,6 +437,18 @@ long fsio_debug_format_check(const double* v, long n, int decimals, long* first_
     if (std::strcmp(a, b) != 0) { if (!bad && first_bad) *first_bad = i; bad++; }
   }
   return bad;
+}
+
+// test hook: out[i] = strtof of in[i] as the .csv.gz writer formats it with `decimals` decimals (six when negative) --
+// the values the matcher's reader returns from that text; the reference for fs_get_points_as_read
+void fsio_debug_as_read(const double* in, long n, int decimals, float* out) {
+  const int dec = decimals >= 0 ? decimals : 6;
+#pragma omp parallel for schedule(static)
+  for (long i = 0; i < n; i++) {
+    char a[512];
+    a[fsio::format_fixed(in[i], dec, a, sizeof a - 1)] = 0;
+    out[i] = std::strtof(a, nullptr);
+  }
 }
 
 int fsio_write_bounds_json(const char* path, const int* dims, const double* spacing, const double* origin) {

@@ -2,6 +2,7 @@
 #pragma once
 
 #include <cstdint>
+#include <cstdio>
 #include <string>
 #include <vector>
 
@@ -20,7 +21,8 @@ struct Volume {
 // Uncompressed little-endian MetaImage, one component, element types MET_UCHAR / MET_SHORT / MET_USHORT / MET_INT /
 // MET_FLOAT, data in the same file (ElementDataFile = LOCAL) or in the named file next to the header.  Axis flips for
 // negative TransformMatrix diagonals (vtkRobustImageReader.h:52-60, 97-113) are applied.
-bool read_metaimage(const std::string& path, Volume& out, std::string& err);
+// (`warnings`: where the reader's axis-flip notices go; bin/surf3d prints them on stdout like the reference.)
+bool read_metaimage(const std::string& path, Volume& out, std::string& err, FILE* warnings = stdout);
 bool write_metaimage(const std::string& path, const Volume& v, std::string& err);
 
 // vtk3DSURF::WritePointsCSV / WritePointsCSVGZ / WritePointsBinary (vtk3DSURF.cxx:405-525): voxel-unit keypoints are
@@ -38,6 +40,27 @@ bool write_points_bin(const std::string& path, const fs_point* pts, const float*
 // reports as "outside image" (they are kept).
 bool read_points_file(const std::string& path, const double spacing[3], const double origin[3], const int dims[3],
                       std::vector<float>& xyzs, size_t& n_outside, std::string& err);
+
+// bin/surf3d's options (surf3d.cxx:16-157), shared with bin/match's -surf3d key so that the two cannot drift apart.
+struct SurfOptions {
+  double spacing = 0, threshold = 0;
+  int maxSize = 0, writeJSON = 0, writeBIN = 0, writeCSV = 0, writeCSVGZ = 1, descriptorType = 0, numberOfPoints = -1;
+  int pad = 0, subVolumeRadius = 5, precision = -1, gpu = 0;
+  const char *maskfilename = nullptr, *pointFile = nullptr, *gzOpts = nullptr;
+  bool clampMinValues = false, clampMaxValues = false, normalize = true;
+  float clampMinValue = 0, clampMaxValue = 0;
+  std::string outfilename = "points";
+};
+// The reference's option loop over argv[first ..): every key consumes two tokens, unknown keys are ignored.  The
+// strings stay argv's.
+void parse_surf_options(int argc, char* const argv[], int first, SurfOptions& o);
+// Options that need a VTK image filter this build does not restate (-s / -d, -m, -pad, -type 2) or picojson
+// (-json 1): the one to name in the refusal, nullptr when there is none.
+const char* unsupported_surf_option(const SurfOptions& o);
+// the refusal both executables print for it before leaving with exit code 7
+std::string unsupported_surf_message(const char* what);
+// -cmin / -cmax: vtkImageThreshold with ReplaceOut (surf3d.cxx:232-255) on the volume as read
+void clamp_volume(Volume& v, const SurfOptions& o);
 
 // surf3d.cxx:269-285: {"bounds":{"xmax":..,"xmin":..,...}} in picojson's number format
 bool write_bounds_json(const std::string& path, const Volume& v);

@@ -21,20 +21,10 @@ namespace {
 double now() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
 int unsupported(const char* what) {
-  std::cerr << "surf3d (B200): " << what << " needs a VTK image filter that this build does not restate; terminating." << endl;
+  std::cerr << fsio::unsupported_surf_message(what) << endl;
   return 7;
 }
 
-template <typename T>
-void clamp_values(std::vector<unsigned char>& data, bool lo_on, float lo, bool hi_on, float hi) {
-  // vtkImageThreshold with ReplaceOut (surf3d.cxx:232-255): values below -cmin become cmin, above -cmax become cmax
-  T* p = reinterpret_cast<T*>(data.data());
-  const size_t n = data.size() / sizeof(T);
-  for (size_t i = 0; i < n; i++) {
-    if (lo_on && (double)p[i] < (double)lo) p[i] = (T)lo;
-    if (hi_on && (double)p[i] > (double)hi) p[i] = (T)hi;
-  }
-}
 }  // namespace
 
 int main(int argc, char* argv[]) {
@@ -61,45 +51,9 @@ int main(int argc, char* argv[]) {
     exit(1);
   }
 
-  double spacing = 0, threshold = 0;
-  int maxSize = 0, writeJSON = 0, writeBIN = 0, writeCSV = 0, writeCSVGZ = 1, descriptorType = 0, numberOfPoints = -1;
-  int pad = 0, subVolumeRadius = 5, precision = -1, gpu = 0;
-  char *maskfilename = 0, *pointFile = 0, *gzOpts = 0;
-  bool clampMinValues = false, clampMaxValues = false, normalize = true;
-  float clampMinValue = 0, clampMaxValue = 0;
-  std::string outfilename("points");
-
-  int argumentsIndex = 2;
-  while (argumentsIndex < argc) {
-    char* key = argv[argumentsIndex];
-    char* value = argumentsIndex + 1 < argc ? argv[argumentsIndex + 1] : (char*)"";
-    if (strcmp(key, "-d") == 0) maxSize = atoi(value);
-    if (strcmp(key, "-s") == 0) spacing = atof(value);
-    if (strcmp(key, "-t") == 0) threshold = atof(value);
-    if (strcmp(key, "-cmin") == 0) { clampMinValues = true; clampMinValue = atof(value); }
-    if (strcmp(key, "-cmax") == 0) { clampMaxValues = true; clampMaxValue = atof(value); }
-    if (strcmp(key, "-m") == 0) maskfilename = value;
-    if (strcmp(key, "-o") == 0) outfilename = value;
-    if (strcmp(key, "-json") == 0) writeJSON = atoi(value);
-    if (strcmp(key, "-csv") == 0) writeCSV = atoi(value);
-    if (strcmp(key, "-bin") == 0) writeBIN = atoi(value);
-    if (strcmp(key, "-csvgz") == 0) writeCSVGZ = atoi(value);
-    if (strcmp(key, "-type") == 0) descriptorType = atoi(value);
-    if (strcmp(key, "-n") == 0) numberOfPoints = atoi(value);
-    if (strcmp(key, "-p") == 0) pointFile = value;
-    if (strcmp(key, "-r") == 0) subVolumeRadius = atoi(value);
-    if (strcmp(key, "-normalize") == 0) normalize = atoi(value);
-    if (strcmp(key, "-pad") == 0) pad = atoi(value);
-    if (strcmp(key, "-gz") == 0) gzOpts = value;
-    if (strcmp(key, "-precision") == 0) precision = atoi(value);
-    if (strcmp(key, "-gpu") == 0) gpu = atoi(value);
-    argumentsIndex += 2;
-  }
-  if (spacing != 0 || maxSize > 0) return unsupported("-s / -d (vtkImageResample)");
-  if (maskfilename) return unsupported("-m (mask resampling)");
-  if (pad) return unsupported("-pad (vtkImageMirrorPad)");
-  if (descriptorType == 2) return unsupported("-type 2 (vtkImageResize)");
-  if (writeJSON) return unsupported("-json 1 (picojson point dump)");
+  fsio::SurfOptions o;
+  fsio::parse_surf_options(argc, argv, 2, o);
+  if (const char* what = fsio::unsupported_surf_option(o)) return unsupported(what);
 
   cout << "load : " << argv[1] << endl;
   double t0 = now();
@@ -110,20 +64,12 @@ int main(int argc, char* argv[]) {
     std::cerr << err << endl;
     return 5;
   }
-  if (clampMinValues || clampMaxValues) {
-    switch (vol.voxel_type) {
-      case FS_U8: clamp_values<uint8_t>(vol.data, clampMinValues, clampMinValue, clampMaxValues, clampMaxValue); break;
-      case FS_I16: clamp_values<int16_t>(vol.data, clampMinValues, clampMinValue, clampMaxValues, clampMaxValue); break;
-      case FS_U16: clamp_values<uint16_t>(vol.data, clampMinValues, clampMinValue, clampMaxValues, clampMaxValue); break;
-      case FS_I32: clamp_values<int32_t>(vol.data, clampMinValues, clampMinValue, clampMaxValues, clampMaxValue); break;
-      default: clamp_values<float>(vol.data, clampMinValues, clampMinValue, clampMaxValues, clampMaxValue); break;
-    }
-  }
+  fsio::clamp_volume(vol, o);
   cout << "Image loaded in " << now() - t0 << "s" << endl;
-  fsio::write_bounds_json(outfilename + ".json", vol);
+  fsio::write_bounds_json(o.outfilename + ".json", vol);
 
   fs_ctx* ctx = nullptr;
-  if (fs_create(gpu, &ctx) != FS_OK) {
+  if (fs_create(o.gpu, &ctx) != FS_OK) {
     std::cerr << "surf3d (B200): " << fs_last_error(nullptr) << endl;
     return 1;
   }
@@ -140,12 +86,12 @@ int main(int argc, char* argv[]) {
   cout << "Integral computed in " << now() - t0 << "s" << endl;
   t0 = now();
   uint32_t n = 0;
-  if (pointFile) {  // vtk3DSURF.cxx:183: ReadIPoints instead of the detector
-    cout << "Use points in " << pointFile << endl;
-    cout << "Read : " << pointFile << endl;
+  if (o.pointFile) {  // vtk3DSURF.cxx:183: ReadIPoints instead of the detector
+    cout << "Use points in " << o.pointFile << endl;
+    cout << "Read : " << o.pointFile << endl;
     std::vector<float> xyzs;
     size_t outside = 0;
-    if (!fsio::read_points_file(pointFile, vol.spacing, vol.origin, vol.dims, xyzs, outside, err)) {
+    if (!fsio::read_points_file(o.pointFile, vol.spacing, vol.origin, vol.dims, xyzs, outside, err)) {
       std::cerr << "surf3d (B200): " << err << endl;
       fs_destroy(ctx);
       return 1;
@@ -154,14 +100,14 @@ int main(int argc, char* argv[]) {
     n = (uint32_t)(xyzs.size() / 4);
     if (fs_set_points(ctx, xyzs.data(), n) != FS_OK) return die("points");
   } else {
-    if (fs_detect(ctx, (float)threshold, &n) != FS_OK) return die("detector");
+    if (fs_detect(ctx, (float)o.threshold, &n) != FS_OK) return die("detector");
     cout << " Ipoints : " << n << endl;
     cout << "FastHessian computed in " << now() - t0 << "s" << endl;
   }
   t0 = now();
-  if (fs_select(ctx, numberOfPoints) != FS_OK) return die("select");
+  if (fs_select(ctx, o.numberOfPoints) != FS_OK) return die("select");
   uint32_t dsize = 0;
-  if (fs_describe(ctx, descriptorType, subVolumeRadius, normalize) != FS_OK) return die("descriptors");
+  if (fs_describe(ctx, o.descriptorType, o.subVolumeRadius, o.normalize) != FS_OK) return die("descriptors");
   fs_num_points(ctx, &n, &dsize);
   cout << "Number of keypoints : " << n << endl;
   std::vector<fs_point> pts(n);
@@ -174,19 +120,19 @@ int main(int argc, char* argv[]) {
   if (st.n_clamped) cout << "Warning : " << st.n_clamped << " keypoints have descriptor windows leaving the volume" << endl;
   fs_destroy(ctx);
 
-  if (writeBIN) {
+  if (o.writeBIN) {
     t0 = now();
-    fsio::write_points_bin(outfilename + ".bin", pts.data(), desc.data(), n, dsize, vol.spacing, vol.origin);
+    fsio::write_points_bin(o.outfilename + ".bin", pts.data(), desc.data(), n, dsize, vol.spacing, vol.origin);
     cout << "bin written in " << now() - t0 << "s" << endl;
   }
-  if (writeCSV) {
+  if (o.writeCSV) {
     t0 = now();
-    fsio::write_points_csv(outfilename + ".csv", pts.data(), desc.data(), n, dsize, vol.spacing, vol.origin);
+    fsio::write_points_csv(o.outfilename + ".csv", pts.data(), desc.data(), n, dsize, vol.spacing, vol.origin);
     cout << "csv written in " << now() - t0 << "s" << endl;
   }
-  if (writeCSVGZ) {
+  if (o.writeCSVGZ) {
     t0 = now();
-    fsio::write_points_csvgz(outfilename + ".csv.gz", gzOpts, precision, pts.data(), desc.data(), n, dsize, vol.spacing, vol.origin);
+    fsio::write_points_csvgz(o.outfilename + ".csv.gz", o.gzOpts, o.precision, pts.data(), desc.data(), n, dsize, vol.spacing, vol.origin);
     cout << "csvgz written in " << now() - t0 << "s" << endl;
   }
   return 0;

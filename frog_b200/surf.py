@@ -15,7 +15,7 @@ from . import build
 
 PUBLIC_SYMBOLS = [
     "fs_device_count", "fs_create", "fs_destroy", "fs_last_error", "fs_version", "fs_set_volume", "fs_detect",
-    "fs_select", "fs_set_points", "fs_describe", "fs_num_points", "fs_get_points", "fs_get_stats",
+    "fs_select", "fs_set_points", "fs_describe", "fs_num_points", "fs_get_points", "fs_get_points_as_read", "fs_get_stats",
     "fs_get_cast_volume", "fs_get_integral", "fs_num_layers", "fs_get_layer",
 ]
 
@@ -58,6 +58,7 @@ def load():
     L.fs_describe.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int]
     L.fs_num_points.argtypes = [C.c_void_p, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]
     L.fs_get_points.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+    L.fs_get_points_as_read.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.fs_get_stats.argtypes = [C.c_void_p, C.POINTER(Stats)]
     L.fs_get_cast_volume.argtypes = [C.c_void_p, C.c_void_p]
     L.fs_get_integral.argtypes = [C.c_void_p, C.c_void_p]
@@ -73,6 +74,7 @@ def load():
     L.fs_debug_keep_cast_volume.argtypes = [C.c_void_p, C.c_int]
     L.fs_debug_set_option.argtypes = [C.c_char_p, C.c_int]
     L.fs_debug_sort_keys.argtypes = [C.c_void_p, C.c_uint32, C.c_void_p]
+    L.fs_debug_as_read.argtypes = [C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]
     L.fs_debug_select.restype = C.c_uint32
     L.fs_debug_select.argtypes = [C.c_void_p, C.c_uint32, C.c_int, C.c_void_p]
     _lib = L
@@ -138,6 +140,19 @@ class Producer:
         desc = np.zeros((n.value, d.value), np.float32) if with_descriptors and d.value else None
         self._check(self._L.fs_get_points(self._h, pts.ctypes.data, desc.ctypes.data if desc is not None and n.value else None))
         return pts, desc
+
+    def points_as_read(self, precision: int = -1, spacing=(1.0, 1.0, 1.0), origin=(0.0, 0.0, 0.0)):
+        """(head [n, 6], desc [n, d]) float32: the keypoints exactly as the .csv.gz reader returns them from the file
+        surf3d writes for a volume of this spacing / origin at -precision `precision` (converted on the device)."""
+        n, d = C.c_uint32(), C.c_uint32()
+        self._check(self._L.fs_num_points(self._h, C.byref(n), C.byref(d)))
+        head = np.zeros((n.value, 6), np.float32)
+        desc = np.zeros((n.value, d.value), np.float32)
+        sp = np.asarray(spacing, np.float64)
+        org = np.asarray(origin, np.float64)
+        self._check(self._L.fs_get_points_as_read(self._h, precision, sp.ctypes.data, org.ctypes.data, head.ctypes.data,
+                                                  desc.ctypes.data))
+        return head, desc
 
     def stats(self) -> dict:
         s = Stats()
@@ -221,6 +236,16 @@ def debug_layers(nx, ny, nz) -> np.ndarray:
     return out[:n]
 
 
+def debug_as_read(values: np.ndarray, precision: int) -> np.ndarray:
+    """fs_get_points_as_read's conversion of float64 values on device 0 (float32 results; needs a GPU)."""
+    v = np.ascontiguousarray(values, np.float64)
+    out = np.zeros(v.shape, np.float32)
+    rc = load().fs_debug_as_read(v.ctypes.data, v.size, precision, out.ctypes.data)
+    if rc != 0:
+        raise FrogSurfError(f"fs_debug_as_read: status {rc}")
+    return out
+
+
 def debug_select(response: np.ndarray, number_of_points: int) -> np.ndarray:
     L = load()
     r = np.ascontiguousarray(response, np.float32)
@@ -244,6 +269,7 @@ def _io():
         L.fsio_read_metaimage.argtypes = [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                           C.c_size_t, C.c_void_p]
         L.fsio_write_bounds_json.argtypes = [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p]
+        L.fsio_debug_as_read.argtypes = [C.c_void_p, C.c_long, C.c_int, C.c_void_p]
         L.fsio_read_points.restype = C.c_long
         L.fsio_read_points.argtypes = [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_long, C.c_void_p]
         _fsio = L
@@ -262,6 +288,14 @@ def write_points(path: str, fmt: str, pts: np.ndarray, desc: np.ndarray, spacing
                                  org.ctypes.data)
     if rc != 0:
         raise FrogSurfError(f"cannot write {path}")
+
+
+def as_read_host(values: np.ndarray, precision: int) -> np.ndarray:
+    """strtof of each float64 value as the .csv.gz writer formats it at -precision `precision` (host, no CUDA)."""
+    v = np.ascontiguousarray(values, np.float64)
+    out = np.zeros(v.shape, np.float32)
+    _io().fsio_debug_as_read(v.ctypes.data, v.size, precision, out.ctypes.data)
+    return out
 
 
 def read_points_file(path: str, spacing, origin, shape):

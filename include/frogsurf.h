@@ -111,6 +111,18 @@ int fs_num_points(fs_ctx* ctx, uint32_t* n, uint32_t* descriptor_size);
 /* Copy the keypoints (n fs_point) and, when desc != NULL, their descriptors (n * descriptor_size floats) to the host. */
 int fs_get_points(fs_ctx* ctx, fs_point* points, float* desc);
 
+/*
+ * The current keypoints and descriptors exactly as the matcher's .csv / .csv.gz reader returns them from the file that
+ * surf3d's writer formats (vtk3DSURF::WritePointsCSVGZ): head = n x 6 floats (x * spacing + origin, y.., z..,
+ * scale * cbrt(spacing product), laplacian, response), desc = n x descriptor_size floats.  Every field is
+ * strtof of its fixed-decimal text: six decimals for the header fields, `precision` for the descriptors (six when
+ * negative).  spacing / origin: the volume's, as the MetaImage header gives them.  Converted on the device; values the
+ * text needs more than 64-bit integers for (|v| * 10^decimals >= 9e18, precision > 9, inf / nan) are finished on the
+ * host with snprintf + strtof.  FS_ERR_INVALID when a value's text is out of float range (the reader rejects it).
+ */
+int fs_get_points_as_read(fs_ctx* ctx, int precision, const double spacing[3], const double origin[3], float* head,
+                          float* desc);
+
 int fs_get_stats(fs_ctx* ctx, fs_stats* out);
 
 /* ---- stage outputs, for the parity tests ------------------------------------------------------ */

@@ -33,6 +33,9 @@ void fs_debug_sort_keys(const uint64_t* keys, uint32_t n, uint32_t* order);
 int fs_debug_set_option(const char* name, int value);
 struct fs_ctx;
 void fs_debug_keep_cast_volume(struct fs_ctx* ctx, int on);
+/* fs_get_points_as_read's conversion of n given values at `precision` decimals (six when negative), on device 0 (needs a
+ * GPU): out[i] = strtof of in[i]'s fixed-decimal text */
+int fs_debug_as_read(const double* in, size_t n, int precision, float* out);
 
 #ifdef __cplusplus
 }
