@@ -31,8 +31,10 @@ PUBLIC_SYMBOLS = [
     "fm_links_device_data", "fm_links_build_ms", "fm_links_free",
 ]
 DEBUG_SYMBOLS = ["fm_debug_image", "fm_debug_image_norms", "fm_debug_score_unit", "fm_debug_set_option",
-                 "fm_debug_reject_rows", "fm_debug_wide_unit"]
+                 "fm_debug_reject_rows", "fm_debug_wide_unit", "fm_debug_compact"]
 ERR_INVALID = -1  # FM_ERR_INVALID
+# fm_debug_compact paths (include/frogmatch_debug.h)
+COMPACT_AUTO, COMPACT_ONE, COMPACT_THREE, COMPACT_LOOKALL = 0, 1, 2, 3
 
 
 class Stats(C.Structure):
@@ -103,6 +105,8 @@ def load():
     L.fm_debug_set_option.argtypes = [C.c_char_p, C.c_int]
     L.fm_debug_reject_rows.argtypes = [vp, C.c_uint32, C.c_uint32, vp, vp, vp, vp, u32p]
     L.fm_debug_wide_unit.argtypes = [vp, C.c_uint32, C.c_uint32, C.c_uint32, vp, C.c_uint32, vp, vp, vp, f32p, u32p]
+    L.fm_debug_compact.argtypes = [vp, vp, vp, C.c_uint32, vp, C.c_uint32, C.c_int, C.c_uint64, vp, vp, C.c_uint64,
+                                   vp, C.c_uint32, C.POINTER(C.c_uint64), vp, u32p]
     L.fm_links_build.argtypes = [vp, vp, vp, vp, C.POINTER(vp)]
     L.fm_links_total.argtypes = [vp]
     L.fm_links_total.restype = C.c_uint64
@@ -364,6 +368,29 @@ class Matcher:
             return None
         self._check(rc)
         return dict(args=args[:n_rows], rowstat=stat[:n_rows], bands=bands[:n_rows], survivors=surv[:ns.value])
+
+    def debug_compact(self, rowres, chunks, path: int, base: int, out_pairs, pair_counts, rowdist=None, out_dist=None,
+                      epoch=None, status: bool = False) -> dict:
+        """One batch's compaction through the library's launch routine on this context (fm_debug_compact).
+        rowres [n] uint32 (0xFFFFFFFF = no match), chunks [k, 4] uint32 records, path COMPACT_*, out_pairs [slots, 2]
+        uint32 and pair_counts uint32 are in/out (updated in place), as is out_dist [slots] float32 with rowdist.
+        epoch: set the context's launch epoch counter first.  Returns dict(total, epoch, status) -- status the 1536
+        look-back words when asked for.  FrogMatchError when the library refuses the arguments."""
+        rowres = np.ascontiguousarray(rowres, np.uint32)
+        chunks = np.ascontiguousarray(chunks, np.uint32).reshape(-1, 4)
+        assert out_pairs.dtype == np.uint32 and out_pairs.flags.c_contiguous and out_pairs.ndim == 2
+        assert pair_counts.dtype == np.uint32 and pair_counts.flags.c_contiguous
+        rd = None if rowdist is None else np.ascontiguousarray(rowdist, np.float32)
+        if out_dist is not None:
+            assert out_dist.dtype == np.float32 and out_dist.flags.c_contiguous
+        total = C.c_uint64()
+        ep = C.c_uint32(0 if epoch is None else epoch)
+        st = np.zeros(1536, np.uint64) if status else None
+        self._check(self._L.fm_debug_compact(
+            self._h, _ptr(rowres), None if rd is None else _ptr(rd), rowres.shape[0], _ptr(chunks), chunks.shape[0], path,
+            base, _ptr(out_pairs), None if out_dist is None else _ptr(out_dist), out_pairs.shape[0], _ptr(pair_counts),
+            pair_counts.shape[0], C.byref(total), None if st is None else _ptr(st), C.byref(ep) if epoch is not None else None))
+        return dict(total=total.value, epoch=ep.value if epoch is not None else None, status=st)
 
 
 def debug_set_option(name: str, value: int) -> None:

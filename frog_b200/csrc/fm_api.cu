@@ -189,6 +189,69 @@ struct Batch {
   bool any_exact, any_fast;
 };
 
+// The look-back status words of the one-pass compaction kernel: fresh memory may hold anything, so it is cleared once
+// here; afterwards the launch epoch tells stale words from current ones (and compact_launch clears the words again
+// whenever the epoch counter wraps).
+cudaError_t ensure_chunk_status(fm_ctx* c) {
+  if (c->d_chunk_status.p) return cudaSuccess;
+  cudaError_t e = c->d_chunk_status.ensure((size_t)kOnePassChunks * sizeof(unsigned long long));
+  if (e != cudaSuccess) return e;
+  return cudaMemsetAsync(c->d_chunk_status.p, 0, c->d_chunk_status.cap, c->stream);
+}
+
+// Compaction of one batch (fm_compact.cuh) on the context stream: `ca` carries the batch's chunks, rows and outputs;
+// the context's scratch (d_chunk_count / d_chunk_out / d_chunk_stage, sized for ca.n_chunks, and d_chunk_status) and
+// its epoch counter are filled in here.  `path` is an FM_COMPACT_* value (include/frogmatch_debug.h): fm_match passes
+// FM_COMPACT_AUTO, fm_debug_compact whatever the test asks for.  Returns the number of kernel launches.
+uint32_t compact_launch(fm_ctx* c, CompactArgs ca, bool want_dist, int path) {
+  ca.chunk_count = c->d_chunk_count.as<uint32_t>();
+  ca.chunk_out = c->d_chunk_out.as<unsigned long long>();
+  ca.stage = c->d_chunk_stage.as<uint2>();
+  if (path == FM_COMPACT_AUTO) path = ca.n_chunks <= kOnePassChunks ? FM_COMPACT_ONE : FM_COMPACT_THREE;
+  if (path == FM_COMPACT_ONE || path == FM_COMPACT_LOOKALL) {
+    ca.status = c->d_chunk_status.as<unsigned long long>();
+    const uint32_t prev = c->compact_epoch;
+    c->compact_epoch = (c->compact_epoch % 0x3FFFFFFEu) + 1u;  // 1 .. 2^30 - 2: never the cleared value 0
+    // Back at epoch 1 after a wrap: words an earlier epoch-1 launch left past the chunks later launches rewrote would
+    // pass for current ones.  (A failure here is left to the caller's cudaGetLastError.)
+    if (c->compact_epoch == 1u && prev != 0u) cudaMemsetAsync(c->d_chunk_status.p, 0, c->d_chunk_status.cap, c->stream);
+    ca.epoch = c->compact_epoch;
+    if (path == FM_COMPACT_LOOKALL) {
+      if (want_dist) compact_onepass_kernel<true, true><<<ca.n_chunks, kCompactThreads, 0, c->stream>>>(ca);
+      else compact_onepass_kernel<false, true><<<ca.n_chunks, kCompactThreads, 0, c->stream>>>(ca);
+    } else {
+      if (want_dist) compact_onepass_kernel<true><<<ca.n_chunks, kCompactThreads, 0, c->stream>>>(ca);
+      else compact_onepass_kernel<false><<<ca.n_chunks, kCompactThreads, 0, c->stream>>>(ca);
+    }
+    return 1;
+  }
+  const uint32_t grid = std::min<uint32_t>(ca.n_chunks, (uint32_t)c->sm_count * 8u);  // grid-stride over the chunks
+  if (g_debug.compact_v >= 2) {
+    // persistent, software-pipelined count pass: three CTAs per SM, each with the next chunk's rows in flight
+    const uint32_t grid_count = std::min<uint32_t>(ca.n_chunks, (uint32_t)c->sm_count * 3u);
+    if (want_dist) {
+      if (g_debug.compact_v >= 3) compact_count3_kernel<true><<<grid_count, kCompactThreads, 0, c->stream>>>(ca);
+      else compact_count2_kernel<true><<<grid_count, kCompactThreads, 0, c->stream>>>(ca);
+      compact_scan2_kernel<<<1, 1024, 0, c->stream>>>(ca);
+      compact_scatter2_kernel<true><<<grid, kCompactThreads, 0, c->stream>>>(ca);
+    } else {
+      if (g_debug.compact_v >= 3) compact_count3_kernel<false><<<grid_count, kCompactThreads, 0, c->stream>>>(ca);
+      else compact_count2_kernel<false><<<grid_count, kCompactThreads, 0, c->stream>>>(ca);
+      compact_scan2_kernel<<<1, 1024, 0, c->stream>>>(ca);
+      compact_scatter2_kernel<false><<<grid, kCompactThreads, 0, c->stream>>>(ca);
+    }
+  } else if (want_dist) {
+    compact_count_kernel<true><<<ca.n_chunks, kCompactThreads, 0, c->stream>>>(ca);  // (one CTA per chunk measured faster here)
+    compact_scan_kernel<<<1, 1024, 0, c->stream>>>(ca);
+    compact_scatter_kernel<true><<<grid, kCompactThreads, 0, c->stream>>>(ca);
+  } else {
+    compact_count_kernel<false><<<ca.n_chunks, kCompactThreads, 0, c->stream>>>(ca);
+    compact_scan_kernel<<<1, 1024, 0, c->stream>>>(ca);
+    compact_scatter_kernel<false><<<grid, kCompactThreads, 0, c->stream>>>(ca);
+  }
+  return 3;
+}
+
 }  // namespace
 
 extern "C" {
@@ -515,11 +578,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
   FM_CUDA_R(c->d_chunk_count.ensure((size_t)max_chunks * sizeof(uint32_t)));
   FM_CUDA_R(c->d_chunk_out.ensure((size_t)max_chunks * sizeof(unsigned long long)));
   FM_CUDA_R(c->d_chunk_stage.ensure((size_t)max_chunks * kStageCap * sizeof(uint2)));
-  if (!c->d_chunk_status.p) {
-    // fresh memory may hold anything: clear it once, then the launch epoch tells stale words from current ones
-    FM_CUDA_R(c->d_chunk_status.ensure((size_t)kOnePassChunks * sizeof(unsigned long long)));
-    FM_CUDA_R(cudaMemsetAsync(c->d_chunk_status.p, 0, c->d_chunk_status.cap, c->stream));
-  }
+  FM_CUDA_R(ensure_chunk_status(c));
   FM_CUDA_R(c->d_totals.ensure(sizeof(DeviceCounters)));
   FM_CUDA_R(r->d_out.ensure(std::max<uint64_t>(total_rows, 1) * sizeof(uint2)));
   FM_CUDA_R(r->d_counts.ensure(std::max<size_t>(n_pairs, 1) * sizeof(uint32_t)));
@@ -658,49 +717,11 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
         ca.n_chunks = b.chunks;
         ca.rowres = d_rowres;
         ca.rowdist = d_rowdist;
-        ca.chunk_count = c->d_chunk_count.as<uint32_t>();
-        ca.chunk_out = c->d_chunk_out.as<unsigned long long>();
-        ca.stage = c->d_chunk_stage.as<uint2>();
         ca.pair_count = r->d_counts.as<uint32_t>();
         ca.running_total = &d_counters->running_total;
         ca.out_pairs = r->d_out.as<uint2>();
         ca.out_dist = want_dist ? r->d_dist.as<float>() : nullptr;
-        if (b.chunks <= kOnePassChunks) {
-          ca.status = c->d_chunk_status.as<unsigned long long>();
-          c->compact_epoch = (c->compact_epoch % 0x3FFFFFFEu) + 1u;  // 1 .. 2^30 - 2: never the cleared value 0
-          ca.epoch = c->compact_epoch;
-          if (want_dist) compact_onepass_kernel<true><<<b.chunks, kCompactThreads, 0, c->stream>>>(ca);
-          else compact_onepass_kernel<false><<<b.chunks, kCompactThreads, 0, c->stream>>>(ca);
-          c->stats.kernel_launches += 1;
-        } else if (g_debug.compact_v >= 2) {
-          // persistent, software-pipelined count pass: three CTAs per SM, each with the next chunk's rows in flight
-          const uint32_t grid_count = std::min<uint32_t>(b.chunks, (uint32_t)c->sm_count * 3u);
-          const uint32_t grid = std::min<uint32_t>(b.chunks, (uint32_t)c->sm_count * 8u);
-          if (want_dist) {
-            if (g_debug.compact_v >= 3) compact_count3_kernel<true><<<grid_count, kCompactThreads, 0, c->stream>>>(ca);
-            else compact_count2_kernel<true><<<grid_count, kCompactThreads, 0, c->stream>>>(ca);
-            compact_scan2_kernel<<<1, 1024, 0, c->stream>>>(ca);
-            compact_scatter2_kernel<true><<<grid, kCompactThreads, 0, c->stream>>>(ca);
-          } else {
-            if (g_debug.compact_v >= 3) compact_count3_kernel<false><<<grid_count, kCompactThreads, 0, c->stream>>>(ca);
-            else compact_count2_kernel<false><<<grid_count, kCompactThreads, 0, c->stream>>>(ca);
-            compact_scan2_kernel<<<1, 1024, 0, c->stream>>>(ca);
-            compact_scatter2_kernel<false><<<grid, kCompactThreads, 0, c->stream>>>(ca);
-          }
-          c->stats.kernel_launches += 3;
-        } else if (want_dist) {
-          const uint32_t grid = std::min<uint32_t>(b.chunks, (uint32_t)c->sm_count * 8u);  // grid-stride over the chunks
-          compact_count_kernel<true><<<b.chunks, kCompactThreads, 0, c->stream>>>(ca);  // (one CTA per chunk measured faster here)
-          compact_scan_kernel<<<1, 1024, 0, c->stream>>>(ca);
-          compact_scatter_kernel<true><<<grid, kCompactThreads, 0, c->stream>>>(ca);
-          c->stats.kernel_launches += 3;
-        } else {
-          const uint32_t grid = std::min<uint32_t>(b.chunks, (uint32_t)c->sm_count * 8u);
-          compact_count_kernel<false><<<b.chunks, kCompactThreads, 0, c->stream>>>(ca);
-          compact_scan_kernel<<<1, 1024, 0, c->stream>>>(ca);
-          compact_scatter_kernel<false><<<grid, kCompactThreads, 0, c->stream>>>(ca);
-          c->stats.kernel_launches += 3;
-        }
+        c->stats.kernel_launches += compact_launch(c, ca, want_dist, FM_COMPACT_AUTO);
       }
       if (two_phase_possible && !two_phase && !probed && b.any_fast && !b.any_exact && bi + 1 < batches.size() &&
           !(flags & FM_FLAG_ASYNC)) {
@@ -1111,6 +1132,87 @@ int fm_debug_reject_rows(fm_ctx* c, uint32_t task, uint32_t n_rows, float* args,
   if (bands && n_rows) memcpy(bands, st.bands.data(), (size_t)n_rows * sizeof(uint2));
   if (survivors && !st.survivors.empty()) memcpy(survivors, st.survivors.data(), st.survivors.size() * sizeof(uint32_t));
   if (n_survivors) *n_survivors = (uint32_t)st.survivors.size();
+  return FM_OK;
+}
+
+int fm_debug_compact(fm_ctx* c, const uint32_t* rowres, const float* rowdist, uint32_t n_rows, const uint32_t* chunks,
+                     uint32_t n_chunks, int path, uint64_t base, uint32_t* out_pairs, float* out_dist, uint64_t out_slots,
+                     uint32_t* pair_counts, uint32_t n_pairs, uint64_t* total_out, uint64_t* status_out,
+                     uint32_t* epoch_inout) {
+  if (!c) return FM_ERR_INVALID;
+  if (path < FM_COMPACT_AUTO || path > FM_COMPACT_LOOKALL || n_chunks == 0 || !chunks || !out_pairs || !pair_counts ||
+      (n_rows && !rowres) || (rowdist && !out_dist))
+    return fail(c, FM_ERR_INVALID, "fm_debug_compact: bad path or missing argument");
+  if ((path == FM_COMPACT_ONE || path == FM_COMPACT_LOOKALL) && n_chunks > kOnePassChunks)
+    return fail(c, FM_ERR_INVALID, "fm_debug_compact: one launch takes at most 1536 chunks");
+  const bool want_dist = rowdist != nullptr;
+  uint64_t total = 0;
+  for (uint32_t k = 0; k < n_chunks; k++) {
+    const ChunkDesc d{chunks[4 * k], chunks[4 * k + 1], chunks[4 * k + 2], chunks[4 * k + 3]};
+    const uint32_t n = d.n_swap & 0x7FFFFFFFu;
+    if (n > (uint32_t)kCompactChunk || (uint64_t)d.row_abs + n > n_rows || d.pair >= n_pairs)
+      return fail(c, FM_ERR_INVALID, "fm_debug_compact: a chunk has more than 4096 rows, reaches past n_rows or names no pair");
+    for (uint32_t i = 0; i < n; i++) total += rowres[d.row_abs + i] != kNone;
+  }
+  if (base + total > out_slots) return fail(c, FM_ERR_INVALID, "fm_debug_compact: base + matches exceeds out_slots");
+  FM_CUDA(c, cudaSetDevice(c->device));
+  DevBuf d_chunks, d_out, d_dist, d_counts, d_total;
+  auto release = [&] { d_chunks.release(); d_out.release(); d_dist.release(); d_counts.release(); d_total.release(); };
+#define FM_CUDA_H(expr)                                  \
+  do {                                                   \
+    cudaError_t e__ = (expr);                            \
+    if (e__ != cudaSuccess) {                            \
+      release();                                         \
+      return cuda_fail(c, e__, #expr);                   \
+    }                                                    \
+  } while (0)
+  FM_CUDA_H(c->d_rowres.ensure(std::max<size_t>(n_rows, 1) * sizeof(uint32_t)));
+  if (want_dist) FM_CUDA_H(c->d_rowdist.ensure(std::max<size_t>(n_rows, 1) * sizeof(float)));
+  FM_CUDA_H(c->d_chunk_count.ensure((size_t)n_chunks * sizeof(uint32_t)));
+  FM_CUDA_H(c->d_chunk_out.ensure((size_t)n_chunks * sizeof(unsigned long long)));
+  FM_CUDA_H(c->d_chunk_stage.ensure((size_t)n_chunks * kStageCap * sizeof(uint2)));
+  FM_CUDA_H(ensure_chunk_status(c));
+  FM_CUDA_H(d_chunks.ensure((size_t)n_chunks * sizeof(ChunkDesc)));
+  FM_CUDA_H(d_out.ensure(std::max<uint64_t>(out_slots, 1) * sizeof(uint2)));
+  if (want_dist) FM_CUDA_H(d_dist.ensure(std::max<uint64_t>(out_slots, 1) * sizeof(float)));
+  FM_CUDA_H(d_counts.ensure(std::max<size_t>(n_pairs, 1) * sizeof(uint32_t)));
+  FM_CUDA_H(d_total.ensure(sizeof(unsigned long long)));
+  const unsigned long long base_ull = base;
+  if (n_rows) FM_CUDA_H(cudaMemcpyAsync(c->d_rowres.p, rowres, (size_t)n_rows * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+  if (want_dist && n_rows)
+    FM_CUDA_H(cudaMemcpyAsync(c->d_rowdist.p, rowdist, (size_t)n_rows * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  FM_CUDA_H(cudaMemcpyAsync(d_chunks.p, chunks, (size_t)n_chunks * sizeof(ChunkDesc), cudaMemcpyHostToDevice, c->stream));
+  if (out_slots) FM_CUDA_H(cudaMemcpyAsync(d_out.p, out_pairs, out_slots * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
+  if (want_dist && out_slots)
+    FM_CUDA_H(cudaMemcpyAsync(d_dist.p, out_dist, out_slots * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+  if (n_pairs) FM_CUDA_H(cudaMemcpyAsync(d_counts.p, pair_counts, (size_t)n_pairs * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+  FM_CUDA_H(cudaMemcpyAsync(d_total.p, &base_ull, sizeof base_ull, cudaMemcpyHostToDevice, c->stream));
+  if (epoch_inout) c->compact_epoch = *epoch_inout;
+  CompactArgs ca{};
+  ca.chunks = d_chunks.as<ChunkDesc>();
+  ca.n_chunks = n_chunks;
+  ca.rowres = c->d_rowres.as<uint32_t>();
+  ca.rowdist = want_dist ? c->d_rowdist.as<float>() : nullptr;
+  ca.pair_count = d_counts.as<uint32_t>();
+  ca.running_total = d_total.as<unsigned long long>();
+  ca.out_pairs = d_out.as<uint2>();
+  ca.out_dist = want_dist ? d_dist.as<float>() : nullptr;
+  compact_launch(c, ca, want_dist, path);
+  FM_CUDA_H(cudaGetLastError());
+  unsigned long long total_dev = 0;
+  if (out_slots) FM_CUDA_H(cudaMemcpyAsync(out_pairs, d_out.p, out_slots * sizeof(uint2), cudaMemcpyDeviceToHost, c->stream));
+  if (want_dist && out_slots)
+    FM_CUDA_H(cudaMemcpyAsync(out_dist, d_dist.p, out_slots * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+  if (n_pairs) FM_CUDA_H(cudaMemcpyAsync(pair_counts, d_counts.p, (size_t)n_pairs * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+  FM_CUDA_H(cudaMemcpyAsync(&total_dev, d_total.p, sizeof total_dev, cudaMemcpyDeviceToHost, c->stream));
+  if (status_out)
+    FM_CUDA_H(cudaMemcpyAsync(status_out, c->d_chunk_status.p, (size_t)kOnePassChunks * sizeof(unsigned long long),
+                              cudaMemcpyDeviceToHost, c->stream));
+  FM_CUDA_H(cudaStreamSynchronize(c->stream));
+#undef FM_CUDA_H
+  release();
+  if (total_out) *total_out = total_dev;
+  if (epoch_inout) *epoch_inout = c->compact_epoch;
   return FM_OK;
 }
 

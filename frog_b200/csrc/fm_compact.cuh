@@ -56,7 +56,7 @@ struct CompactArgs {
   unsigned long long* running_total;  // matches written before this batch; += this batch's
   uint2* out_pairs;
   float* out_dist;                // kDist only
-  unsigned long long* status;     // one-pass kernel: n_chunks look-back words (never cleared: epoch-tagged)
+  unsigned long long* status;     // one-pass kernel: n_chunks look-back words (epoch-tagged; cleared when the epoch wraps)
   uint32_t epoch;                 // one-pass kernel: 30 bits, different from the previous launches that used `status`
 };
 
@@ -536,13 +536,16 @@ compact_scatter2_kernel(const CompactArgs a) {
 // ---- small batches: ONE launch -------------------------------------------------------------------------
 // Up to a wave or two of chunks the three launches above are launch latency and nothing else (C2: 19 us against 11).
 // Here a chunk obtains the exclusive prefix of the chunk totals by decoupled look-back over one 64-bit status word per
-// chunk (launch epoch | state | value: no clearing between launches; 1024 predecessors inspected per round).  CTAs of
+// chunk (launch epoch | state | value: no clearing between launches, only when the 30-bit epoch counter wraps back to
+// 1; 1024 predecessors inspected per round).  CTAs of
 // a 1-D grid are dispatched in index order, so a chunk's predecessors are always running or done (the assumption every
 // single-pass scan makes).  For large batches the look-back chain is what bounds this design (95-140 us per 24 M rows
 // in every variant measured), hence the three-launch form there.
 constexpr int kCompactLook = 4;  // status words inspected per thread and look-back round
 
-template <bool kDist>
+// kLookAll (test study, fm_debug_compact): every chunk but chunk 0 publishes only its aggregate, so chunk k sums all k
+// predecessors in ceil(k / 1024) look-back rounds -- the multi-round path that production batches rarely reach.
+template <bool kDist, bool kLookAll = false>
 __global__ void __launch_bounds__(kCompactThreads)
 compact_onepass_kernel(const CompactArgs a) {
   __shared__ uint32_t s_slice[kCompactSlices];  // slice totals, then their exclusive prefix
@@ -640,7 +643,7 @@ compact_onepass_kernel(const CompactArgs a) {
     }
     excl = s_sum;
     if (tid == 0) {
-      if (chunk != 0) status[chunk] = chunk_word(a.epoch, kChunkPrefix, excl + total);
+      if (!kLookAll && chunk != 0) status[chunk] = chunk_word(a.epoch, kChunkPrefix, excl + total);
       if (total) atomicAdd(a.pair_count + d.pair, total);
       if (chunk == a.n_chunks - 1) *a.running_total = base0 + excl + total;
     }

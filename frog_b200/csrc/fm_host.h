@@ -129,7 +129,9 @@ struct fm_ctx {
   uint32_t dim = 0;
   // per-call scratch
   fm::DevBuf d_meta_blob, d_rowres, d_rowdist, d_chunk_count, d_chunk_out, d_chunk_stage, d_chunk_status, d_totals;
-  uint32_t compact_epoch = 0;  // tags the look-back status words of a one-pass compaction launch (fm_compact.cuh)
+  // tags the look-back status words of a one-pass compaction launch (fm_compact.cuh); d_chunk_status is cleared when
+  // the buffer is allocated and each time this counter wraps back to 1 (compact_launch in fm_api.cu)
+  uint32_t compact_epoch = 0;
   fm::DevBuf d_bands, d_cands, d_redo, d_taskinfo;
   fm::DevBuf d_rowstat, d_surv;  // two-phase scoring: per-row rejection flags; survivor counts / unit prefix / lists
   // fm_debug_set_option("reject_dump", 1): per task of the most recent fm_match, what its reject pass computed

@@ -1,8 +1,8 @@
 /*
  * frogmatch_debug.h -- test hooks of libfrogmatch.so.  NOT part of the drop-in boundary: these
  * exist so tests/ can check each device stage (sort + class table, FP16 operand packing, the
- * tcgen05 score tile, gate bands, candidate capture, the reject pass's per-row bounds) against numpy
- * in isolation.
+ * tcgen05 score tile, gate bands, candidate capture, the reject pass's per-row bounds, compaction) against
+ * numpy in isolation.
  */
 #ifndef FROGMATCH_DEBUG_H_
 #define FROGMATCH_DEBUG_H_
@@ -77,6 +77,37 @@ int fm_debug_reject_rows(fm_ctx* ctx, uint32_t task, uint32_t n_rows, float* arg
                          uint32_t* survivors, uint32_t* n_survivors);
 
 /*
+ * Run ONE batch's compaction (the last device stage of fm_match: accepted rows -> dense per-pair lists) on
+ * caller-given data, through the launch routine fm_match uses, with the context's own scratch and look-back state
+ * (status words and launch epoch counter), so hook calls and fm_match calls share them as production calls do.
+ *   rowres[n_rows]   matched column per row, or 0xFFFFFFFF (no match)
+ *   rowdist[n_rows]  squared distance per row, or NULL for a compaction without distances
+ *   chunks[n_chunks * 4]  the 16-byte chunk records {row_abs, n_rows | swap << 31, row_local, pair} in output order
+ *                    (n_rows <= 4096; rows of rowres that no chunk covers are ignored)
+ *   path             FM_COMPACT_AUTO (fm_match's choice), FM_COMPACT_ONE (one launch, <= 1536 chunks),
+ *                    FM_COMPACT_THREE (count / scan / scatter, version set by the "compact_v" option) or
+ *                    FM_COMPACT_LOOKALL (one launch in which every chunk looks back all the way to chunk 0)
+ *   base             matches written before this batch (the running total on entry)
+ *   out_pairs[out_slots * 2], out_dist[out_slots] (out_dist required with rowdist): in/out -- uploaded first, so
+ *                    slots outside [base, base + matches) come back as the caller left them unless a kernel wrote there
+ *   pair_counts[n_pairs]  in/out: each chunk's matches are added to its pair's count
+ *   total_out        running total after the call (may be NULL)
+ *   status_out[1536] the one-pass look-back status words after the call (may be NULL)
+ *   epoch_inout      in/out launch epoch counter of the context (may be NULL); the next one-launch call uses
+ *                    *epoch_inout % (2^30 - 2) + 1
+ * Returns FM_ERR_INVALID, before any launch, for a chunk of more than 4096 rows, one reaching past n_rows or naming a
+ * pair >= n_pairs, no chunks, a one-launch path with more than 1536 chunks, or base + matches > out_slots.
+ */
+#define FM_COMPACT_AUTO 0
+#define FM_COMPACT_ONE 1
+#define FM_COMPACT_THREE 2
+#define FM_COMPACT_LOOKALL 3
+int fm_debug_compact(fm_ctx* ctx, const uint32_t* rowres, const float* rowdist, uint32_t n_rows, const uint32_t* chunks,
+                     uint32_t n_chunks, int path, uint64_t base, uint32_t* out_pairs, float* out_dist, uint64_t out_slots,
+                     uint32_t* pair_counts, uint32_t n_pairs, uint64_t* total_out, uint64_t* status_out,
+                     uint32_t* epoch_inout);
+
+/*
  * Experiment switches for kernel studies (process-wide; the defaults are the production configuration):
  *   "probe"     1 | 2   timing-attribution builds of the scoring kernel -- results are GARBAGE
  *   "variant"   n       experiment builds of the scoring kernel -- results stay exact
@@ -85,6 +116,7 @@ int fm_debug_reject_rows(fm_ctx* ctx, uint32_t task, uint32_t n_rows, float* arg
  *                       -- results are exact either way
  *   "surv_cap"  n       survivor units the capture pass may use per batch (-1 = built-in); a small value forces the
  *                       overflow route (surplus survivors go to the exact row kernel)
+ *   "compact_v" 3|2|1   version of the three-launch compaction (batches of more than 1536 chunks) -- results stay exact
  *   "reject_dump" 0|1   two-phase scoring: keep what the reject pass computed for fm_debug_reject_rows (a dump build
  *                       of the reject kernel and a synchronisation per batch) -- results stay exact
  * Returns FM_ERR_INVALID for an unknown name.  Nothing reads environment variables.
