@@ -100,9 +100,10 @@ int ensure(fs_ctx* c, T*& p, size_t& cap, size_t need) {
 
 size_t voxel_size(int t) {
   switch (t) {
-    case FS_U8: return 1;
+    case FS_U8: case FS_I8: return 1;
     case FS_I16: case FS_U16: return 2;
-    case FS_I32: case FS_F32: return 4;
+    case FS_I32: case FS_U32: case FS_F32: return 4;
+    case FS_F64: return 8;
   }
   return 0;
 }
@@ -405,6 +406,9 @@ int fs_set_volume(fs_ctx* c, const void* voxels, int voxel_type, int nx, int ny,
     case FS_U16: rc = run_integral(c, static_cast<const uint16_t*>(src), &shift); break;
     case FS_I32: rc = run_integral(c, static_cast<const int32_t*>(src), &shift); break;
     case FS_F32: rc = run_integral(c, static_cast<const float*>(src), &shift); break;
+    case FS_I8: rc = run_integral(c, static_cast<const int8_t*>(src), &shift); break;
+    case FS_U32: rc = run_integral(c, static_cast<const uint32_t*>(src), &shift); break;
+    case FS_F64: rc = run_integral(c, static_cast<const double*>(src), &shift); break;
   }
   if (rc) return rc;
   FS_CUDA(c, cudaEventRecord(c->ev[1], c->stream));

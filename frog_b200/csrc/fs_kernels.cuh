@@ -13,6 +13,7 @@
 #pragma once
 
 #include <cuda_runtime.h>
+#include <math_constants.h>
 #include <stdint.h>
 #include <string.h>
 
@@ -38,10 +39,10 @@ __device__ __forceinline__ int cast_shift(T v, double shift) {
   return clamp_to_int(__dmul_rn(__dadd_rn((double)c, shift), 1.0));
 }
 
-// per-block minimum of the volume, as double (exact for every supported voxel type)
+// per-block minimum of the volume, as double (exact for every supported voxel type); +inf for a block without voxels
 template <typename T>
 __global__ void volume_min_kernel(const T* __restrict__ in, size_t n, double* __restrict__ block_min) {
-  double m = 1.0e300;
+  double m = CUDART_INF;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
     const double v = (double)in[i];
     m = v < m ? v : m;

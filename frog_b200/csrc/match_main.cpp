@@ -25,9 +25,10 @@
 // `-gather nccl` sends the lists GPU-to-GPU over NVLink to worker 0 instead (one communicator rank
 // per worker) -- identical bytes, but communicator start-up costs more than it saves a one-shot run.
 //
-// Volume entries.  A list entry ending in ".mha" is a MetaImage volume: the load loop reads it (in parallel, like the
-// keypoint files) and hands it to the SURF3D producer, which yields exactly the keypoints that
-// `surf3d <volume> <options>` followed by the .csv.gz reader would (`-surf3d "<surf3d options>"`, one token; the
+// Volume entries.  A list entry ending in ".mha" or ".mhd" is a MetaImage volume (data in the header's file or in the
+// file it names; raw or compressed, either byte order, the element types fsio::read_metaimage lists): the load loop
+// reads it (in parallel, like the keypoint files) and hands it to the SURF3D producer, which yields exactly the
+// keypoints that `surf3d <volume> <options>` followed by the .csv.gz reader would (`-surf3d "<surf3d options>"`, one token; the
 // conversion to the text's values runs on the device, fs_get_points_as_read).  This removes a process start -- and so
 // a CUDA start-up, ~0.55 s -- and a text round trip per volume.  Producer calls go to ONE fs_ctx on this process's
 // GPU 0, created by the first volume after the workers are forked and used by one loader thread at a time: a 400^3
@@ -335,7 +336,9 @@ void worker_run(Control* ctl, int g, int device, fm_ctx* warm) {
 
 // ---- volume entries: the SURF3D producer (libfrogsurf.so, loaded at run time) --------------------------------------
 
-bool is_volume(const string& f) { return f.size() > 4 && f.compare(f.size() - 4, 4, ".mha") == 0; }
+bool is_volume(const string& f) {
+  return f.size() > 4 && (f.compare(f.size() - 4, 4, ".mha") == 0 || f.compare(f.size() - 4, 4, ".mhd") == 0);
+}
 
 struct SurfApi {
   void* handle = nullptr;
@@ -577,9 +580,13 @@ int run_job(int argc, char* argv[], std::ostream& cout, std::ostream& cerr, Warm
       const string& f = filenames[i];
       if (is_volume(f)) {
         // At most one extremum per middle response layer position, layers sampled every 2 voxels or more: fewer than
-        // voxels / 3 keypoints, and a voxel takes at least one byte of the file.
+        // voxels / 3 keypoints.  An uncompressed .mha takes at least one byte per voxel; a .mhd header or a compressed
+        // stream can be far smaller than the voxel count its header states.
+        fsio::MetaHeader h;
+        string herr;
+        const double voxels = std::max(bytes, fsio::read_metaimage_header(f, h, herr) ? (double)h.dims[0] * h.dims[1] * h.dims[2] : 0.0);
         const double d = surfOpts.descriptorType == 1 ? 24.0 * std::pow((double)surfOpts.subVolumeRadius, 3) : 48.0;
-        const double n_vol = surfOpts.numberOfPoints > 0 ? std::min<double>(surfOpts.numberOfPoints, bytes / 3) : bytes / 3;
+        const double n_vol = surfOpts.numberOfPoints > 0 ? std::min<double>(surfOpts.numberOfPoints, voxels / 3) : voxels / 3;
         est_bytes += n_vol * (d + 2) * sizeof(float);
         pts += n_vol;
         pts2 += n_vol * n_vol;
@@ -636,7 +643,7 @@ int run_job(int argc, char* argv[], std::ostream& cout, std::ostream& cerr, Warm
   if (std::any_of(filenames.begin(), filenames.begin() + nb, is_volume)) {
     string err;
     if (!producer.api->load(err)) {
-      cerr << "match: the list holds MetaImage volumes (.mha), which need libfrogsurf.so: " << err << endl;
+      cerr << "match: the list holds MetaImage volumes (.mha / .mhd), which need libfrogsurf.so: " << err << endl;
       return 1;
     }
   }

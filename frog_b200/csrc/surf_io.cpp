@@ -2,6 +2,8 @@
 
 #include <zlib.h>
 
+#include <algorithm>
+#include <chrono>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -14,7 +16,7 @@ namespace fsio {
 
 namespace {
 
-size_t type_size(int t) { return t == FS_U8 ? 1 : (t == FS_I16 || t == FS_U16) ? 2 : 4; }
+double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
 std::string trim(const std::string& s) {
   size_t a = s.find_first_not_of(" \t\r\n"), b = s.find_last_not_of(" \t\r\n");
@@ -22,8 +24,8 @@ std::string trim(const std::string& s) {
 }
 
 template <typename T>
-void flip_axis(std::vector<unsigned char>& data, const int dims[3], int axis) {
-  T* p = reinterpret_cast<T*>(data.data());
+void flip_axis(unsigned char* data, const int dims[3], int axis) {
+  T* p = reinterpret_cast<T*>(data);
   const size_t nx = dims[0], ny = dims[1], nz = dims[2];
   const size_t n[3] = {nx, ny, nz};
   for (size_t z = 0; z < nz; z++)
@@ -93,73 +95,213 @@ inline size_t format_fixed(double v, int decimals, char* out, size_t cap) {
 
 }  // namespace
 
-bool read_metaimage(const std::string& path, Volume& out, std::string& err, FILE* warnings) {
+size_t type_size(int t) {
+  switch (t) {
+    case FS_U8: case FS_I8: return 1;
+    case FS_I16: case FS_U16: return 2;
+    case FS_F64: return 8;
+    default: return 4;
+  }
+}
+
+bool read_metaimage_header(const std::string& path, MetaHeader& h, std::string& err) {
+  h = MetaHeader{};
+  auto fail = [&](const std::string& what) { err = "MetaImage " + path + ": " + what; return false; };
   std::ifstream f(path, std::ios::binary);
   if (!f) { err = "cannot open " + path; return false; }
   std::map<std::string, std::string> kv;
   std::string line, datafile;
+  bool have_datafile = false;
   while (std::getline(f, line)) {
     const size_t eq = line.find('=');
     if (eq == std::string::npos) continue;
     const std::string k = trim(line.substr(0, eq)), v = trim(line.substr(eq + 1));
     kv[k] = v;
-    if (k == "ElementDataFile") { datafile = v; break; }
+    if (k == "ElementDataFile") { datafile = v; have_datafile = true; break; }
   }
+  if (!have_datafile) return fail("no ElementDataFile");
   auto ints = [&](const char* k, int* o, int n) { std::istringstream s(kv[k]); for (int i = 0; i < n; i++) if (!(s >> o[i])) return false; return true; };
   auto dbls = [&](const char* k, double* o, int n) { std::istringstream s(kv[k]); for (int i = 0; i < n; i++) if (!(s >> o[i])) return false; return true; };
+  auto is_true = [&](const char* k) { const std::string& v = kv.count(k) ? kv[k] : std::string(); return v == "True" || v == "true" || v == "TRUE"; };
+  auto key_value = [&](const char* k) { return std::string(k) + " = " + kv[k]; };
   int ndims = 0;
   if (!ints("NDims", &ndims, 1) || ndims != 3) { err = "MetaImage: NDims must be 3"; return false; }
-  if (!ints("DimSize", out.dims, 3)) { err = "MetaImage: DimSize"; return false; }
-  if (kv.count("ElementSpacing")) dbls("ElementSpacing", out.spacing, 3);
-  else if (kv.count("ElementSize")) dbls("ElementSize", out.spacing, 3);
-  if (kv.count("Offset")) dbls("Offset", out.origin, 3);
-  else if (kv.count("Position")) dbls("Position", out.origin, 3);
-  else if (kv.count("Origin")) dbls("Origin", out.origin, 3);
-  if (kv.count("ElementNumberOfChannels") && kv["ElementNumberOfChannels"] != "1") { err = "MetaImage: one channel only"; return false; }
-  if (kv.count("CompressedData") && (kv["CompressedData"] == "True" || kv["CompressedData"] == "true")) { err = "MetaImage: compressed data unsupported"; return false; }
-  if (kv.count("BinaryDataByteOrderMSB") && (kv["BinaryDataByteOrderMSB"] == "True" || kv["BinaryDataByteOrderMSB"] == "true")) { err = "MetaImage: big-endian data unsupported"; return false; }
+  if (!ints("DimSize", h.dims, 3) || h.dims[0] <= 0 || h.dims[1] <= 0 || h.dims[2] <= 0) { err = "MetaImage: DimSize"; return false; }
+  if (kv.count("ElementSpacing")) dbls("ElementSpacing", h.spacing, 3);
+  else if (kv.count("ElementSize")) dbls("ElementSize", h.spacing, 3);
+  if (kv.count("Offset")) dbls("Offset", h.origin, 3);
+  else if (kv.count("Position")) dbls("Position", h.origin, 3);
+  else if (kv.count("Origin")) dbls("Origin", h.origin, 3);
+  if (kv.count("ElementNumberOfChannels") && kv["ElementNumberOfChannels"] != "1")
+    return fail(key_value("ElementNumberOfChannels") + ": one channel only");
+  if (kv.count("BinaryData") && !is_true("BinaryData")) return fail(key_value("BinaryData") + ": ASCII element data is not supported");
   const std::string et = kv["ElementType"];
-  if (et == "MET_UCHAR") out.voxel_type = FS_U8;
-  else if (et == "MET_SHORT") out.voxel_type = FS_I16;
-  else if (et == "MET_USHORT") out.voxel_type = FS_U16;
-  else if (et == "MET_INT") out.voxel_type = FS_I32;
-  else if (et == "MET_FLOAT") out.voxel_type = FS_F32;
-  else { err = "MetaImage: unsupported ElementType " + et; return false; }
-  const size_t bytes = (size_t)out.dims[0] * out.dims[1] * out.dims[2] * type_size(out.voxel_type);
-  out.data.resize(bytes);
+  if (et == "MET_UCHAR") h.voxel_type = FS_U8;
+  else if (et == "MET_CHAR") h.voxel_type = FS_I8;
+  else if (et == "MET_SHORT") h.voxel_type = FS_I16;
+  else if (et == "MET_USHORT") h.voxel_type = FS_U16;
+  else if (et == "MET_INT") h.voxel_type = FS_I32;
+  else if (et == "MET_UINT") h.voxel_type = FS_U32;
+  else if (et == "MET_FLOAT") h.voxel_type = FS_F32;
+  else if (et == "MET_DOUBLE") h.voxel_type = FS_F64;
+  else if (et == "MET_LONG" || et == "MET_ULONG")  // sizeof(long) of the program that wrote the file
+    return fail(key_value("ElementType") + ": its width depends on the platform that wrote the file");
+  else if (et == "MET_LONG_LONG" || et == "MET_ULONG_LONG")
+    return fail(key_value("ElementType") + ": 64-bit integers above 2^53 have no exact double value");
+  else return fail("unsupported " + key_value("ElementType"));
+  if (datafile == "LIST" || datafile.find('%') != std::string::npos)
+    return fail(key_value("ElementDataFile") + ": lists and file patterns of data files are not supported");
+  h.big_endian = is_true("BinaryDataByteOrderMSB") || is_true("ElementByteOrderMSB");
+  h.compressed = is_true("CompressedData");
+  if (h.compressed && kv.count("CompressedDataSize")) {
+    std::istringstream s(kv["CompressedDataSize"]);
+    if (!(s >> h.compressed_size) || h.compressed_size < 0) return fail("bad " + key_value("CompressedDataSize"));
+  }
   if (datafile == "LOCAL") {
-    f.read(reinterpret_cast<char*>(out.data.data()), bytes);
-    if ((size_t)f.gcount() != bytes) { err = "MetaImage: short data"; return false; }
+    h.data_file = path;
+    h.data_offset = (long long)f.tellg();
+    if (h.data_offset < 0) {  // the header ends the file: the data read reports it short
+      f.clear();
+      f.seekg(0, std::ios::end);
+      h.data_offset = (long long)f.tellg();
+    }
   } else {
     std::string dir;
     const size_t slash = path.find_last_of('/');
     if (slash != std::string::npos && datafile[0] != '/') dir = path.substr(0, slash + 1);
-    std::ifstream d(dir + datafile, std::ios::binary);
-    if (!d) { err = "cannot open " + dir + datafile; return false; }
-    d.read(reinterpret_cast<char*>(out.data.data()), bytes);
-    if ((size_t)d.gcount() != bytes) { err = "MetaImage: short data file"; return false; }
+    h.data_file = dir + datafile;
+    if (kv.count("HeaderSize")) {
+      std::istringstream s(kv["HeaderSize"]);
+      if (!(s >> h.data_offset) || h.data_offset < -1) return fail("bad " + key_value("HeaderSize"));
+      if (h.data_offset == -1 && h.compressed) return fail(key_value("HeaderSize") + " with compressed data: the data's start is unknown");
+    }
   }
   // vtkRobustImageReader.h:52-60, 97-113
   for (const char* key : {"TransformMatrix", "Orientation", "Rotation"}) {
     if (!kv.count(key)) continue;
     double m[9];
     if (!dbls(key, m, 9)) continue;
-    for (int i = 0; i < 3; i++) {
-      if (!(m[4 * i] < 0)) continue;
-      if (warnings) std::fprintf(warnings, "Warning : RobustReader flipping dimension %d\n", i);
-      switch (type_size(out.voxel_type)) {
-        case 1: flip_axis<uint8_t>(out.data, out.dims, i); break;
-        case 2: flip_axis<uint16_t>(out.data, out.dims, i); break;
-        default: flip_axis<uint32_t>(out.data, out.dims, i); break;
-      }
-      out.origin[i] = out.origin[i] - out.spacing[i] * (out.dims[i] - 1);
-    }
+    for (int i = 0; i < 3; i++) h.flips[i] += m[4 * i] < 0;
   }
   return true;
 }
 
+namespace {
+
+// Inflates one zlib or gzip stream (header detected by zlib) of at most `avail` bytes (< 0: to the end of the file)
+// from `in` straight into dst[0, bytes): the stream must end exactly there.
+bool inflate_into(std::ifstream& in, long long avail, unsigned char* dst, size_t bytes, const std::string& file,
+                  std::string& err, ReadTimes* t) {
+  auto fail = [&](const std::string& what) { err = "MetaImage " + file + ": " + what; return false; };
+  z_stream zs{};
+  if (inflateInit2(&zs, 15 + 32) != Z_OK) return fail("inflateInit2 failed");
+  std::vector<unsigned char> buf(1 << 20);
+  unsigned char spare;  // receives output beyond the expected size, to tell a longer stream from a complete one
+  size_t done = 0;
+  bool eof = false, ok = false;
+  for (;;) {
+    if (zs.avail_in == 0 && !eof) {
+      const double t0 = now_s();
+      const size_t want = avail < 0 ? buf.size() : (size_t)std::min<long long>(avail, (long long)buf.size());
+      in.read(reinterpret_cast<char*>(buf.data()), (std::streamsize)want);
+      const size_t got = (size_t)in.gcount();
+      if (avail >= 0) avail -= (long long)got;
+      eof = got < want || avail == 0;
+      zs.next_in = buf.data();
+      zs.avail_in = (uInt)got;
+      if (t) t->read_s += now_s() - t0;
+    }
+    const double t0 = now_s();
+    const bool full = done == bytes;
+    zs.next_out = full ? &spare : dst + done;
+    zs.avail_out = full ? 1u : (uInt)std::min<size_t>(bytes - done, 1u << 30);
+    const uInt out0 = zs.avail_out;
+    const int rc = inflate(&zs, Z_NO_FLUSH);
+    const size_t produced = out0 - zs.avail_out;
+    if (t) t->inflate_s += now_s() - t0;
+    if (full && produced) { err = "decompresses to more than " + std::to_string(bytes) + " bytes (DimSize x element size)"; break; }
+    done += produced;
+    if (rc == Z_STREAM_END) {
+      if (done == bytes) ok = true;
+      else err = "compressed stream ends after " + std::to_string(done) + " of " + std::to_string(bytes) + " bytes";
+      break;
+    }
+    if (rc == Z_BUF_ERROR && zs.avail_in == 0 && eof) {
+      err = "compressed stream is truncated after " + std::to_string(done) + " of " + std::to_string(bytes) + " bytes";
+      break;
+    }
+    if (rc != Z_OK && rc != Z_BUF_ERROR) { err = std::string("corrupt compressed stream: ") + (zs.msg ? zs.msg : "inflate failed"); break; }
+  }
+  inflateEnd(&zs);
+  return ok || fail(err);
+}
+
+template <typename T>
+void swap_elements(unsigned char* p, size_t bytes) {
+  for (size_t i = 0; i + sizeof(T) <= bytes; i += sizeof(T)) std::reverse(p + i, p + i + sizeof(T));
+}
+
+}  // namespace
+
+bool read_metaimage_data(const MetaHeader& h, unsigned char* dst, std::string& err, FILE* warnings, ReadTimes* t) {
+  auto fail = [&](const std::string& what) { err = "MetaImage " + h.data_file + ": " + what; return false; };
+  const size_t bytes = h.bytes();
+  double t0 = now_s();
+  std::ifstream d(h.data_file, std::ios::binary);
+  if (!d) { err = "cannot open " + h.data_file; return false; }
+  d.seekg(0, std::ios::end);
+  const long long file_size = (long long)d.tellg();
+  long long start = h.data_offset;
+  if (start < 0) start = file_size - (long long)bytes;  // HeaderSize = -1: the data ends the file
+  if (start < 0 || start > file_size) return fail("short data: " + std::to_string(file_size) + " bytes, " + std::to_string(bytes) + " needed");
+  d.seekg(start);
+  if (h.compressed) {
+    if (h.compressed_size > file_size - start)
+      return fail("CompressedDataSize = " + std::to_string(h.compressed_size) + " exceeds the " + std::to_string(file_size - start) +
+                  " bytes after the header");
+    if (t) t->read_s += now_s() - t0;
+    if (!inflate_into(d, h.compressed_size, dst, bytes, h.data_file, err, t)) return false;
+  } else {
+    d.read(reinterpret_cast<char*>(dst), (std::streamsize)bytes);
+    if ((size_t)d.gcount() != bytes) return fail("short data: " + std::to_string(d.gcount()) + " of " + std::to_string(bytes) + " bytes");
+    if (t) t->read_s += now_s() - t0;
+  }
+  t0 = now_s();
+  const size_t es = type_size(h.voxel_type);
+  if (h.big_endian) {
+    switch (es) {
+      case 2: swap_elements<uint16_t>(dst, bytes); break;
+      case 4: swap_elements<uint32_t>(dst, bytes); break;
+      case 8: swap_elements<uint64_t>(dst, bytes); break;
+    }
+  }
+  for (int i = 0; i < 3; i++) {
+    for (int k = 0; k < h.flips[i]; k++) {  // once per key with a negative diagonal, as vtkRobustImageReader.h:97-113
+      if (warnings) std::fprintf(warnings, "Warning : RobustReader flipping dimension %d\n", i);
+      switch (es) {
+        case 1: flip_axis<uint8_t>(dst, h.dims, i); break;
+        case 2: flip_axis<uint16_t>(dst, h.dims, i); break;
+        case 4: flip_axis<uint32_t>(dst, h.dims, i); break;
+        default: flip_axis<uint64_t>(dst, h.dims, i); break;
+      }
+    }
+  }
+  if (t) t->swap_s += now_s() - t0;
+  return true;
+}
+
+bool read_metaimage(const std::string& path, Volume& out, std::string& err, FILE* warnings) {
+  MetaHeader h;
+  if (!read_metaimage_header(path, h, err)) return false;
+  out.data.resize(h.bytes());
+  if (!read_metaimage_data(h, out.data.data(), err, warnings)) return false;
+  for (int i = 0; i < 3; i++) { out.dims[i] = h.dims[i]; out.spacing[i] = h.spacing[i]; out.origin[i] = h.flipped_origin(i); }
+  out.voxel_type = h.voxel_type;
+  return true;
+}
+
 bool write_metaimage(const std::string& path, const Volume& v, std::string& err) {
-  static const char* names[] = {"MET_UCHAR", "MET_SHORT", "MET_USHORT", "MET_INT", "MET_FLOAT"};
+  static const char* names[] = {"MET_UCHAR", "MET_SHORT", "MET_USHORT", "MET_INT", "MET_FLOAT", "MET_CHAR", "MET_UINT", "MET_DOUBLE"};
   std::ofstream f(path, std::ios::binary);
   if (!f) { err = "cannot write " + path; return false; }
   f << "ObjectType = Image\nNDims = 3\nBinaryData = True\nBinaryDataByteOrderMSB = False\nCompressedData = False\n";
@@ -355,6 +497,9 @@ void clamp_volume(Volume& v, const SurfOptions& o) {
     case FS_I16: clamp_values<int16_t>(v.data, lo, o.clampMinValue, hi, o.clampMaxValue); break;
     case FS_U16: clamp_values<uint16_t>(v.data, lo, o.clampMinValue, hi, o.clampMaxValue); break;
     case FS_I32: clamp_values<int32_t>(v.data, lo, o.clampMinValue, hi, o.clampMaxValue); break;
+    case FS_I8: clamp_values<int8_t>(v.data, lo, o.clampMinValue, hi, o.clampMaxValue); break;
+    case FS_U32: clamp_values<uint32_t>(v.data, lo, o.clampMinValue, hi, o.clampMaxValue); break;
+    case FS_F64: clamp_values<double>(v.data, lo, o.clampMinValue, hi, o.clampMaxValue); break;
     default: clamp_values<float>(v.data, lo, o.clampMinValue, hi, o.clampMaxValue); break;
   }
 }
@@ -397,17 +542,31 @@ int fsio_write_points(const char* path, int fmt, const char* gz_opts, int precis
   return ok ? 0 : -1;
 }
 
-// Reads a MetaImage header + data; returns 0 and fills dims / spacing / origin / voxel_type, copying at most `cap`
-// bytes of voxel data into `data` (may be null to query the size through *bytes).
+namespace {
+thread_local std::string g_fsio_error;
+}
+
+// Text of this thread's most recent fsio_read_metaimage failure.
+const char* fsio_last_error(void) { return g_fsio_error.c_str(); }
+
+// Reads a MetaImage header and fills dims / spacing / origin / voxel_type / *bytes; with `data` non-null it also reads
+// the voxels into data[0, *bytes) (cap must hold them) and, when `seconds` is non-null, stores the time spent on the
+// header, reading, inflating and byte swaps / flips there (four values).  Returns 0, or -1 with fsio_last_error().
 int fsio_read_metaimage(const char* path, int* dims, double* spacing, double* origin, int* voxel_type, void* data, size_t cap,
-                        size_t* bytes) {
-  fsio::Volume v;
-  std::string err;
-  if (!fsio::read_metaimage(path, v, err)) return -1;
-  for (int i = 0; i < 3; i++) { dims[i] = v.dims[i]; spacing[i] = v.spacing[i]; origin[i] = v.origin[i]; }
-  *voxel_type = v.voxel_type;
-  if (bytes) *bytes = v.data.size();
-  if (data) std::memcpy(data, v.data.data(), v.data.size() < cap ? v.data.size() : cap);
+                        size_t* bytes, double* seconds) {
+  const double t0 = fsio::now_s();
+  fsio::MetaHeader h;
+  std::string& err = g_fsio_error;
+  if (!fsio::read_metaimage_header(path, h, err)) return -1;
+  for (int i = 0; i < 3; i++) { dims[i] = h.dims[i]; spacing[i] = h.spacing[i]; origin[i] = h.flipped_origin(i); }
+  *voxel_type = h.voxel_type;
+  if (bytes) *bytes = h.bytes();
+  if (!data) return 0;
+  if (cap < h.bytes()) { err = "fsio_read_metaimage: " + std::to_string(cap) + " bytes given, " + std::to_string(h.bytes()) + " needed"; return -1; }
+  fsio::ReadTimes t;
+  const double t1 = fsio::now_s();
+  if (!fsio::read_metaimage_data(h, static_cast<unsigned char*>(data), err, stdout, &t)) return -1;
+  if (seconds) { seconds[0] = t1 - t0; seconds[1] = t.read_s; seconds[2] = t.inflate_s; seconds[3] = t.swap_s; }
   return 0;
 }
 

@@ -18,11 +18,49 @@ struct Volume {
   std::vector<unsigned char> data;
 };
 
-// Uncompressed little-endian MetaImage, one component, element types MET_UCHAR / MET_SHORT / MET_USHORT / MET_INT /
-// MET_FLOAT, data in the same file (ElementDataFile = LOCAL) or in the named file next to the header.  Axis flips for
-// negative TransformMatrix diagonals (vtkRobustImageReader.h:52-60, 97-113) are applied.
+size_t type_size(int voxel_type);  // bytes per element of an fs_voxel_type
+
+// A MetaImage header (.mha / .mhd): what read_metaimage_data needs to fill a buffer of bytes() bytes.
+struct MetaHeader {
+  int dims[3] = {0, 0, 0};
+  double spacing[3] = {1, 1, 1};
+  double origin[3] = {0, 0, 0};  // as written; flipped_origin() is the volume's
+  int voxel_type = FS_I16;
+  std::string data_file;          // the header's own path for ElementDataFile = LOCAL
+  long long data_offset = 0;      // where the data starts in data_file; -1: it ends the file (HeaderSize = -1)
+  bool compressed = false;        // CompressedData: one zlib or gzip stream
+  long long compressed_size = -1; // CompressedDataSize; -1: the stream runs to the end of the file
+  bool big_endian = false;        // BinaryDataByteOrderMSB or ElementByteOrderMSB
+  int flips[3] = {0, 0, 0};       // keys whose direction cosine of this axis is negative
+  size_t bytes() const { return (size_t)dims[0] * dims[1] * dims[2] * type_size(voxel_type); }
+  double flipped_origin(int i) const {
+    double o = origin[i];
+    for (int k = 0; k < flips[i]; k++) o = o - spacing[i] * (dims[i] - 1);
+    return o;
+  }
+};
+
+// Seconds spent by read_metaimage_data: reading the file, inflating, byte swaps and axis flips.
+struct ReadTimes {
+  double read_s = 0, inflate_s = 0, swap_s = 0;
+};
+
+// MetaImage with one component and binary element data, in the same file (ElementDataFile = LOCAL) or in the named
+// file next to the header (after HeaderSize bytes; HeaderSize = -1: the data ends the file).  Element types
+// MET_UCHAR / MET_CHAR / MET_SHORT / MET_USHORT / MET_INT / MET_UINT / MET_FLOAT / MET_DOUBLE.  CompressedData = True:
+// one deflate stream with a zlib or gzip wrapper, CompressedDataSize bytes long or running to the end of the file,
+// inflated in chunks into the voxel buffer; it must yield exactly DimSize x element size bytes.  Big-endian data
+// (BinaryDataByteOrderMSB / ElementByteOrderMSB) is swapped to native order, then axis flips for negative
+// TransformMatrix diagonals (vtkRobustImageReader.h:52-60, 97-113) are applied.  Refused, with the key named:
+// MET_LONG / MET_ULONG (their width is the writer's platform's), 64-bit integers (not exact through double), LIST and
+// pattern data files, ASCII data, more than one channel.
 // (`warnings`: where the reader's axis-flip notices go; bin/surf3d prints them on stdout like the reference.)
 bool read_metaimage(const std::string& path, Volume& out, std::string& err, FILE* warnings = stdout);
+// The same in two steps: the header alone, then the data into dst[0, h.bytes()) (nothing partial is reported as read:
+// on failure dst's contents are undefined).
+bool read_metaimage_header(const std::string& path, MetaHeader& h, std::string& err);
+bool read_metaimage_data(const MetaHeader& h, unsigned char* dst, std::string& err, FILE* warnings = stdout,
+                         ReadTimes* times = nullptr);
 bool write_metaimage(const std::string& path, const Volume& v, std::string& err);
 
 // vtk3DSURF::WritePointsCSV / WritePointsCSVGZ / WritePointsBinary (vtk3DSURF.cxx:405-525): voxel-unit keypoints are

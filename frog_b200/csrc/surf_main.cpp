@@ -2,7 +2,8 @@
 // Same command line as the reference's surf3d (vtkOpenSURF3D/surf3d.cxx:16-157): the option loop advances two
 // tokens per key and ignores keys it does not know.  Options that need VTK's own image filters (-s / -d
 // resampling, -m mask, -pad, -type 2) or picojson (-json 1) are rejected loudly instead of being approximated; the input is a
-// MetaImage volume already at its final sampling.
+// MetaImage volume already at its final sampling (.mha or .mhd, raw or compressed, either byte order, the element types
+// fsio::read_metaimage lists).
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>

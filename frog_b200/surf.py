@@ -20,7 +20,7 @@ PUBLIC_SYMBOLS = [
 ]
 
 VOXEL_TYPES = {np.dtype(np.uint8): 0, np.dtype(np.int16): 1, np.dtype(np.uint16): 2, np.dtype(np.int32): 3,
-               np.dtype(np.float32): 4}
+               np.dtype(np.float32): 4, np.dtype(np.int8): 5, np.dtype(np.uint32): 6, np.dtype(np.float64): 7}
 
 POINT_DTYPE = np.dtype([("x", np.float32), ("y", np.float32), ("z", np.float32), ("scale", np.float32),
                         ("response", np.float32), ("laplacian", np.int32)])
@@ -267,7 +267,9 @@ def _io():
         L.fsio_write_points.argtypes = [C.c_char_p, C.c_int, C.c_char_p, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t,
                                         C.c_size_t, C.c_void_p, C.c_void_p]
         L.fsio_read_metaimage.argtypes = [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
-                                          C.c_size_t, C.c_void_p]
+                                          C.c_size_t, C.c_void_p, C.c_void_p]
+        L.fsio_last_error.restype = C.c_char_p
+        L.fsio_last_error.argtypes = []
         L.fsio_write_bounds_json.argtypes = [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.fsio_debug_as_read.argtypes = [C.c_void_p, C.c_long, C.c_int, C.c_void_p]
         L.fsio_read_points.restype = C.c_long
@@ -314,35 +316,69 @@ def read_points_file(path: str, spacing, origin, shape):
     return out, outside.value
 
 
-_MET = {0: np.uint8, 1: np.int16, 2: np.uint16, 3: np.int32, 4: np.float32}
+_MET = {0: np.uint8, 1: np.int16, 2: np.uint16, 3: np.int32, 4: np.float32, 5: np.int8, 6: np.uint32, 7: np.float64}
 _MET_NAME = {np.dtype(np.uint8): "MET_UCHAR", np.dtype(np.int16): "MET_SHORT", np.dtype(np.uint16): "MET_USHORT",
-             np.dtype(np.int32): "MET_INT", np.dtype(np.float32): "MET_FLOAT"}
+             np.dtype(np.int32): "MET_INT", np.dtype(np.float32): "MET_FLOAT", np.dtype(np.int8): "MET_CHAR",
+             np.dtype(np.uint32): "MET_UINT", np.dtype(np.float64): "MET_DOUBLE"}
 
 
-def read_metaimage(path: str):
-    """(volume [z, y, x], spacing, origin) through bin/surf3d's own reader."""
+def read_metaimage(path: str, phases: dict | None = None):
+    """(volume [z, y, x] in native byte order, spacing, origin) through bin/surf3d's own reader.  `phases`, when given,
+    receives the seconds spent on the header, reading, inflating and byte swaps / axis flips."""
     dims = (C.c_int * 3)()
     sp = (C.c_double * 3)()
     org = (C.c_double * 3)()
     vt = C.c_int()
     nbytes = C.c_size_t()
-    if _io().fsio_read_metaimage(path.encode(), dims, sp, org, C.byref(vt), None, 0, C.byref(nbytes)) != 0:
-        raise FrogSurfError(f"cannot read {path}")
-    vol = np.zeros((dims[2], dims[1], dims[0]), _MET[vt.value])
-    _io().fsio_read_metaimage(path.encode(), dims, sp, org, C.byref(vt), vol.ctypes.data, vol.nbytes, C.byref(nbytes))
+    L = _io()
+    if L.fsio_read_metaimage(path.encode(), dims, sp, org, C.byref(vt), None, 0, C.byref(nbytes), None) != 0:
+        raise FrogSurfError(f"cannot read {path}: {L.fsio_last_error().decode()}")
+    vol = np.empty((dims[2], dims[1], dims[0]), _MET[vt.value])
+    secs = (C.c_double * 4)()
+    if L.fsio_read_metaimage(path.encode(), dims, sp, org, C.byref(vt), vol.ctypes.data, vol.nbytes, C.byref(nbytes), secs) != 0:
+        raise FrogSurfError(f"cannot read {path}: {L.fsio_last_error().decode()}")
+    if phases is not None:
+        phases.update(zip(("header_s", "read_s", "inflate_s", "swap_s"), secs))
     return vol, tuple(sp), tuple(org)
 
 
-def write_metaimage(path: str, volume: np.ndarray, spacing=(1.0, 1.0, 1.0), origin=(0.0, 0.0, 0.0), transform=None) -> None:
-    """Single-file MetaImage (.mha) of a [z, y, x] volume, for feeding bin/surf3d."""
+def write_metaimage(path: str, volume: np.ndarray, spacing=(1.0, 1.0, 1.0), origin=(0.0, 0.0, 0.0), transform=None, *,
+                    compress: int | None = None, gzip: bool = False, compressed_size: bool = True, byte_order: str = "<",
+                    data_file: str | None = None, header_size: int | None = None) -> None:
+    """MetaImage of a [z, y, x] volume, for feeding bin/surf3d and bin/match.
+
+    compress: zlib level (CompressedData = True), the stream wrapped as zlib or, with `gzip`, as a gzip member;
+    compressed_size: write CompressedDataSize.  byte_order: "<" or ">" (BinaryDataByteOrderMSB = True).
+    data_file: the data goes to this file (a name next to the header, usually .raw or .zraw) instead of after the
+    header; header_size: HeaderSize of that file, as many filler bytes written before the data (-1: 61 filler bytes,
+    HeaderSize = -1, the data ends the file)."""
+    import zlib
     v = np.ascontiguousarray(volume)
+    data = v.astype(v.dtype.newbyteorder(byte_order)).tobytes()
+    if compress is not None:
+        z = zlib.compressobj(compress, zlib.DEFLATED, 31 if gzip else 15)
+        data = z.compress(data) + z.flush()
+    hdr = "ObjectType = Image\nNDims = 3\nBinaryData = True\n"
+    hdr += "BinaryDataByteOrderMSB = %s\n" % ("True" if byte_order == ">" else "False")
+    hdr += "CompressedData = %s\n" % ("True" if compress is not None else "False")
+    if compress is not None and compressed_size:
+        hdr += "CompressedDataSize = %d\n" % len(data)
+    if transform is not None:
+        hdr += "TransformMatrix = " + " ".join(repr(float(t)) for t in transform) + "\n"
+    hdr += "Offset = %r %r %r\n" % tuple(float(o) for o in origin)
+    hdr += "ElementSpacing = %r %r %r\n" % tuple(float(s) for s in spacing)
+    hdr += "DimSize = %d %d %d\n" % (v.shape[2], v.shape[1], v.shape[0])
+    hdr += "ElementType = %s\n" % _MET_NAME[np.dtype(v.dtype)]
+    if data_file is None:
+        with open(path, "wb") as f:
+            f.write((hdr + "ElementDataFile = LOCAL\n").encode())
+            f.write(data)
+        return
+    if header_size is not None:
+        hdr += "HeaderSize = %d\n" % header_size
     with open(path, "wb") as f:
-        hdr = "ObjectType = Image\nNDims = 3\nBinaryData = True\nBinaryDataByteOrderMSB = False\nCompressedData = False\n"
-        if transform is not None:
-            hdr += "TransformMatrix = " + " ".join(repr(float(t)) for t in transform) + "\n"
-        hdr += "Offset = %r %r %r\n" % tuple(float(o) for o in origin)
-        hdr += "ElementSpacing = %r %r %r\n" % tuple(float(s) for s in spacing)
-        hdr += "DimSize = %d %d %d\n" % (v.shape[2], v.shape[1], v.shape[0])
-        hdr += "ElementType = %s\nElementDataFile = LOCAL\n" % _MET_NAME[v.dtype]
-        f.write(hdr.encode())
-        f.write(v.tobytes())
+        f.write((hdr + "ElementDataFile = %s\n" % data_file).encode())
+    filler = 61 if header_size == -1 else (header_size or 0)
+    with open(os.path.join(os.path.dirname(path), data_file), "wb") as f:
+        f.write(bytes((i * 37 + 11) & 255 for i in range(filler)))
+        f.write(data)

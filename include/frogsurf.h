@@ -47,7 +47,10 @@ typedef enum fs_voxel_type {
   FS_I16 = 1,
   FS_U16 = 2,
   FS_I32 = 3,
-  FS_F32 = 4
+  FS_F32 = 4,
+  FS_I8 = 5,
+  FS_U32 = 6,
+  FS_F64 = 7
 } fs_voxel_type;
 
 /* one keypoint as FastHessian leaves it (ipoint.h:26-66): voxel units, before the writers apply spacing / origin */
