@@ -29,10 +29,14 @@ PUBLIC_SYMBOLS = [
     "fm_result_device_pairs", "fm_result_free", "fm_get_stats", "fm_result_stats", "fm_version",
     "fm_links_build", "fm_links_total", "fm_links_fetch", "fm_links_offsets", "fm_links_data", "fm_links_device_offsets",
     "fm_links_device_data", "fm_links_build_ms", "fm_links_free",
+    "fm_group_create", "fm_group_destroy", "fm_group_last_error", "fm_group_synchronize", "fm_group_clear_images",
+    "fm_group_upload_image", "fm_group_match",
 ]
 DEBUG_SYMBOLS = ["fm_debug_image", "fm_debug_image_norms", "fm_debug_score_unit", "fm_debug_set_option",
                  "fm_debug_reject_rows", "fm_debug_wide_unit", "fm_debug_compact"]
 ERR_INVALID = -1  # FM_ERR_INVALID
+ERR_CUDA = -2  # FM_ERR_CUDA
+ERR_UNSUPPORTED = -4  # FM_ERR_UNSUPPORTED
 # fm_debug_compact paths (include/frogmatch_debug.h)
 COMPACT_AUTO, COMPACT_ONE, COMPACT_THREE, COMPACT_LOOKALL = 0, 1, 2, 3
 
@@ -119,6 +123,15 @@ def load():
     L.fm_links_build_ms.restype = C.c_float
     L.fm_links_free.argtypes = [vp]
     L.fm_links_free.restype = None
+    L.fm_group_create.argtypes = [C.POINTER(C.c_int), C.c_int, C.POINTER(vp)]
+    L.fm_group_destroy.argtypes = [vp]
+    L.fm_group_destroy.restype = None
+    L.fm_group_last_error.argtypes = [vp]
+    L.fm_group_last_error.restype = C.c_char_p
+    L.fm_group_synchronize.argtypes = [vp]
+    L.fm_group_clear_images.argtypes = [vp]
+    L.fm_group_upload_image.argtypes = [vp, C.c_uint32, vp, vp, vp, C.c_uint32, C.c_uint32]
+    L.fm_group_match.argtypes = [vp, vp, vp, C.c_size_t, C.c_float, C.c_float, C.c_uint32, C.POINTER(vp)]
     _lib = L
     return L
 
@@ -127,10 +140,16 @@ def _ptr(a: np.ndarray):
     return a.ctypes.data_as(C.c_void_p)
 
 
-class Result:
-    """Owns one fm_result: per-pair match lists, on the host and/or on the device."""
+def _flags(sym, force_exact, device_only, asynchronous, match_all, distances) -> int:
+    return (FLAG_SYM if sym else 0) | (FLAG_FORCE_EXACT if force_exact else 0) | \
+        (FLAG_DEVICE_ONLY if device_only else 0) | (FLAG_ASYNC if asynchronous else 0) | \
+        (FLAG_MATCH_ALL if match_all else 0) | (FLAG_DISTANCES if distances else 0)
 
-    def __init__(self, matcher: "Matcher", handle, pending: bool = False):
+
+class Result:
+    """Owns one fm_result (of a Matcher or a Group): per-pair match lists, on the host and/or on the device."""
+
+    def __init__(self, matcher, handle, pending: bool = False):
         self._m, self._h = matcher, handle
         matcher._live.add(self)
         self.n_pairs = matcher._L.fm_result_num_pairs(handle)
@@ -292,9 +311,7 @@ class Matcher:
               match_all: bool = False, distances: bool = False) -> Result:
         pf = np.ascontiguousarray(pair_first, np.uint32)
         ps = np.ascontiguousarray(pair_second, np.uint32)
-        flags = (FLAG_SYM if sym else 0) | (FLAG_FORCE_EXACT if force_exact else 0) | \
-                (FLAG_DEVICE_ONLY if device_only else 0) | (FLAG_ASYNC if asynchronous else 0) | \
-                (FLAG_MATCH_ALL if match_all else 0) | (FLAG_DISTANCES if distances else 0)
+        flags = _flags(sym, force_exact, device_only, asynchronous, match_all, distances)
         h = C.c_void_p()
         self._check(self._L.fm_match(self._h, _ptr(pf), _ptr(ps), pf.shape[0], dist, ratio, flags, C.byref(h)))
         return Result(self, h, pending=asynchronous)
@@ -391,6 +408,69 @@ class Matcher:
             base, _ptr(out_pairs), None if out_dist is None else _ptr(out_dist), out_pairs.shape[0], _ptr(pair_counts),
             pair_counts.shape[0], C.byref(total), None if st is None else _ptr(st), C.byref(ep) if epoch is not None else None))
         return dict(total=total.value, epoch=ep.value if epoch is not None else None, status=st)
+
+
+class Group:
+    """One libfrogmatch group (fm_group_*): a context per device, used as one.  devices[0] is the lead: match() splits
+    the pairs over the devices and returns one Result whose lists are gathered on the lead, in submission order."""
+
+    def __init__(self, devices):
+        self._L = load()
+        self.devices = [int(d) for d in devices]
+        devs = (C.c_int * len(self.devices))(*self.devices)
+        h = C.c_void_p()
+        rc = self._L.fm_group_create(devs, len(self.devices), C.byref(h))
+        if rc != 0:
+            self._h = None
+            raise FrogMatchError(f"fm_group_create failed ({rc}): {self._L.fm_group_last_error(None).decode()}")
+        self._h = h
+        self._live = set()  # results that still own native buffers: freed before the group goes away
+
+    def _check(self, rc: int) -> None:
+        if rc != 0:
+            raise FrogMatchError(f"libfrogmatch error {rc}: {self._L.fm_group_last_error(self._h).decode()}")
+
+    def close(self) -> None:
+        if self._h:
+            for r in list(self._live):
+                r.free()
+            self._L.fm_group_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def synchronize(self) -> None:
+        self._check(self._L.fm_group_synchronize(self._h))
+
+    def clear(self) -> None:
+        self._check(self._L.fm_group_clear_images(self._h))
+
+    def upload(self, img: int, desc, scale, lap) -> None:
+        desc = np.ascontiguousarray(desc, np.float32)
+        scale = np.ascontiguousarray(scale, np.float32)
+        lap = np.ascontiguousarray(lap, np.float32)
+        n, d = desc.shape
+        self._check(self._L.fm_group_upload_image(self._h, img, _ptr(desc), _ptr(scale), _ptr(lap), n, d))
+        self.synchronize()  # the numpy temporaries above may be freed after return
+
+    def upload_raw(self, img: int, desc_ptr: int, scale_ptr: int, lap_ptr: int, n: int, d: int) -> None:
+        """Asynchronous upload from caller-owned pinned host memory or device memory of any member's GPU."""
+        self._check(self._L.fm_group_upload_image(self._h, img, C.c_void_p(desc_ptr), C.c_void_p(scale_ptr),
+                                                  C.c_void_p(lap_ptr), n, d))
+
+    def match(self, pair_first, pair_second, dist: float = 0.22, ratio: float = 1.0, sym: bool = False,
+              force_exact: bool = False, device_only: bool = False, asynchronous: bool = False,
+              match_all: bool = False, distances: bool = False) -> Result:
+        pf = np.ascontiguousarray(pair_first, np.uint32)
+        ps = np.ascontiguousarray(pair_second, np.uint32)
+        flags = _flags(sym, force_exact, device_only, asynchronous, match_all, distances)
+        h = C.c_void_p()
+        self._check(self._L.fm_group_match(self._h, _ptr(pf), _ptr(ps), pf.shape[0], dist, ratio, flags, C.byref(h)))
+        return Result(self, h, pending=asynchronous)
 
 
 def debug_set_option(name: str, value: int) -> None:

@@ -11,11 +11,23 @@
 #include "fm_exact.cuh"
 #include "fm_fast.cuh"
 #include "fm_generic.cuh"
+#include "fm_group.cuh"
 #include "fm_host.h"
 #include "fm_links.cuh"
+#include "fm_shard.h"
 #include "fm_wide.cuh"
 
 using namespace fm;
+
+// One member's share of a group result (fm_group_match): the member's own result of its shard, whose device buffers go
+// back to the member's free lists once the gather is queued (its pinned block and events stay until the group result is
+// complete), and the member-side scratch of the gather.
+struct GroupPart {
+  fm_result* sub = nullptr;
+  DevBuf scratch;                 // member device: local offsets (n + 1 u64) | global positions (n u32)
+  void* pin = nullptr;            // member's pinned staging of the global positions
+  size_t pin_cap = 0;
+};
 
 struct fm_result {
   fm_ctx* ctx = nullptr;
@@ -38,6 +50,10 @@ struct fm_result {
   bool waited = false;
   EventPool ev;     // this call's phase brackets (and `done`)
   fm_stats stats{};  // launch-side counters; device counters and event times are filled in by finalize()
+  uint64_t slots = 0;  // matches d_out is sized for: the call's outer-loop rows (-all: its exact total)
+  // group results (fm_group_match): one part per member that had pairs; the lead's submission-order offsets
+  std::vector<GroupPart> parts;
+  DevBuf d_goff;
 };
 
 struct fm_links {
@@ -71,19 +87,29 @@ int cuda_fail(fm_ctx* c, cudaError_t e, const char* what) {
   } while (0)
 
 // Upload the ImageDev table, prepare the images uploaded since the last call (one batch of
-// kernels) and read the per-image metas (flags, class tables) back.
-int sync_images(fm_ctx* c) {
+// kernels) and read the per-image metas (flags, class tables) back.  prep_queue queues the table and the kernels;
+// prep_finish reads the metas back (a pageable copy: it waits for the stream).  A group queues every member's
+// preparation before it waits for any, so that its members prepare at the same time.
+int prep_queue(fm_ctx* c) {
   if (!c->images_dirty) return FM_OK;
   const size_t n = c->h_images.size();
+  FM_CUDA(c, cudaSetDevice(c->device));
   FM_CUDA(c, c->d_images.ensure(std::max<size_t>(1, n) * sizeof(ImageDev)));
   c->h_metas.assign(n, ImageMeta{});
   if (n) {
     FM_CUDA(c, cudaMemcpyAsync(c->d_images.p, c->h_images.data(), n * sizeof(ImageDev), cudaMemcpyHostToDevice, c->stream));
-    {
-      Span sp(&c->ev_prep, c->stream, kPhPrep);
-      cudaError_t e = fast_prepare_dirty(c);
-      if (e != cudaSuccess) return cuda_fail(c, e, "image preparation");
-    }
+    Span sp(&c->ev_prep, c->stream, kPhPrep);
+    cudaError_t e = fast_prepare_dirty(c);
+    if (e != cudaSuccess) return cuda_fail(c, e, "image preparation");
+  }
+  return FM_OK;
+}
+
+int prep_finish(fm_ctx* c) {
+  if (!c->images_dirty) return FM_OK;
+  const size_t n = c->h_images.size();
+  FM_CUDA(c, cudaSetDevice(c->device));
+  if (n) {
     FM_CUDA(c, cudaMemcpyAsync(c->h_metas.data(), c->d_metas.p, n * sizeof(ImageMeta), cudaMemcpyDeviceToHost, c->stream));
     FM_CUDA(c, cudaStreamSynchronize(c->stream));
     // the bracket above has completed: fold it into the running sum and recycle its events (a long-lived context that
@@ -96,6 +122,11 @@ int sync_images(fm_ctx* c) {
   }
   c->images_dirty = false;
   return FM_OK;
+}
+
+int sync_images(fm_ctx* c) {
+  int rc = prep_queue(c);
+  return rc != FM_OK ? rc : prep_finish(c);
 }
 
 // Small free lists so that several results can be in flight (FM_FLAG_ASYNC) without a cudaMalloc /
@@ -122,6 +153,12 @@ void give_buf(std::vector<DevBuf>& list, DevBuf& b) {
   if (list.size() < 4) list.push_back(b);
   else cudaFree(b.p);
   b = DevBuf{};
+}
+
+// give_buf for a buffer that queued work still reads: it goes back only when the list has room, and otherwise stays
+// with its result until fm_result_free (a cudaFree now would wait for the whole device).
+void give_buf_queued(std::vector<DevBuf>& list, DevBuf& b) {
+  if (b.p && list.size() < 4) give_buf(list, b);
 }
 
 cudaError_t take_pinned(fm_ctx* c, size_t bytes, void** out, size_t* cap) {
@@ -173,6 +210,30 @@ int finalize(fm_result* r) {
   r->stats.ms_rescore = acc[kPhRescore] + acc[kPhBands];
   r->stats.ms_exact = acc[kPhExact];
   r->stats.ms_compact = acc[kPhCompact];
+  if (!r->parts.empty()) {
+    // a group result: counters summed over the members' calls, each phase time the longest member's
+    fm_stats s{};
+    for (auto& gp : r->parts) {
+      fm_result* q = gp.sub;
+      if (finalize(q) != FM_OK) return fail(c, FM_ERR_CUDA, "fm_group_match: device " + std::to_string(q->ctx->device) + ": " + q->ctx->err);
+      const fm_stats& t = q->stats;
+      s.descriptor_pairs += t.descriptor_pairs;
+      s.scored_pairs += t.scored_pairs;
+      s.rows += t.rows;
+      s.rows_exact += t.rows_exact;
+      s.candidates += t.candidates;
+      s.kernel_launches += t.kernel_launches;
+      s.score_launches += t.score_launches;
+      s.rows_rejected_early += t.rows_rejected_early;
+      s.two_phase_batches += t.two_phase_batches;
+      s.ms_total = std::max(s.ms_total, t.ms_total);
+      s.ms_score = std::max(s.ms_score, t.ms_score);
+      s.ms_rescore = std::max(s.ms_rescore, t.ms_rescore);
+      s.ms_exact = std::max(s.ms_exact, t.ms_exact);
+      s.ms_compact = std::max(s.ms_compact, t.ms_compact);
+    }
+    r->stats = s;
+  }
   r->waited = true;
   const float ms_prep = c->stats.ms_prep;
   c->stats = r->stats;
@@ -514,6 +575,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
   r->flags = flags;
   r->ratio = dist2second;
   r->d48 = !wide;
+  r->slots = total_rows;
   r->d_out = take_buf(c->out_free, std::max<uint64_t>(total_rows, 1) * sizeof(uint2));
   r->d_counts = take_buf(c->counts_free, std::max<size_t>(n_pairs, 1) * sizeof(uint32_t));
   const bool want_dist = (flags & FM_FLAG_DISTANCES) && !match_all;
@@ -629,6 +691,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
         pair_counts[pair_of_task[t]] = (uint32_t)pc;
       }
       FM_CUDA_R(r->d_out.ensure(std::max<unsigned long long>(grand, 1) * sizeof(uint2)));
+      r->slots = grand;
       FM_CUDA_R(cudaMemcpyAsync(d_task_base, task_base.data(), (size_t)n_tasks * sizeof(unsigned long long), cudaMemcpyHostToDevice, c->stream));
       {
         Span sp(&c->ev_match, c->stream, kPhExact);
@@ -831,6 +894,14 @@ void fm_result_free(fm_result* r) {
       cudaFreeHost(r->h_pairs);
     }
   }
+  give_buf(c->counts_free, r->d_goff);
+  for (auto& gp : r->parts) {  // (the lead's `done` follows every member's gather: nothing below is still in use)
+    fm_ctx* m = gp.sub->ctx;
+    fm_result_free(gp.sub);
+    cudaSetDevice(m->device);
+    give_buf(m->counts_free, gp.scratch);
+    give_pinned(m, gp.pin, gp.pin_cap);
+  }
   delete r;
 }
 
@@ -971,6 +1042,337 @@ void fm_links_free(fm_links* l) {
   delete l;
 }
 
+// ---- device groups (fm_group_*): several contexts that act as one -------------------------------------------------
+
+}  // extern "C"
+
+struct fm_group {
+  std::vector<fm_ctx*> m;         // one context per device; m[0] is the lead
+  std::vector<cudaEvent_t> ev;    // per member, on its device: the member's stream up to the latest hand-off
+  cudaEvent_t ev_lead = nullptr;  // the lead's scan of the gathered counts
+  std::vector<std::vector<char>> peer;  // peer[k][j]: member k reads member j's memory directly (same GPU, or peer access)
+};
+
+namespace {
+
+thread_local std::string g_group_create_error;
+
+int group_fail(fm_group* g, int code, const std::string& msg) {
+  if (g) g->m[0]->err = msg; else g_group_create_error = msg;
+  return code;
+}
+
+// An error of member k's own call, reported on the group with the device named.
+int member_fail(fm_group* g, size_t k, int code) {
+  return group_fail(g, code, "device " + std::to_string(g->m[k]->device) + ": " + g->m[k]->err);
+}
+
+}  // namespace
+
+extern "C" {
+
+int fm_group_create(const int* devices, int n, fm_group** out) {
+  if (!out) return group_fail(nullptr, FM_ERR_INVALID, "fm_group_create: out is NULL");
+  *out = nullptr;
+  int n_dev = 0;
+  cudaError_t e = cudaGetDeviceCount(&n_dev);
+  if (e != cudaSuccess || n_dev == 0)
+    return group_fail(nullptr, FM_ERR_CUDA, std::string("fm_group_create: no CUDA device (") + cudaGetErrorString(e) +
+                                                "); libfrogmatch has no CPU fallback");
+  if (!devices || n <= 0) return group_fail(nullptr, FM_ERR_INVALID, "fm_group_create: no devices given");
+  for (int k = 0; k < n; k++) {
+    if (devices[k] < 0 || devices[k] >= n_dev)
+      return group_fail(nullptr, FM_ERR_INVALID, "fm_group_create: device " + std::to_string(devices[k]) + " is out of range (" +
+                                                     std::to_string(n_dev) + " visible)");
+    for (int j = 0; j < k && !g_debug.group_repeat; j++)
+      if (devices[j] == devices[k])
+        return group_fail(nullptr, FM_ERR_INVALID, "fm_group_create: device " + std::to_string(devices[k]) + " is given twice");
+  }
+  for (int k = 1; k < n; k++) {
+    if (devices[k] == devices[0]) continue;  // (fm_debug_set_option "group_repeat")
+    int can = 0;
+    if ((e = cudaDeviceCanAccessPeer(&can, devices[k], devices[0])) != cudaSuccess)
+      return group_fail(nullptr, FM_ERR_CUDA, std::string("fm_group_create: cudaDeviceCanAccessPeer: ") + cudaGetErrorString(e));
+    if (!can)
+      return group_fail(nullptr, FM_ERR_UNSUPPORTED, "fm_group_create: device " + std::to_string(devices[k]) +
+                                                         " cannot access the lead device " + std::to_string(devices[0]) + " as a peer");
+  }
+  fm_group* g = new (std::nothrow) fm_group();
+  if (!g) return group_fail(nullptr, FM_ERR_NOMEM, "fm_group_create: out of host memory");
+  auto undo = [&](int code, const std::string& msg) {
+    fm_group_destroy(g);
+    return group_fail(nullptr, code, msg);
+  };
+  for (int k = 0; k < n; k++) {
+    fm_ctx* c = nullptr;
+    int rc = fm_create(devices[k], &c);
+    if (rc != FM_OK) return undo(rc, std::string(fm_last_error(nullptr)));
+    g->m.push_back(c);
+    cudaEvent_t ev = nullptr;
+    if ((e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming)) != cudaSuccess)
+      return undo(FM_ERR_CUDA, std::string("fm_group_create: ") + cudaGetErrorString(e));
+    g->ev.push_back(ev);
+  }
+  // Peer access (process state, left enabled at destroy) for every ordered pair of members that supports it: members
+  // store into the lead's memory (the gather; required, checked above), and uploads copy between members.
+  g->peer.assign(n, std::vector<char>(n, 0));
+  for (int k = 0; k < n; k++)
+    for (int j = 0; j < n; j++) {
+      if (devices[k] == devices[j]) { g->peer[k][j] = 1; continue; }  // (the same GPU: fm_debug_set_option "group_repeat")
+      int can = 0;
+      if (cudaDeviceCanAccessPeer(&can, devices[k], devices[j]) != cudaSuccess || !can) { cudaGetLastError(); continue; }
+      cudaSetDevice(devices[k]);
+      e = cudaDeviceEnablePeerAccess(devices[j], 0);
+      if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
+      else if (e != cudaSuccess) {
+        cudaGetLastError();
+        if (j == 0)
+          return undo(FM_ERR_UNSUPPORTED, "fm_group_create: device " + std::to_string(devices[k]) + " cannot map the lead device " +
+                                              std::to_string(devices[0]) + ": " + cudaGetErrorString(e));
+        continue;
+      }
+      g->peer[k][j] = 1;
+    }
+  cudaSetDevice(devices[0]);
+  if ((e = cudaEventCreateWithFlags(&g->ev_lead, cudaEventDisableTiming)) != cudaSuccess)
+    return undo(FM_ERR_CUDA, std::string("fm_group_create: ") + cudaGetErrorString(e));
+  *out = g;
+  return FM_OK;
+}
+
+void fm_group_destroy(fm_group* g) {
+  if (!g) return;
+  for (size_t k = 0; k < g->m.size(); k++) {
+    cudaSetDevice(g->m[k]->device);
+    cudaStreamSynchronize(g->m[k]->stream);
+    if (k < g->ev.size()) cudaEventDestroy(g->ev[k]);
+  }
+  if (g->ev_lead) {
+    cudaSetDevice(g->m[0]->device);
+    cudaEventDestroy(g->ev_lead);
+  }
+  for (auto* c : g->m) fm_destroy(c);
+  delete g;
+}
+
+const char* fm_group_last_error(const fm_group* g) { return g ? g->m[0]->err.c_str() : g_group_create_error.c_str(); }
+
+int fm_group_synchronize(fm_group* g) {
+  if (!g) return FM_ERR_INVALID;
+  for (size_t k = 0; k < g->m.size(); k++)
+    if (int rc = fm_synchronize(g->m[k])) return member_fail(g, k, rc);
+  return FM_OK;
+}
+
+int fm_group_clear_images(fm_group* g) {
+  if (!g) return FM_ERR_INVALID;
+  for (size_t k = 0; k < g->m.size(); k++)
+    if (int rc = fm_clear_images(g->m[k])) return member_fail(g, k, rc);
+  return FM_OK;
+}
+
+int fm_group_upload_image(fm_group* g, uint32_t img, const float* desc, const float* scale, const float* lap, uint32_t n,
+                          uint32_t d) {
+  if (!g) return FM_ERR_INVALID;
+  const size_t G = g->m.size();
+  if (G == 1) return fm_upload_image(g->m[0], img, desc, scale, lap, n, d);
+  // The owner copies the caller's image: a host image goes to member img % n, a device image to the member on its GPU.
+  // The lead, then every other member, copies a member's device copy it can read as a peer: the owner's, otherwise the
+  // lead's (every member reads the lead's memory).  So each image crosses PCIe at most once.  The lead owns the image
+  // when it cannot read the owner's memory (or the image lies on a GPU outside the group).
+  cudaPointerAttributes attr{};
+  const bool on_device = n && desc && cudaPointerGetAttributes(&attr, desc) == cudaSuccess && attr.type == cudaMemoryTypeDevice;
+  cudaGetLastError();
+  size_t o = img % G;
+  if (on_device) {
+    o = 0;
+    for (size_t k = 0; k < G; k++)
+      if (g->m[k]->device == attr.device) { o = k; break; }
+  }
+  if (!g->peer[0][o]) o = 0;
+  fm_ctx* owner = g->m[o];
+  if (int rc = fm_upload_image(owner, img, desc, scale, lap, n, d)) return o ? member_fail(g, o, rc) : rc;
+  FM_CUDA(g->m[0], cudaSetDevice(owner->device));
+  FM_CUDA(g->m[0], cudaEventRecord(g->ev[o], owner->stream));
+  std::vector<size_t> order;  // the lead first: members that cannot read the owner copy the lead's copy
+  if (o != 0) order.push_back(0);
+  for (size_t k = 1; k < G; k++)
+    if (k != o) order.push_back(k);
+  for (size_t k : order) {
+    const size_t src = g->peer[k][o] ? o : 0;
+    const ImageDev& v = g->m[src]->h_images[img];
+    fm_ctx* c = g->m[k];
+    FM_CUDA(g->m[0], cudaSetDevice(c->device));
+    FM_CUDA(g->m[0], cudaStreamWaitEvent(c->stream, g->ev[src], 0));
+    if (int rc = fm_upload_image(c, img, v.desc, v.scale, v.lap, n, d)) return k ? member_fail(g, k, rc) : rc;
+    FM_CUDA(g->m[0], cudaEventRecord(g->ev[k], c->stream));
+  }
+  // the sources' copies must outlive the members' reads of them (a later upload may reuse their slabs)
+  for (size_t s : {o, (size_t)0}) {
+    FM_CUDA(g->m[0], cudaSetDevice(g->m[s]->device));
+    for (size_t k : order)
+      if (k != s) FM_CUDA(g->m[0], cudaStreamWaitEvent(g->m[s]->stream, g->ev[k], 0));
+  }
+  return FM_OK;
+}
+
+int fm_group_match(fm_group* g, const uint32_t* pair_first, const uint32_t* pair_second, size_t n_pairs, float dist,
+                   float dist2second, uint32_t flags, fm_result** out) {
+  if (!g || !out) return FM_ERR_INVALID;
+  *out = nullptr;
+  const size_t G = g->m.size();
+  fm_ctx* lead = g->m[0];
+  if (G == 1) return fm_match(lead, pair_first, pair_second, n_pairs, dist, dist2second, flags, out);
+  if (n_pairs && (!pair_first || !pair_second)) return fail(lead, FM_ERR_INVALID, "fm_match: null pair arrays");
+  if (!(dist < 1.8e19f)) return fail(lead, FM_ERR_UNSUPPORTED, "fm_match: distance threshold must be below 1.8e19");
+  for (size_t p = 0; p < n_pairs; p++) {  // (every member holds every image: the lead's table speaks for all)
+    uint32_t a = pair_first[p], b = pair_second[p];
+    if (a >= lead->images.size() || b >= lead->images.size() || !lead->images[a].valid || !lead->images[b].valid)
+      return fail(lead, FM_ERR_INVALID, "fm_match: pair " + std::to_string(p) + " names an image that was not uploaded");
+  }
+  if (flags & FM_FLAG_MATCH_ALL) {  // the limit of one context's call, for the whole call rather than each shard
+    uint64_t rows = 0;
+    for (size_t p = 0; p < n_pairs; p++)
+      rows += lead->images[pair_second[p]].n + ((flags & FM_FLAG_SYM) ? lead->images[pair_first[p]].n : 0u);
+    if (rows > 0xFFFFFFF0ull) return fail(lead, FM_ERR_UNSUPPORTED, "fm_match: -all supports at most 2^32 outer-loop rows per call");
+  }
+  // Prepare new images on every member at once: fm_match would otherwise wait for each member's preparation in turn.
+  for (size_t k = 0; k < G; k++)
+    if (int rc = prep_queue(g->m[k])) return member_fail(g, k, rc);
+  for (size_t k = 0; k < G; k++)
+    if (int rc = prep_finish(g->m[k])) return member_fail(g, k, rc);
+
+  std::vector<double> weight(n_pairs);
+  for (size_t p = 0; p < n_pairs; p++) weight[p] = (double)lead->images[pair_first[p]].n * (double)lead->images[pair_second[p]].n;
+  const std::vector<std::vector<size_t>> shard = shard_pairs(weight, (int)G);
+  const bool want_dist = (flags & FM_FLAG_DISTANCES) && !(flags & FM_FLAG_MATCH_ALL);
+
+  fm_result* r = new (std::nothrow) fm_result();
+  if (!r) return fail(lead, FM_ERR_NOMEM, "fm_group_match: out of host memory");
+  r->ctx = lead;
+  r->n_pairs = n_pairs;
+  r->flags = flags;
+  r->ratio = dist2second;
+  std::vector<size_t> part_of(G, SIZE_MAX);  // member -> its entry in r->parts
+  auto bail = [&](int code) {
+    for (auto* c : g->m) { cudaSetDevice(c->device); cudaStreamSynchronize(c->stream); }
+    fm_result_free(r);
+    return code;
+  };
+#define FM_CUDA_G(expr)                                  \
+  do {                                                   \
+    cudaError_t e__ = (expr);                            \
+    if (e__ != cudaSuccess) return bail(cuda_fail(lead, e__, #expr)); \
+  } while (0)
+
+  // Members store into lead buffers taken from the lead's free lists, whose earlier users may still be queued on the
+  // lead stream: members start storing only behind this event.
+  FM_CUDA_G(cudaSetDevice(lead->device));
+  FM_CUDA_G(cudaEventRecord(g->ev_lead, lead->stream));
+  // 1. every member queues the match of its shard (FM_FLAG_MATCH_ALL calls run one after another: they size on the host)
+  {
+    std::vector<uint32_t> pf, ps;
+    for (size_t k = 0; k < G; k++) {
+      if (shard[k].empty()) continue;
+      pf.clear();
+      ps.clear();
+      for (size_t p : shard[k]) { pf.push_back(pair_first[p]); ps.push_back(pair_second[p]); }
+      fm_result* q = nullptr;
+      if (int rc = fm_match(g->m[k], pf.data(), ps.data(), pf.size(), dist, dist2second, flags | FM_FLAG_ASYNC | FM_FLAG_DEVICE_ONLY, &q))
+        return bail(member_fail(g, k, rc));
+      part_of[k] = r->parts.size();
+      r->parts.push_back(GroupPart{});
+      r->parts.back().sub = q;
+      r->slots += q->slots;
+    }
+  }
+  FM_CUDA_G(cudaSetDevice(lead->device));
+  r->d_out = take_buf(lead->out_free, std::max<uint64_t>(r->slots, 1) * sizeof(uint2));
+  r->d_counts = take_buf(lead->counts_free, std::max<size_t>(n_pairs, 1) * sizeof(uint32_t));
+  r->d_goff = take_buf(lead->counts_free, (n_pairs + 1) * sizeof(unsigned long long));
+  if (want_dist) r->d_dist = take_buf(lead->dist_free, std::max<uint64_t>(r->slots, 1) * sizeof(float));
+  FM_CUDA_G(r->d_out.ensure(std::max<uint64_t>(r->slots, 1) * sizeof(uint2)));
+  FM_CUDA_G(r->d_counts.ensure(std::max<size_t>(n_pairs, 1) * sizeof(uint32_t)));
+  FM_CUDA_G(r->d_goff.ensure((n_pairs + 1) * sizeof(unsigned long long)));
+  if (want_dist) FM_CUDA_G(r->d_dist.ensure(std::max<uint64_t>(r->slots, 1) * sizeof(float)));
+  FM_CUDA_G(take_pinned(lead, sizeof(DeviceCounters) + std::max<size_t>(n_pairs, 1) * sizeof(uint32_t), &r->h_block, &r->h_block_cap));
+  memset(r->h_block, 0, sizeof(DeviceCounters));
+
+  // 2. each member's counts to their submission positions on the lead; its local offsets
+  for (size_t k = 0; k < G; k++) {
+    if (part_of[k] == SIZE_MAX) continue;
+    GroupPart& gp = r->parts[part_of[k]];
+    fm_ctx* c = g->m[k];
+    const uint32_t nk = (uint32_t)shard[k].size();
+    FM_CUDA_G(cudaSetDevice(c->device));
+    FM_CUDA_G(take_pinned(c, (size_t)nk * sizeof(uint32_t), &gp.pin, &gp.pin_cap));
+    uint32_t* h_idx = static_cast<uint32_t*>(gp.pin);
+    for (uint32_t i = 0; i < nk; i++) h_idx[i] = (uint32_t)shard[k][i];
+    const size_t loff_bytes = ((size_t)nk + 1) * sizeof(unsigned long long);
+    gp.scratch = take_buf(c->counts_free, loff_bytes + (size_t)nk * sizeof(uint32_t));
+    FM_CUDA_G(gp.scratch.ensure(loff_bytes + (size_t)nk * sizeof(uint32_t)));
+    unsigned long long* loff = gp.scratch.as<unsigned long long>();
+    uint32_t* d_idx = reinterpret_cast<uint32_t*>(loff + nk + 1);
+    FM_CUDA_G(cudaMemcpyAsync(d_idx, h_idx, (size_t)nk * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+    if (k) FM_CUDA_G(cudaStreamWaitEvent(c->stream, g->ev_lead, 0));
+    const uint32_t* counts = gp.sub->d_counts.as<uint32_t>();
+    group_counts_kernel<<<(nk + 255) / 256, 256, 0, c->stream>>>(counts, d_idx, nk, r->d_counts.as<uint32_t>());
+    links_scan_kernel<<<1, 1024, 0, c->stream>>>(counts, nk, loff);
+    FM_CUDA_G(cudaGetLastError());
+    FM_CUDA_G(cudaEventRecord(g->ev[k], c->stream));
+  }
+  // 3. the lead scans the gathered counts into submission-order offsets
+  FM_CUDA_G(cudaSetDevice(lead->device));
+  for (size_t k = 1; k < G; k++)
+    if (part_of[k] != SIZE_MAX) FM_CUDA_G(cudaStreamWaitEvent(lead->stream, g->ev[k], 0));
+  links_scan_kernel<<<1, 1024, 0, lead->stream>>>(r->d_counts.as<uint32_t>(), (uint32_t)n_pairs, r->d_goff.as<unsigned long long>());
+  FM_CUDA_G(cudaGetLastError());
+  FM_CUDA_G(cudaEventRecord(g->ev_lead, lead->stream));
+  // 4. each member pushes its lists into the lead's buffer; its own buffers go back to its free lists when they have
+  // room (stream order keeps them until the push has read them), else at fm_result_free
+  for (size_t k = 0; k < G; k++) {
+    if (part_of[k] == SIZE_MAX) continue;
+    GroupPart& gp = r->parts[part_of[k]];
+    fm_ctx* c = g->m[k];
+    fm_result* q = gp.sub;
+    const uint32_t nk = (uint32_t)shard[k].size();
+    FM_CUDA_G(cudaSetDevice(c->device));
+    if (k) FM_CUDA_G(cudaStreamWaitEvent(c->stream, g->ev_lead, 0));
+    const unsigned long long* loff = gp.scratch.as<unsigned long long>();
+    const uint32_t* d_idx = reinterpret_cast<const uint32_t*>(loff + nk + 1);
+    const unsigned grid = (nk + kGatherWarps - 1) / kGatherWarps;
+    if (want_dist)
+      group_push_kernel<true><<<grid, kGatherThreads, 0, c->stream>>>(q->d_out.as<uint2>(), q->d_dist.as<float>(), loff, d_idx, nk,
+                                                                      r->d_goff.as<unsigned long long>(), r->d_out.as<uint2>(), r->d_dist.as<float>());
+    else
+      group_push_kernel<false><<<grid, kGatherThreads, 0, c->stream>>>(q->d_out.as<uint2>(), nullptr, loff, d_idx, nk,
+                                                                       r->d_goff.as<unsigned long long>(), r->d_out.as<uint2>(), nullptr);
+    FM_CUDA_G(cudaGetLastError());
+    FM_CUDA_G(cudaEventRecord(g->ev[k], c->stream));
+    give_buf_queued(c->out_free, q->d_out);
+    give_buf_queued(c->counts_free, q->d_counts);
+    give_buf_queued(c->dist_free, q->d_dist);
+  }
+  // 5. the lead waits for every push; total and counts to the result's pinned block, as fm_match leaves them
+  FM_CUDA_G(cudaSetDevice(lead->device));
+  for (size_t k = 1; k < G; k++)
+    if (part_of[k] != SIZE_MAX) FM_CUDA_G(cudaStreamWaitEvent(lead->stream, g->ev[k], 0));
+  FM_CUDA_G(cudaMemcpyAsync(static_cast<char*>(r->h_block) + offsetof(DeviceCounters, running_total), r->d_goff.as<unsigned long long>() + n_pairs,
+                            sizeof(unsigned long long), cudaMemcpyDeviceToHost, lead->stream));
+  if (n_pairs)
+    FM_CUDA_G(cudaMemcpyAsync(static_cast<char*>(r->h_block) + sizeof(DeviceCounters), r->d_counts.p, n_pairs * sizeof(uint32_t),
+                              cudaMemcpyDeviceToHost, lead->stream));
+  r->done = r->ev.get();
+  FM_CUDA_G(cudaEventRecord(r->done, lead->stream));
+#undef FM_CUDA_G
+  if (!(flags & FM_FLAG_ASYNC)) {
+    int rc = fm_result_wait(r);
+    if (rc != FM_OK) { fm_result_free(r); return rc; }
+  }
+  *out = r;
+  return FM_OK;
+}
+
 // ---- debug / test hooks (include/frogmatch_debug.h) ---------------------------------------------
 
 int fm_debug_set_option(const char* name, int value) {
@@ -982,6 +1384,7 @@ int fm_debug_set_option(const char* name, int value) {
   else if (!strcmp(name, "surv_cap")) g_debug.surv_cap = value;
   else if (!strcmp(name, "compact_v")) g_debug.compact_v = value;
   else if (!strcmp(name, "reject_dump")) g_debug.reject_dump = value;
+  else if (!strcmp(name, "group_repeat")) g_debug.group_repeat = value;
   else return FM_ERR_INVALID;
   return FM_OK;
 }

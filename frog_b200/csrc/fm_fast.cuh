@@ -124,6 +124,7 @@ struct DebugOptions {
   int compact_v = 3;   // large-batch compaction (fm_compact.cuh): 3 = warp-autonomous pipelined count, 2 = pipelined count with the
                        // block-wide ranking, 1 = the first version (one CTA per chunk, scan with the per-pair counts)
   int reject_dump = 0;  // two-phase scoring: 1 = keep every task's reject-pass output on the host (fm_debug_reject_rows)
+  int group_repeat = 0;  // 1 = fm_group_create takes a device more than once (one context per entry): the group path on one GPU
 };
 inline DebugOptions g_debug;
 

@@ -60,6 +60,7 @@
 #include <vector>
 
 #include "frogmatch.h"
+#include "fm_shard.h"
 #include "frogsurf.h"
 #include "keypoint_io.h"
 #include "surf_io.h"
@@ -797,21 +798,13 @@ int run_job(int argc, char* argv[], std::ostream& cout, std::ostream& cerr, Warm
   if (target >= nb) { cerr << "match: -targ " << target << " is not a valid image index" << endl; return leave(1); }
 
   cout << "Pairing... " << endl;
-  std::vector<std::vector<size_t>> shard(G);
+  std::vector<std::vector<size_t>> shard;
   {
-    // longest-processing-time-first sharding of image pairs (independent units, match.cpp:638-652)
-    std::vector<size_t> order(indices.size());
-    std::iota(order.begin(), order.end(), 0);
-    auto weight = [&](size_t id) { return (double)images[indices[id].first].n * (double)images[indices[id].second].n; };
-    std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t b) { return weight(a) > weight(b); });
-    std::vector<double> load(G, 0.0);
-    for (size_t id : order) {
-      int g = (int)(std::min_element(load.begin(), load.end()) - load.begin());
-      shard[g].push_back(id);
-      load[g] += weight(id);
-    }
+    std::vector<double> weight(indices.size());
+    for (size_t id = 0; id < indices.size(); id++)
+      weight[id] = (double)images[indices[id].first].n * (double)images[indices[id].second].n;
+    shard = fm::shard_pairs(weight, G);
     for (int g = 0; g < G; g++) {
-      std::sort(shard[g].begin(), shard[g].end());  // consecutive pairs share the first image
       WorkerSlot& w = ctl->worker[g];
       w.n_pairs = shard[g].size();
       w.pairs_off = ctl->alloc(std::max<uint64_t>(w.n_pairs, 1) * 2 * sizeof(uint32_t));

@@ -10,9 +10,10 @@
  * Conventions: plain C, plain pointers and sizes.  Every function returns FM_OK (0) or a negative
  * fm_status and never throws.  Input pointers are borrowed for the duration of the call; results
  * are owned by the library until fm_result_free().  A context is bound to ONE CUDA device and
- * must be used from one host thread at a time; multi-GPU callers create one context per device
+ * must be used from one host thread at a time; multi-GPU callers either create one context per device
  * (one per thread or one per process/rank) and shard image pairs between them -- image pairs are
- * independent (match.cpp:638-652), so no data-path collective is needed.
+ * independent (match.cpp:638-652), so no data-path collective is needed -- or use one fm_group (below),
+ * which does that in-process and gathers the lists on one GPU.
  *
  * There is NO CPU fallback: without a CUDA device fm_create() fails with FM_ERR_CUDA.
  */
@@ -189,8 +190,49 @@ typedef struct fm_stats {
 
 /* Statistics of the most recent fm_match on this context (synchronises the stream). */
 int fm_get_stats(fm_ctx* ctx, fm_stats* out);
-/* Statistics of the call that produced `r` (waits for it; ms_prep is not attributed to a call: 0). */
+/* Statistics of the call that produced `r` (waits for it; ms_prep is not attributed to a call: 0).  For a result of
+ * fm_group_match the counters are summed over the members' calls and each ms_* field is the maximum over members. */
 int fm_result_stats(fm_result* r, fm_stats* out);
+
+/* ---- device groups: one library handle over several GPUs --------------------------------------------------------- */
+
+/*
+ * A group is one fm_ctx per device, used as one: every member holds every image, fm_group_match splits the pairs over
+ * the members and gathers their lists over NVLink into one result on the LEAD device (devices[0]), in submission
+ * order.  Like a context, a group is used from one host thread at a time.
+ */
+typedef struct fm_group fm_group;
+/* Create a group over `n` distinct devices; devices[0] is the lead.  Enables peer access between every ordered pair of
+ * members that supports it (process state, left enabled by fm_group_destroy); every member must be able to access the
+ * lead.  FM_ERR_INVALID for a repeated or out-of-range device, FM_ERR_UNSUPPORTED when a member cannot access the lead
+ * as a peer, FM_ERR_CUDA without a device; the text is in fm_group_last_error(NULL).  A group of one device behaves
+ * exactly like fm_create(devices[0]). */
+int fm_group_create(const int* devices, int n, fm_group** out);
+/* Destroy a group.  Every fm_result it produced must have been freed first. */
+void fm_group_destroy(fm_group* g);
+/* Text of the most recent error on this group (NULL: of the last failed fm_group_create on this thread).  Never NULL. */
+const char* fm_group_last_error(const fm_group* g);
+/* Block until every member's queued work has finished. */
+int fm_group_synchronize(fm_group* g);
+int fm_group_clear_images(fm_group* g);
+/* fm_upload_image on every member (same arguments and checks).  The image is copied once to its owner: member img % n
+ * for a host image, the member on the image's GPU for device memory (the lead when it cannot access the owner as a
+ * peer, or for device memory outside the group).  Every other member then copies, GPU to GPU, the device copy of a
+ * member it can access as a peer: the owner's, otherwise the lead's.  So a host image crosses PCIe once.  Pinned and
+ * device buffers must stay valid until the next fm_group_synchronize / fm_group_match. */
+int fm_group_upload_image(fm_group* g, uint32_t img, const float* desc, const float* scale, const float* lap, uint32_t n,
+                          uint32_t d);
+/* fm_match over the group, with the same arguments and flags.  Pairs are split longest-first by N_first * N_second;
+ * each member matches its share; the lists (and distances) are then stored into the lead's memory at their
+ * submission-order offsets, all in stream order.  The result is an ordinary fm_result of the lead (every fm_result_*
+ * call and fm_links_build take it; link image indices are the lead's, which are all of them), byte-identical to what
+ * one context returns for the same call.  Its device views are on the lead.  Members run their shares with
+ * FM_FLAG_ASYNC, so a group never probes the first batch of a synchronous call to switch to two-phase scoring within
+ * that call (see fm_match): the first call at dist2second < 1 runs single-pass where one context might not, and later
+ * calls use each member's rejection rate of its previous call.  Results are exact either way.  The -all row limit
+ * applies to the whole call, as for one context. */
+int fm_group_match(fm_group* g, const uint32_t* pair_first, const uint32_t* pair_second, size_t n_pairs, float dist,
+                   float dist2second, uint32_t flags, fm_result** out);
 
 /* Library/build description, e.g. "frogmatch 0.1 sm_100a". */
 const char* fm_version(void);

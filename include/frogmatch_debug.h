@@ -119,6 +119,8 @@ int fm_debug_compact(fm_ctx* ctx, const uint32_t* rowres, const float* rowdist, 
  *   "compact_v" 3|2|1   version of the three-launch compaction (batches of more than 1536 chunks) -- results stay exact
  *   "reject_dump" 0|1   two-phase scoring: keep what the reject pass computed for fm_debug_reject_rows (a dump build
  *                       of the reject kernel and a synchronisation per batch) -- results stay exact
+ *   "group_repeat" 0|1  fm_group_create accepts a device more than once, one context per entry, so that the whole group
+ *                       path (sharding, gather, ordering) runs on one GPU -- results stay exact
  * Returns FM_ERR_INVALID for an unknown name.  Nothing reads environment variables.
  */
 int fm_debug_set_option(const char* name, int value);
