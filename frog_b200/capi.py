@@ -20,6 +20,9 @@ FLAG_DEVICE_ONLY = 4
 FLAG_ASYNC = 8
 FLAG_MATCH_ALL = 16
 FLAG_DISTANCES = 32
+FLAG_ROW_TABLE = 64
+# one row of a row table (fm_row, include/frogmatch.h)
+ROW_DTYPE = np.dtype([("d1", "<f4"), ("d2", "<f4"), ("nearest", "<u4")])
 
 # every symbol include/frogmatch.h declares (checked by tests/test_abi.py)
 PUBLIC_SYMBOLS = [
@@ -31,6 +34,7 @@ PUBLIC_SYMBOLS = [
     "fm_links_device_data", "fm_links_build_ms", "fm_links_free",
     "fm_group_create", "fm_group_destroy", "fm_group_last_error", "fm_group_synchronize", "fm_group_clear_images",
     "fm_group_upload_image", "fm_group_match",
+    "fm_result_select", "fm_result_rows_device", "fm_result_row_offset", "fm_result_rows_copy",
 ]
 DEBUG_SYMBOLS = ["fm_debug_image", "fm_debug_image_norms", "fm_debug_score_unit", "fm_debug_set_option",
                  "fm_debug_reject_rows", "fm_debug_wide_unit", "fm_debug_compact"]
@@ -132,6 +136,12 @@ def load():
     L.fm_group_clear_images.argtypes = [vp]
     L.fm_group_upload_image.argtypes = [vp, C.c_uint32, vp, vp, vp, C.c_uint32, C.c_uint32]
     L.fm_group_match.argtypes = [vp, vp, vp, C.c_size_t, C.c_float, C.c_float, C.c_uint32, C.POINTER(vp)]
+    L.fm_result_select.argtypes = [vp, C.c_float, C.c_float, C.c_uint32, C.POINTER(vp)]
+    L.fm_result_rows_device.argtypes = [vp]
+    L.fm_result_rows_device.restype = vp
+    L.fm_result_row_offset.argtypes = [vp, C.c_size_t]
+    L.fm_result_row_offset.restype = C.c_uint64
+    L.fm_result_rows_copy.argtypes = [vp, C.c_size_t, vp]
     _lib = L
     return L
 
@@ -140,10 +150,11 @@ def _ptr(a: np.ndarray):
     return a.ctypes.data_as(C.c_void_p)
 
 
-def _flags(sym, force_exact, device_only, asynchronous, match_all, distances) -> int:
+def _flags(sym, force_exact, device_only, asynchronous, match_all, distances, row_table=False) -> int:
     return (FLAG_SYM if sym else 0) | (FLAG_FORCE_EXACT if force_exact else 0) | \
         (FLAG_DEVICE_ONLY if device_only else 0) | (FLAG_ASYNC if asynchronous else 0) | \
-        (FLAG_MATCH_ALL if match_all else 0) | (FLAG_DISTANCES if distances else 0)
+        (FLAG_MATCH_ALL if match_all else 0) | (FLAG_DISTANCES if distances else 0) | \
+        (FLAG_ROW_TABLE if row_table else 0)
 
 
 class Result:
@@ -234,6 +245,31 @@ class Result:
     def all_pairs(self):
         return [self.pairs(p) for p in range(self.n_pairs)]
 
+    def select(self, dist: float, ratio: float, distances: bool = False, device_only: bool = False,
+               asynchronous: bool = False) -> "Result":
+        """The lists match() would return at (dist, ratio) on the same pairs, from this result's row table
+        (match(..., row_table=True)) without scoring again: a new, independent Result."""
+        flags = _flags(False, False, device_only, asynchronous, False, distances)
+        h = C.c_void_p()
+        self._m._check(self._m._L.fm_result_select(self._h, dist, ratio, flags, C.byref(h)))
+        return Result(self._m, h, pending=asynchronous)
+
+    def row_offset(self, p: int) -> int:
+        """First row of pair p in the row table (p == n_pairs: the number of rows)."""
+        return int(self._m._L.fm_result_row_offset(self._h, p))
+
+    def rows(self, p: int) -> np.ndarray:
+        """Pair p's rows of the row table: a structured array (d1, d2, nearest) -- N_second rows in keypoint order,
+        then, with sym, the reverse direction's N_first rows."""
+        n = self.row_offset(p + 1) - self.row_offset(p)
+        out = np.zeros(max(n, 0), ROW_DTYPE)
+        self._m._check(self._m._L.fm_result_rows_copy(self._h, p, _ptr(out)))
+        return out
+
+    def rows_device_pointer(self) -> int:
+        """Raw device address of the whole row table (None for a group of several devices or without a table)."""
+        return self._m._L.fm_result_rows_device(self._h)
+
     def device_pointers(self):
         """(counts_ptr, pairs_ptr) raw device addresses, for GPU-to-GPU gathers."""
         L = self._m._L
@@ -308,10 +344,10 @@ class Matcher:
 
     def match(self, pair_first, pair_second, dist: float = 0.22, ratio: float = 1.0, sym: bool = False,
               force_exact: bool = False, device_only: bool = False, asynchronous: bool = False,
-              match_all: bool = False, distances: bool = False) -> Result:
+              match_all: bool = False, distances: bool = False, row_table: bool = False) -> Result:
         pf = np.ascontiguousarray(pair_first, np.uint32)
         ps = np.ascontiguousarray(pair_second, np.uint32)
-        flags = _flags(sym, force_exact, device_only, asynchronous, match_all, distances)
+        flags = _flags(sym, force_exact, device_only, asynchronous, match_all, distances, row_table)
         h = C.c_void_p()
         self._check(self._L.fm_match(self._h, _ptr(pf), _ptr(ps), pf.shape[0], dist, ratio, flags, C.byref(h)))
         return Result(self, h, pending=asynchronous)
@@ -464,10 +500,10 @@ class Group:
 
     def match(self, pair_first, pair_second, dist: float = 0.22, ratio: float = 1.0, sym: bool = False,
               force_exact: bool = False, device_only: bool = False, asynchronous: bool = False,
-              match_all: bool = False, distances: bool = False) -> Result:
+              match_all: bool = False, distances: bool = False, row_table: bool = False) -> Result:
         pf = np.ascontiguousarray(pair_first, np.uint32)
         ps = np.ascontiguousarray(pair_second, np.uint32)
-        flags = _flags(sym, force_exact, device_only, asynchronous, match_all, distances)
+        flags = _flags(sym, force_exact, device_only, asynchronous, match_all, distances, row_table)
         h = C.c_void_p()
         self._check(self._L.fm_group_match(self._h, _ptr(pf), _ptr(ps), pf.shape[0], dist, ratio, flags, C.byref(h)))
         return Result(self, h, pending=asynchronous)

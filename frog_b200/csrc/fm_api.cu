@@ -14,16 +14,25 @@
 #include "fm_group.cuh"
 #include "fm_host.h"
 #include "fm_links.cuh"
+#include "fm_select.cuh"
 #include "fm_shard.h"
 #include "fm_wide.cuh"
 
 using namespace fm;
+
+// One batch of a row-table call, as fm_result_select needs it: its rows' place in the table and its chunk records.
+struct SelectBatch {
+  uint64_t row0;  // first table row of the batch
+  uint32_t rows, chunk0, chunks;  // chunk0: first record in fm_result::sel_chunks
+};
 
 // One member's share of a group result (fm_group_match): the member's own result of its shard, whose device buffers go
 // back to the member's free lists once the gather is queued (its pinned block and events stay until the group result is
 // complete), and the member-side scratch of the gather.
 struct GroupPart {
   fm_result* sub = nullptr;
+  uint32_t member = 0;            // the member's index in the group
+  std::vector<uint32_t> idx;      // submission indices of the member's pairs, in its call's order
   DevBuf scratch;                 // member device: local offsets (n + 1 u64) | global positions (n u32)
   void* pin = nullptr;            // member's pinned staging of the global positions
   size_t pin_cap = 0;
@@ -54,6 +63,15 @@ struct fm_result {
   // group results (fm_group_match): one part per member that had pairs; the lead's submission-order offsets
   std::vector<GroupPart> parts;
   DevBuf d_goff;
+  fm_group* group = nullptr;  // the group of a group result (fm_result_select gathers through it)
+  // FM_FLAG_ROW_TABLE: the table, and the host records fm_result_select compacts with (a group result holds no table of
+  // its own: each part's result holds its share's)
+  bool table = false;
+  DevBuf d_table;                         // one fm_row per outer-loop row, task after task
+  std::vector<uint64_t> row_off;          // n_pairs + 1: pair p's first row, submission order over the whole call
+  std::vector<SelectBatch> sel_batches;   // the call's batches
+  std::vector<ChunkDesc> sel_chunks;      // their compaction chunk records, batch after batch
+  std::vector<uint32_t> pair_part, pair_local;  // group result: pair p's part and its index in that part's call
 };
 
 struct fm_links {
@@ -241,6 +259,22 @@ int finalize(fm_result* r) {
   if (r->offsets[r->n_pairs] != r->total)
     return fail(c, FM_ERR_CUDA, "fm_match: internal error, per-pair counts do not sum to the compacted total");
   return FM_OK;
+}
+
+// The common end of a call on one context: totals and per-pair counts to the result's pinned block, `done` behind them,
+// and the call's counters and event brackets handed to the result.
+cudaError_t queue_tail(fm_ctx* c, fm_result* r) {
+  cudaError_t e = cudaMemcpyAsync(r->h_block, c->d_totals.p, sizeof(DeviceCounters), cudaMemcpyDeviceToHost, c->stream);
+  if (e == cudaSuccess && r->n_pairs)
+    e = cudaMemcpyAsync(static_cast<char*>(r->h_block) + sizeof(DeviceCounters), r->d_counts.p, r->n_pairs * sizeof(uint32_t),
+                        cudaMemcpyDeviceToHost, c->stream);
+  if (e != cudaSuccess) return e;
+  r->done = c->ev_match.get();
+  if ((e = cudaEventRecord(r->done, c->stream)) != cudaSuccess) return e;
+  r->stats = c->stats;
+  r->ev = std::move(c->ev_match);
+  c->ev_match = EventPool{};
+  return cudaSuccess;
 }
 
 struct Batch {
@@ -490,6 +524,8 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
   // stale column id) only if sqrt(FLT_MAX) = 1.8e19 < dist.  No caller passes such a threshold
   // (FROG.py uses 1e10); refuse it rather than imitate an index leak.
   if (!(dist < 1.8e19f)) return fail(c, FM_ERR_UNSUPPORTED, "fm_match: distance threshold must be below 1.8e19");
+  if ((flags & FM_FLAG_ROW_TABLE) && (flags & FM_FLAG_MATCH_ALL))
+    return fail(c, FM_ERR_INVALID, "fm_match: FM_FLAG_ROW_TABLE does not combine with FM_FLAG_MATCH_ALL");
   FM_CUDA(c, cudaSetDevice(c->device));
   for (size_t p = 0; p < n_pairs; p++) {
     uint32_t a = pair_first[p], b = pair_second[p];
@@ -501,6 +537,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
   const bool sym = flags & FM_FLAG_SYM;
   const bool match_all = flags & FM_FLAG_MATCH_ALL;
   const bool force_exact = (flags & FM_FLAG_FORCE_EXACT) != 0;
+  const bool table = (flags & FM_FLAG_ROW_TABLE) != 0;
   // d != 48: the wide tensor-core path (fm_wide.cuh); images it cannot take (kImgBadDim and the other flags) are exact
   const bool wide = c->dim != (uint32_t)kD;
 
@@ -574,8 +611,24 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
   r->n_pairs = n_pairs;
   r->flags = flags;
   r->ratio = dist2second;
-  r->d48 = !wide;
+  r->d48 = !wide && !table;  // (a table call rejects nothing early: it says nothing about the two-phase choice)
   r->slots = total_rows;
+  if (table) {
+    // first, so that a table that does not fit leaves nothing behind
+    cudaError_t e = r->d_table.ensure(std::max<uint64_t>(total_rows, 1) * sizeof(fm_row));
+    if (e != cudaSuccess) {
+      cudaGetLastError();  // (an allocation failure is not sticky: clear it for the context's next call)
+      delete r;
+      return cuda_fail(c, e, ("fm_match: row table of " + std::to_string(total_rows) + " rows").c_str());
+    }
+    r->table = true;
+    r->row_off.assign(n_pairs + 1, 0);
+    for (size_t p = 0; p < n_pairs; p++)
+      r->row_off[p + 1] = r->row_off[p] + c->images[pair_second[p]].n + (sym ? c->images[pair_first[p]].n : 0u);
+    for (size_t bi = 0, row0 = 0; bi < batches.size(); row0 += batches[bi].rows, bi++)
+      r->sel_batches.push_back(SelectBatch{row0, batches[bi].rows, (uint32_t)chunk_cursor[bi], batches[bi].chunks});
+    r->sel_chunks = chunk_desc;
+  }
   r->d_out = take_buf(c->out_free, std::max<uint64_t>(total_rows, 1) * sizeof(uint2));
   r->d_counts = take_buf(c->counts_free, std::max<size_t>(n_pairs, 1) * sizeof(uint32_t));
   const bool want_dist = (flags & FM_FLAG_DISTANCES) && !match_all;
@@ -677,7 +730,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
                                                                                  row_final, nullptr, nullptr, nullptr, nullptr);
         else
           exact_generic_kernel<1><<<b.blocks, kExactRows, 0, c->stream>>>(d_images, d_tasks, d_blk, n_tasks, dist, 1.f, 0u, nullptr, row_count,
-                                                                          row_final, nullptr, nullptr, nullptr, nullptr, nullptr);
+                                                                          row_final, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
         all_scan_kernel<<<(n_tasks + 63) / 64, 64, 0, c->stream>>>(d_images, d_tasks, n_tasks, row_count, row_final, row_carry, row_off,
                                                                     d_task_total);
       }
@@ -700,7 +753,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
                                                                                 row_carry, row_off, d_task_base, r->d_out.as<uint2>());
         else
           exact_generic_kernel<2><<<b.blocks, kExactRows, 0, c->stream>>>(d_images, d_tasks, d_blk, n_tasks, dist, 1.f, 0u, nullptr, nullptr,
-                                                                          nullptr, row_carry, row_off, d_task_base, r->d_out.as<uint2>(), nullptr);
+                                                                          nullptr, row_carry, row_off, d_task_base, r->d_out.as<uint2>(), nullptr, nullptr);
       }
       FM_CUDA_R(cudaStreamSynchronize(c->stream));  // task_base (pageable) must outlive the copy
       c->stats.kernel_launches += 3;
@@ -720,19 +773,22 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
     // call of this kind on this context rejected >= 99 % of its rows, or, inside a synchronous multi-batch call, once
     // the first batch (single pass) has shown that much.
     constexpr double kTwoPhaseMin = 0.99;
-    const bool two_phase_possible = dist2second < 1.f && segs == 1 && !force_exact && !wide;  // reject pass: K = 64 only
+    // (reject pass: K = 64 only; a row table needs every row's exact distances)
+    const bool two_phase_possible = dist2second < 1.f && segs == 1 && !force_exact && !wide && !table;
     bool two_phase = two_phase_possible && c->reject_hint >= kTwoPhaseMin;
     bool probed = false;
     if (g_debug.two_phase >= 0) {  // test hook: force the choice
       two_phase = two_phase_possible && g_debug.two_phase != 0;
       probed = true;
     }
-    for (size_t bi = 0; bi < batches.size(); bi++) {
+    uint64_t row0 = 0;  // the batch's first row in the call
+    for (size_t bi = 0; bi < batches.size(); row0 += batches[bi].rows, bi++) {
       const Batch& b = batches[bi];
       const uint32_t nt = b.t1 - b.t0;
       const uint32_t* blk = d_blk + b.cursor;
       const uint32_t* unt = d_unit + b.cursor;
       if (b.rows == 0) continue;
+      fm_row* tab = table ? r->d_table.as<fm_row>() + row0 : nullptr;
       if (b.any_fast) {
         FastBatchArgs fa{};
         fa.images = d_images;
@@ -752,6 +808,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
         fa.ratio = dist2second;
         fa.rowres = d_rowres;
         fa.rowdist = d_rowdist;
+        fa.table = tab;
         fa.two_phase = two_phase;
         fa.counters = d_counters;
         cudaError_t e = wide ? wide_match_batch(c, fa) : fast_match_batch(c, fa);
@@ -765,10 +822,10 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
         Span sp(&c->ev_match, c->stream, kPhExact);
         if (c->dim == (uint32_t)kD)
           exact_match_kernel<kD><<<b.blocks, kExactRows, exact_smem_bytes(kD), c->stream>>>(
-              d_images, d_tasks + b.t0, blk, nt, dist, dist2second, kTaskExact, d_rowres, d_rowdist);
+              d_images, d_tasks + b.t0, blk, nt, dist, dist2second, kTaskExact, d_rowres, d_rowdist, tab);
         else
           exact_generic_kernel<0><<<b.blocks, kExactRows, 0, c->stream>>>(d_images, d_tasks + b.t0, blk, nt, dist, dist2second, kTaskExact,
-                                                                          d_rowres, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, d_rowdist);
+                                                                          d_rowres, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, d_rowdist, tab);
         c->stats.kernel_launches++;
         for (uint32_t t = b.t0; t < b.t1; t++)
           if (tasks[t].flags & kTaskExact) c->stats.rows_exact += c->images[tasks[t].row_img].n;
@@ -798,17 +855,7 @@ int fm_match(fm_ctx* c, const uint32_t* pair_first, const uint32_t* pair_second,
     }
   }
   FM_CUDA_R(cudaGetLastError());
-
-  // ---- totals and per-pair counts to a pinned block; (optionally) the lists to the host ----------
-  FM_CUDA_R(cudaMemcpyAsync(r->h_block, c->d_totals.p, sizeof(DeviceCounters), cudaMemcpyDeviceToHost, c->stream));
-  if (n_pairs)
-    FM_CUDA_R(cudaMemcpyAsync(static_cast<char*>(r->h_block) + sizeof(DeviceCounters), r->d_counts.p, n_pairs * sizeof(uint32_t),
-                              cudaMemcpyDeviceToHost, c->stream));
-  r->done = c->ev_match.get();
-  FM_CUDA_R(cudaEventRecord(r->done, c->stream));
-  r->stats = c->stats;
-  r->ev = std::move(c->ev_match);
-  c->ev_match = EventPool{};
+  FM_CUDA_R(queue_tail(c, r));
   c->last = r;
   if (!(flags & FM_FLAG_ASYNC)) {
     rc = fm_result_wait(r);
@@ -875,6 +922,10 @@ void fm_result_free(fm_result* r) {
   cudaSetDevice(c->device);
   if (r->done && !r->waited) cudaEventSynchronize(r->done);  // the pinned block is still a copy target
   if (c->last == r) c->last = nullptr;
+  if (r->d_table.p) {  // fm_result_select calls may still read the table
+    cudaStreamSynchronize(c->stream);
+    r->d_table.release();
+  }
   // hand the buffers and events back to the context so the next call does not reallocate
   give_buf(c->out_free, r->d_out);
   give_buf(c->counts_free, r->d_counts);
@@ -1067,6 +1118,100 @@ int member_fail(fm_group* g, size_t k, int code) {
   return group_fail(g, code, "device " + std::to_string(g->m[k]->device) + ": " + g->m[k]->err);
 }
 
+// Steps 2-5 of a group call, behind the members' calls r->parts (each a device-only FM_FLAG_ASYNC result of member
+// parts[i].member over the pairs parts[i].idx; the caller recorded g->ev_lead on the lead stream before queueing them):
+// gather their counts and lists into r's buffers on the lead, in submission order, all in stream order, and record
+// r->done behind it.  On error the caller frees r (after synchronising the members).
+int group_gather(fm_group* g, fm_result* r) {
+  fm_ctx* lead = g->m[0];
+  const size_t G = g->m.size(), n_pairs = r->n_pairs;
+  const bool want_dist = (r->flags & FM_FLAG_DISTANCES) && !(r->flags & FM_FLAG_MATCH_ALL);
+#define FM_CUDA_G(expr)                                  \
+  do {                                                   \
+    cudaError_t e__ = (expr);                            \
+    if (e__ != cudaSuccess) return cuda_fail(lead, e__, #expr); \
+  } while (0)
+  FM_CUDA_G(cudaSetDevice(lead->device));
+  r->d_out = take_buf(lead->out_free, std::max<uint64_t>(r->slots, 1) * sizeof(uint2));
+  r->d_counts = take_buf(lead->counts_free, std::max<size_t>(n_pairs, 1) * sizeof(uint32_t));
+  r->d_goff = take_buf(lead->counts_free, (n_pairs + 1) * sizeof(unsigned long long));
+  if (want_dist) r->d_dist = take_buf(lead->dist_free, std::max<uint64_t>(r->slots, 1) * sizeof(float));
+  FM_CUDA_G(r->d_out.ensure(std::max<uint64_t>(r->slots, 1) * sizeof(uint2)));
+  FM_CUDA_G(r->d_counts.ensure(std::max<size_t>(n_pairs, 1) * sizeof(uint32_t)));
+  FM_CUDA_G(r->d_goff.ensure((n_pairs + 1) * sizeof(unsigned long long)));
+  if (want_dist) FM_CUDA_G(r->d_dist.ensure(std::max<uint64_t>(r->slots, 1) * sizeof(float)));
+  FM_CUDA_G(take_pinned(lead, sizeof(DeviceCounters) + std::max<size_t>(n_pairs, 1) * sizeof(uint32_t), &r->h_block, &r->h_block_cap));
+  memset(r->h_block, 0, sizeof(DeviceCounters));
+
+  // 2. each member's counts to their submission positions on the lead; its local offsets
+  for (GroupPart& gp : r->parts) {
+    const size_t k = gp.member;
+    fm_ctx* c = g->m[k];
+    const uint32_t nk = (uint32_t)gp.idx.size();
+    FM_CUDA_G(cudaSetDevice(c->device));
+    FM_CUDA_G(take_pinned(c, (size_t)nk * sizeof(uint32_t), &gp.pin, &gp.pin_cap));
+    uint32_t* h_idx = static_cast<uint32_t*>(gp.pin);
+    for (uint32_t i = 0; i < nk; i++) h_idx[i] = gp.idx[i];
+    const size_t loff_bytes = ((size_t)nk + 1) * sizeof(unsigned long long);
+    gp.scratch = take_buf(c->counts_free, loff_bytes + (size_t)nk * sizeof(uint32_t));
+    FM_CUDA_G(gp.scratch.ensure(loff_bytes + (size_t)nk * sizeof(uint32_t)));
+    unsigned long long* loff = gp.scratch.as<unsigned long long>();
+    uint32_t* d_idx = reinterpret_cast<uint32_t*>(loff + nk + 1);
+    FM_CUDA_G(cudaMemcpyAsync(d_idx, h_idx, (size_t)nk * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+    if (k) FM_CUDA_G(cudaStreamWaitEvent(c->stream, g->ev_lead, 0));
+    const uint32_t* counts = gp.sub->d_counts.as<uint32_t>();
+    group_counts_kernel<<<(nk + 255) / 256, 256, 0, c->stream>>>(counts, d_idx, nk, r->d_counts.as<uint32_t>());
+    links_scan_kernel<<<1, 1024, 0, c->stream>>>(counts, nk, loff);
+    FM_CUDA_G(cudaGetLastError());
+    FM_CUDA_G(cudaEventRecord(g->ev[k], c->stream));
+  }
+  // 3. the lead scans the gathered counts into submission-order offsets
+  FM_CUDA_G(cudaSetDevice(lead->device));
+  for (const GroupPart& gp : r->parts)
+    if (gp.member) FM_CUDA_G(cudaStreamWaitEvent(lead->stream, g->ev[gp.member], 0));
+  links_scan_kernel<<<1, 1024, 0, lead->stream>>>(r->d_counts.as<uint32_t>(), (uint32_t)n_pairs, r->d_goff.as<unsigned long long>());
+  FM_CUDA_G(cudaGetLastError());
+  FM_CUDA_G(cudaEventRecord(g->ev_lead, lead->stream));
+  // 4. each member pushes its lists into the lead's buffer; its own buffers go back to its free lists when they have
+  // room (stream order keeps them until the push has read them), else at fm_result_free
+  for (GroupPart& gp : r->parts) {
+    const size_t k = gp.member;
+    fm_ctx* c = g->m[k];
+    fm_result* q = gp.sub;
+    const uint32_t nk = (uint32_t)gp.idx.size();
+    FM_CUDA_G(cudaSetDevice(c->device));
+    if (k) FM_CUDA_G(cudaStreamWaitEvent(c->stream, g->ev_lead, 0));
+    const unsigned long long* loff = gp.scratch.as<unsigned long long>();
+    const uint32_t* d_idx = reinterpret_cast<const uint32_t*>(loff + nk + 1);
+    const unsigned grid = (nk + kGatherWarps - 1) / kGatherWarps;
+    if (want_dist)
+      group_push_kernel<true><<<grid, kGatherThreads, 0, c->stream>>>(q->d_out.as<uint2>(), q->d_dist.as<float>(), loff, d_idx, nk,
+                                                                      r->d_goff.as<unsigned long long>(), r->d_out.as<uint2>(), r->d_dist.as<float>());
+    else
+      group_push_kernel<false><<<grid, kGatherThreads, 0, c->stream>>>(q->d_out.as<uint2>(), nullptr, loff, d_idx, nk,
+                                                                       r->d_goff.as<unsigned long long>(), r->d_out.as<uint2>(), nullptr);
+    FM_CUDA_G(cudaGetLastError());
+    FM_CUDA_G(cudaEventRecord(g->ev[k], c->stream));
+    give_buf_queued(c->out_free, q->d_out);
+    give_buf_queued(c->counts_free, q->d_counts);
+    give_buf_queued(c->dist_free, q->d_dist);
+  }
+  // 5. the lead waits for every push; total and counts to the result's pinned block, as fm_match leaves them
+  FM_CUDA_G(cudaSetDevice(lead->device));
+  for (const GroupPart& gp : r->parts)
+    if (gp.member) FM_CUDA_G(cudaStreamWaitEvent(lead->stream, g->ev[gp.member], 0));
+  FM_CUDA_G(cudaMemcpyAsync(static_cast<char*>(r->h_block) + offsetof(DeviceCounters, running_total), r->d_goff.as<unsigned long long>() + n_pairs,
+                            sizeof(unsigned long long), cudaMemcpyDeviceToHost, lead->stream));
+  if (n_pairs)
+    FM_CUDA_G(cudaMemcpyAsync(static_cast<char*>(r->h_block) + sizeof(DeviceCounters), r->d_counts.p, n_pairs * sizeof(uint32_t),
+                              cudaMemcpyDeviceToHost, lead->stream));
+  r->done = r->ev.get();
+  FM_CUDA_G(cudaEventRecord(r->done, lead->stream));
+#undef FM_CUDA_G
+  return FM_OK;
+}
+
+
 }  // namespace
 
 extern "C" {
@@ -1225,6 +1370,8 @@ int fm_group_match(fm_group* g, const uint32_t* pair_first, const uint32_t* pair
   if (G == 1) return fm_match(lead, pair_first, pair_second, n_pairs, dist, dist2second, flags, out);
   if (n_pairs && (!pair_first || !pair_second)) return fail(lead, FM_ERR_INVALID, "fm_match: null pair arrays");
   if (!(dist < 1.8e19f)) return fail(lead, FM_ERR_UNSUPPORTED, "fm_match: distance threshold must be below 1.8e19");
+  if ((flags & FM_FLAG_ROW_TABLE) && (flags & FM_FLAG_MATCH_ALL))
+    return fail(lead, FM_ERR_INVALID, "fm_match: FM_FLAG_ROW_TABLE does not combine with FM_FLAG_MATCH_ALL");
   for (size_t p = 0; p < n_pairs; p++) {  // (every member holds every image: the lead's table speaks for all)
     uint32_t a = pair_first[p], b = pair_second[p];
     if (a >= lead->images.size() || b >= lead->images.size() || !lead->images[a].valid || !lead->images[b].valid)
@@ -1245,7 +1392,6 @@ int fm_group_match(fm_group* g, const uint32_t* pair_first, const uint32_t* pair
   std::vector<double> weight(n_pairs);
   for (size_t p = 0; p < n_pairs; p++) weight[p] = (double)lead->images[pair_first[p]].n * (double)lead->images[pair_second[p]].n;
   const std::vector<std::vector<size_t>> shard = shard_pairs(weight, (int)G);
-  const bool want_dist = (flags & FM_FLAG_DISTANCES) && !(flags & FM_FLAG_MATCH_ALL);
 
   fm_result* r = new (std::nothrow) fm_result();
   if (!r) return fail(lead, FM_ERR_NOMEM, "fm_group_match: out of host memory");
@@ -1253,7 +1399,7 @@ int fm_group_match(fm_group* g, const uint32_t* pair_first, const uint32_t* pair
   r->n_pairs = n_pairs;
   r->flags = flags;
   r->ratio = dist2second;
-  std::vector<size_t> part_of(G, SIZE_MAX);  // member -> its entry in r->parts
+  r->group = g;
   auto bail = [&](int code) {
     for (auto* c : g->m) { cudaSetDevice(c->device); cudaStreamSynchronize(c->stream); }
     fm_result_free(r);
@@ -1280,96 +1426,223 @@ int fm_group_match(fm_group* g, const uint32_t* pair_first, const uint32_t* pair
       fm_result* q = nullptr;
       if (int rc = fm_match(g->m[k], pf.data(), ps.data(), pf.size(), dist, dist2second, flags | FM_FLAG_ASYNC | FM_FLAG_DEVICE_ONLY, &q))
         return bail(member_fail(g, k, rc));
-      part_of[k] = r->parts.size();
       r->parts.push_back(GroupPart{});
-      r->parts.back().sub = q;
+      GroupPart& gp = r->parts.back();
+      gp.sub = q;
+      gp.member = (uint32_t)k;
+      gp.idx.assign(shard[k].begin(), shard[k].end());
       r->slots += q->slots;
     }
   }
-  FM_CUDA_G(cudaSetDevice(lead->device));
-  r->d_out = take_buf(lead->out_free, std::max<uint64_t>(r->slots, 1) * sizeof(uint2));
-  r->d_counts = take_buf(lead->counts_free, std::max<size_t>(n_pairs, 1) * sizeof(uint32_t));
-  r->d_goff = take_buf(lead->counts_free, (n_pairs + 1) * sizeof(unsigned long long));
-  if (want_dist) r->d_dist = take_buf(lead->dist_free, std::max<uint64_t>(r->slots, 1) * sizeof(float));
-  FM_CUDA_G(r->d_out.ensure(std::max<uint64_t>(r->slots, 1) * sizeof(uint2)));
-  FM_CUDA_G(r->d_counts.ensure(std::max<size_t>(n_pairs, 1) * sizeof(uint32_t)));
-  FM_CUDA_G(r->d_goff.ensure((n_pairs + 1) * sizeof(unsigned long long)));
-  if (want_dist) FM_CUDA_G(r->d_dist.ensure(std::max<uint64_t>(r->slots, 1) * sizeof(float)));
-  FM_CUDA_G(take_pinned(lead, sizeof(DeviceCounters) + std::max<size_t>(n_pairs, 1) * sizeof(uint32_t), &r->h_block, &r->h_block_cap));
-  memset(r->h_block, 0, sizeof(DeviceCounters));
-
-  // 2. each member's counts to their submission positions on the lead; its local offsets
-  for (size_t k = 0; k < G; k++) {
-    if (part_of[k] == SIZE_MAX) continue;
-    GroupPart& gp = r->parts[part_of[k]];
-    fm_ctx* c = g->m[k];
-    const uint32_t nk = (uint32_t)shard[k].size();
-    FM_CUDA_G(cudaSetDevice(c->device));
-    FM_CUDA_G(take_pinned(c, (size_t)nk * sizeof(uint32_t), &gp.pin, &gp.pin_cap));
-    uint32_t* h_idx = static_cast<uint32_t*>(gp.pin);
-    for (uint32_t i = 0; i < nk; i++) h_idx[i] = (uint32_t)shard[k][i];
-    const size_t loff_bytes = ((size_t)nk + 1) * sizeof(unsigned long long);
-    gp.scratch = take_buf(c->counts_free, loff_bytes + (size_t)nk * sizeof(uint32_t));
-    FM_CUDA_G(gp.scratch.ensure(loff_bytes + (size_t)nk * sizeof(uint32_t)));
-    unsigned long long* loff = gp.scratch.as<unsigned long long>();
-    uint32_t* d_idx = reinterpret_cast<uint32_t*>(loff + nk + 1);
-    FM_CUDA_G(cudaMemcpyAsync(d_idx, h_idx, (size_t)nk * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
-    if (k) FM_CUDA_G(cudaStreamWaitEvent(c->stream, g->ev_lead, 0));
-    const uint32_t* counts = gp.sub->d_counts.as<uint32_t>();
-    group_counts_kernel<<<(nk + 255) / 256, 256, 0, c->stream>>>(counts, d_idx, nk, r->d_counts.as<uint32_t>());
-    links_scan_kernel<<<1, 1024, 0, c->stream>>>(counts, nk, loff);
-    FM_CUDA_G(cudaGetLastError());
-    FM_CUDA_G(cudaEventRecord(g->ev[k], c->stream));
-  }
-  // 3. the lead scans the gathered counts into submission-order offsets
-  FM_CUDA_G(cudaSetDevice(lead->device));
-  for (size_t k = 1; k < G; k++)
-    if (part_of[k] != SIZE_MAX) FM_CUDA_G(cudaStreamWaitEvent(lead->stream, g->ev[k], 0));
-  links_scan_kernel<<<1, 1024, 0, lead->stream>>>(r->d_counts.as<uint32_t>(), (uint32_t)n_pairs, r->d_goff.as<unsigned long long>());
-  FM_CUDA_G(cudaGetLastError());
-  FM_CUDA_G(cudaEventRecord(g->ev_lead, lead->stream));
-  // 4. each member pushes its lists into the lead's buffer; its own buffers go back to its free lists when they have
-  // room (stream order keeps them until the push has read them), else at fm_result_free
-  for (size_t k = 0; k < G; k++) {
-    if (part_of[k] == SIZE_MAX) continue;
-    GroupPart& gp = r->parts[part_of[k]];
-    fm_ctx* c = g->m[k];
-    fm_result* q = gp.sub;
-    const uint32_t nk = (uint32_t)shard[k].size();
-    FM_CUDA_G(cudaSetDevice(c->device));
-    if (k) FM_CUDA_G(cudaStreamWaitEvent(c->stream, g->ev_lead, 0));
-    const unsigned long long* loff = gp.scratch.as<unsigned long long>();
-    const uint32_t* d_idx = reinterpret_cast<const uint32_t*>(loff + nk + 1);
-    const unsigned grid = (nk + kGatherWarps - 1) / kGatherWarps;
-    if (want_dist)
-      group_push_kernel<true><<<grid, kGatherThreads, 0, c->stream>>>(q->d_out.as<uint2>(), q->d_dist.as<float>(), loff, d_idx, nk,
-                                                                      r->d_goff.as<unsigned long long>(), r->d_out.as<uint2>(), r->d_dist.as<float>());
-    else
-      group_push_kernel<false><<<grid, kGatherThreads, 0, c->stream>>>(q->d_out.as<uint2>(), nullptr, loff, d_idx, nk,
-                                                                       r->d_goff.as<unsigned long long>(), r->d_out.as<uint2>(), nullptr);
-    FM_CUDA_G(cudaGetLastError());
-    FM_CUDA_G(cudaEventRecord(g->ev[k], c->stream));
-    give_buf_queued(c->out_free, q->d_out);
-    give_buf_queued(c->counts_free, q->d_counts);
-    give_buf_queued(c->dist_free, q->d_dist);
-  }
-  // 5. the lead waits for every push; total and counts to the result's pinned block, as fm_match leaves them
-  FM_CUDA_G(cudaSetDevice(lead->device));
-  for (size_t k = 1; k < G; k++)
-    if (part_of[k] != SIZE_MAX) FM_CUDA_G(cudaStreamWaitEvent(lead->stream, g->ev[k], 0));
-  FM_CUDA_G(cudaMemcpyAsync(static_cast<char*>(r->h_block) + offsetof(DeviceCounters, running_total), r->d_goff.as<unsigned long long>() + n_pairs,
-                            sizeof(unsigned long long), cudaMemcpyDeviceToHost, lead->stream));
-  if (n_pairs)
-    FM_CUDA_G(cudaMemcpyAsync(static_cast<char*>(r->h_block) + sizeof(DeviceCounters), r->d_counts.p, n_pairs * sizeof(uint32_t),
-                              cudaMemcpyDeviceToHost, lead->stream));
-  r->done = r->ev.get();
-  FM_CUDA_G(cudaEventRecord(r->done, lead->stream));
 #undef FM_CUDA_G
+  if (flags & FM_FLAG_ROW_TABLE) {
+    // rows in submission order over the whole call, and where each pair's rows lie (fm_result_rows_copy)
+    r->table = true;
+    r->row_off.assign(n_pairs + 1, 0);
+    for (size_t p = 0; p < n_pairs; p++)
+      r->row_off[p + 1] = r->row_off[p] + lead->images[pair_second[p]].n + ((flags & FM_FLAG_SYM) ? lead->images[pair_first[p]].n : 0u);
+    r->pair_part.assign(n_pairs, 0);
+    r->pair_local.assign(n_pairs, 0);
+    for (size_t i = 0; i < r->parts.size(); i++)
+      for (size_t j = 0; j < r->parts[i].idx.size(); j++) {
+        r->pair_part[r->parts[i].idx[j]] = (uint32_t)i;
+        r->pair_local[r->parts[i].idx[j]] = (uint32_t)j;
+      }
+  }
+  if (int rc = group_gather(g, r)) return bail(rc);
   if (!(flags & FM_FLAG_ASYNC)) {
     int rc = fm_result_wait(r);
     if (rc != FM_OK) { fm_result_free(r); return rc; }
   }
   *out = r;
+  return FM_OK;
+}
+
+// ---- re-deciding a call at other thresholds (FM_FLAG_ROW_TABLE, fm_select.cuh) ---------------------------------------
+
+}  // extern "C"
+
+namespace {
+
+// fm_result_select on a result of one context: per batch of the source call, select_kernel turns the table's rows into
+// rowres / rowdist at (dist, ratio), and compact_launch compacts them with the call's own chunk records -- the
+// fm_match tail, with the scoring replaced by one read of the table.
+int select_one(const fm_result* s, float dist, float ratio, uint32_t flags, fm_result** out) {
+  fm_ctx* c = s->ctx;
+  FM_CUDA(c, cudaSetDevice(c->device));
+  const bool want_dist = (flags & FM_FLAG_DISTANCES) != 0;
+  const uint64_t total_rows = s->slots;
+  fm_result* r = new (std::nothrow) fm_result();
+  if (!r) return fail(c, FM_ERR_NOMEM, "fm_result_select: out of host memory");
+  r->ctx = c;
+  r->n_pairs = s->n_pairs;
+  r->flags = flags;
+  r->ratio = ratio;
+  r->slots = total_rows;
+  r->d_out = take_buf(c->out_free, std::max<uint64_t>(total_rows, 1) * sizeof(uint2));
+  r->d_counts = take_buf(c->counts_free, std::max<size_t>(r->n_pairs, 1) * sizeof(uint32_t));
+  if (want_dist) r->d_dist = take_buf(c->dist_free, std::max<uint64_t>(total_rows, 1) * sizeof(float));
+#define FM_CUDA_R(expr)                       \
+  do {                                        \
+    cudaError_t e__ = (expr);                 \
+    if (e__ != cudaSuccess) {                 \
+      int code__ = cuda_fail(c, e__, #expr);  \
+      fm_result_free(r);                      \
+      return code__;                          \
+    }                                         \
+  } while (0)
+  if (c->ev_match.pool.empty() && !c->ev_free.empty()) {
+    c->ev_match = std::move(c->ev_free.back());
+    c->ev_free.pop_back();
+  }
+  c->ev_match.reset();
+  const float ms_prep = c->stats.ms_prep;
+  c->stats = fm_stats{};
+  c->stats.ms_prep = ms_prep;
+  c->stats.rows = total_rows;
+
+  // the chunk records, staged in the result's pinned block behind the counters and counts (as fm_match stages its blob)
+  const size_t off_blob = (sizeof(DeviceCounters) + std::max<size_t>(r->n_pairs, 1) * sizeof(uint32_t) + 15) & ~(size_t)15;
+  const size_t blob_bytes = std::max<size_t>(s->sel_chunks.size() * sizeof(ChunkDesc), 16);
+  FM_CUDA_R(take_pinned(c, off_blob + blob_bytes, &r->h_block, &r->h_block_cap));
+  unsigned char* blob = static_cast<unsigned char*>(r->h_block) + off_blob;
+  if (!s->sel_chunks.empty()) memcpy(blob, s->sel_chunks.data(), s->sel_chunks.size() * sizeof(ChunkDesc));
+  FM_CUDA_R(c->d_meta_blob.ensure(blob_bytes));
+  FM_CUDA_R(cudaMemcpyAsync(c->d_meta_blob.p, blob, blob_bytes, cudaMemcpyHostToDevice, c->stream));
+  const ChunkDesc* d_chunk = c->d_meta_blob.as<ChunkDesc>();
+
+  uint32_t max_rows = 1, max_chunks = 1;
+  for (auto& b : s->sel_batches) { max_rows = std::max(max_rows, b.rows); max_chunks = std::max(max_chunks, b.chunks); }
+  FM_CUDA_R(c->d_rowres.ensure((size_t)max_rows * sizeof(uint32_t)));
+  if (want_dist) {
+    FM_CUDA_R(c->d_rowdist.ensure((size_t)max_rows * sizeof(float)));
+    FM_CUDA_R(r->d_dist.ensure(std::max<uint64_t>(total_rows, 1) * sizeof(float)));
+  }
+  FM_CUDA_R(c->d_chunk_count.ensure((size_t)max_chunks * sizeof(uint32_t)));
+  FM_CUDA_R(c->d_chunk_out.ensure((size_t)max_chunks * sizeof(unsigned long long)));
+  FM_CUDA_R(c->d_chunk_stage.ensure((size_t)max_chunks * kStageCap * sizeof(uint2)));
+  FM_CUDA_R(ensure_chunk_status(c));
+  FM_CUDA_R(c->d_totals.ensure(sizeof(DeviceCounters)));
+  FM_CUDA_R(r->d_out.ensure(std::max<uint64_t>(total_rows, 1) * sizeof(uint2)));
+  FM_CUDA_R(r->d_counts.ensure(std::max<size_t>(r->n_pairs, 1) * sizeof(uint32_t)));
+  FM_CUDA_R(cudaMemsetAsync(r->d_counts.p, 0, std::max<size_t>(r->n_pairs, 1) * sizeof(uint32_t), c->stream));
+  FM_CUDA_R(cudaMemsetAsync(c->d_totals.p, 0, sizeof(DeviceCounters), c->stream));
+
+  uint32_t* d_rowres = c->d_rowres.as<uint32_t>();
+  float* d_rowdist = want_dist ? c->d_rowdist.as<float>() : nullptr;
+  DeviceCounters* d_counters = c->d_totals.as<DeviceCounters>();
+  {
+    Span total_span(&c->ev_match, c->stream, kPhTotal);
+    for (const SelectBatch& b : s->sel_batches) {
+      if (b.rows == 0) continue;
+      {
+        Span sp(&c->ev_match, c->stream, kPhRescore);
+        const uint32_t grid = std::min<uint32_t>((b.rows + kSelectThreads - 1) / kSelectThreads, (uint32_t)c->sm_count * 16u);
+        select_kernel<<<grid, kSelectThreads, 0, c->stream>>>(s->d_table.as<fm_row>() + b.row0, b.rows, dist, ratio, d_rowres,
+                                                              d_rowdist);
+        c->stats.kernel_launches++;
+      }
+      {
+        Span sp(&c->ev_match, c->stream, kPhCompact);
+        CompactArgs ca{};
+        ca.chunks = d_chunk + b.chunk0;
+        ca.n_chunks = b.chunks;
+        ca.rowres = d_rowres;
+        ca.rowdist = d_rowdist;
+        ca.pair_count = r->d_counts.as<uint32_t>();
+        ca.running_total = &d_counters->running_total;
+        ca.out_pairs = r->d_out.as<uint2>();
+        ca.out_dist = want_dist ? r->d_dist.as<float>() : nullptr;
+        c->stats.kernel_launches += compact_launch(c, ca, want_dist, FM_COMPACT_AUTO);
+      }
+    }
+  }
+  FM_CUDA_R(cudaGetLastError());
+  FM_CUDA_R(queue_tail(c, r));
+#undef FM_CUDA_R
+  if (!(flags & FM_FLAG_ASYNC)) {
+    int rc = fm_result_wait(r);
+    if (rc != FM_OK) { fm_result_free(r); return rc; }
+  }
+  *out = r;
+  return FM_OK;
+}
+
+// fm_result_select on a group result: each member selects on its part of the call, and the lists are gathered on the
+// lead exactly as fm_group_match gathers them.
+int select_group(const fm_result* s, float dist, float ratio, uint32_t flags, fm_result** out) {
+  fm_group* g = s->group;
+  fm_ctx* lead = g->m[0];
+  fm_result* r = new (std::nothrow) fm_result();
+  if (!r) return fail(lead, FM_ERR_NOMEM, "fm_result_select: out of host memory");
+  r->ctx = lead;
+  r->n_pairs = s->n_pairs;
+  r->flags = flags;
+  r->ratio = ratio;
+  r->group = g;
+  auto bail = [&](int code) {
+    for (auto* c : g->m) { cudaSetDevice(c->device); cudaStreamSynchronize(c->stream); }
+    fm_result_free(r);
+    return code;
+  };
+  // members store into lead buffers only behind this event (see fm_group_match)
+  cudaError_t e = cudaSetDevice(lead->device);
+  if (e == cudaSuccess) e = cudaEventRecord(g->ev_lead, lead->stream);
+  if (e != cudaSuccess) return bail(cuda_fail(lead, e, "fm_result_select"));
+  for (const GroupPart& sp : s->parts) {
+    fm_result* q = nullptr;
+    if (int rc = select_one(sp.sub, dist, ratio, (flags & FM_FLAG_DISTANCES) | FM_FLAG_ASYNC | FM_FLAG_DEVICE_ONLY, &q))
+      return bail(member_fail(g, sp.member, rc));
+    r->parts.push_back(GroupPart{});
+    GroupPart& gp = r->parts.back();
+    gp.sub = q;
+    gp.member = sp.member;
+    gp.idx = sp.idx;
+    r->slots += q->slots;
+  }
+  if (int rc = group_gather(g, r)) return bail(rc);
+  if (!(flags & FM_FLAG_ASYNC)) {
+    int rc = fm_result_wait(r);
+    if (rc != FM_OK) { fm_result_free(r); return rc; }
+  }
+  *out = r;
+  return FM_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int fm_result_select(const fm_result* r, float dist, float dist2second, uint32_t flags, fm_result** out) {
+  if (!r || !out) return FM_ERR_INVALID;
+  *out = nullptr;
+  fm_ctx* c = r->ctx;
+  if (flags & ~(FM_FLAG_DISTANCES | FM_FLAG_DEVICE_ONLY | FM_FLAG_ASYNC))
+    return fail(c, FM_ERR_INVALID, "fm_result_select: flags other than FM_FLAG_DISTANCES, FM_FLAG_DEVICE_ONLY and FM_FLAG_ASYNC");
+  if (!r->table) return fail(c, FM_ERR_INVALID, "fm_result_select: the result has no row table (FM_FLAG_ROW_TABLE)");
+  if (dist != dist || dist2second != dist2second) return fail(c, FM_ERR_INVALID, "fm_result_select: NaN threshold");
+  if (!(dist < 1.8e19f)) return fail(c, FM_ERR_UNSUPPORTED, "fm_result_select: distance threshold must be below 1.8e19");
+  return r->group ? select_group(r, dist, dist2second, flags, out) : select_one(r, dist, dist2second, flags, out);
+}
+
+const fm_row* fm_result_rows_device(const fm_result* r) {
+  return (r && r->table && !r->group) ? r->d_table.as<fm_row>() : nullptr;
+}
+
+uint64_t fm_result_row_offset(const fm_result* r, size_t p) {
+  return (r && r->table && p <= r->n_pairs) ? r->row_off[p] : UINT64_MAX;
+}
+
+int fm_result_rows_copy(fm_result* r, size_t p, fm_row* dst) {
+  if (!r) return FM_ERR_INVALID;
+  if (!r->table || p >= r->n_pairs || !dst) return fail(r->ctx, FM_ERR_INVALID, "fm_result_rows_copy: no row table, bad pair or null dst");
+  const fm_result* t = r->group ? r->parts[r->pair_part[p]].sub : r;  // the result holding the pair's rows
+  const size_t q = r->group ? r->pair_local[p] : p;
+  fm_ctx* c = t->ctx;
+  const uint64_t n = t->row_off[q + 1] - t->row_off[q];
+  FM_CUDA(r->ctx, cudaSetDevice(c->device));
+  if (n) FM_CUDA(r->ctx, cudaMemcpyAsync(dst, t->d_table.as<fm_row>() + t->row_off[q], n * sizeof(fm_row), cudaMemcpyDeviceToHost, c->stream));
+  FM_CUDA(r->ctx, cudaStreamSynchronize(c->stream));
   return FM_OK;
 }
 

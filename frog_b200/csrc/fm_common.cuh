@@ -6,9 +6,17 @@
 #include <cstdint>
 #include <cstring>
 
+#include "../../include/frogmatch.h"
+
 namespace fm {
 
 constexpr uint32_t kNone = 0xFFFFFFFFu;  // "row has no accepted match"
+
+// FM_FLAG_ROW_TABLE: a decision site's record of one row (fm_row, include/frogmatch.h).  d1 < FLT_MAX iff a gated-in
+// column set it, and only then does `nearest` name a column.
+__device__ __forceinline__ void put_row(fm_row* rows, uint32_t i, float d1, float d2, uint32_t nearest) {
+  rows[i] = fm_row{d1, d2, d1 < FLT_MAX ? nearest : kNone};
+}
 constexpr uint32_t kTaskSwap = 1u;       // Task::flags: -sym reverse pass (match.cpp:643-646)
 constexpr uint32_t kTaskExact = 2u;      // Task::flags: task must use the exact brute-force kernel
 constexpr int kD = 48;                   // SURF3D descriptor length the tensor-core path is built for

@@ -66,11 +66,13 @@ __device__ __forceinline__ uint32_t find_segment_near(const uint32_t* __restrict
 
 // D_T: descriptor length, known at compile time; the row's descriptor lives in registers.
 // require_flags: only tasks whose flags contain these bits are processed (0 = every task).
+// rows: FM_FLAG_ROW_TABLE only (else null), the batch's records, indexed like rowres.
 template <int D_T>
 __global__ void __launch_bounds__(kExactRows)
 exact_match_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ tasks,
                    const uint32_t* __restrict__ task_blk_off, uint32_t n_tasks, float thr, float ratio,
-                   uint32_t require_flags, uint32_t* __restrict__ rowres, float* __restrict__ rowdist) {
+                   uint32_t require_flags, uint32_t* __restrict__ rowres, float* __restrict__ rowdist,
+                   fm_row* __restrict__ rows) {
   extern __shared__ float smem[];
   const uint32_t t = find_segment(task_blk_off, n_tasks, blockIdx.x);
   const Task task = tasks[t];
@@ -132,6 +134,7 @@ exact_match_kernel(const ImageDev* __restrict__ images, const Task* __restrict__
   if (active) {
     rowres[task.row_off + row] = accept_rule(d1, d2, thr, ratio) ? match : kNone;
     if (rowdist) rowdist[task.row_off + row] = d1;  // FM_FLAG_DISTANCES: the reference's norm() of the emitted pair
+    if (rows) put_row(rows, task.row_off + row, d1, d2, match);
   }
 }
 

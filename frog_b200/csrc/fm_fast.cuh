@@ -145,6 +145,7 @@ struct FastBatchArgs {
   float thr, ratio;
   uint32_t* rowres;
   float* rowdist;  // null unless FM_FLAG_DISTANCES
+  fm_row* table;   // null unless FM_FLAG_ROW_TABLE: the batch's records (then two_phase is false)
   bool two_phase;  // reject pass + capture pass instead of the single pass (see score_kernel)
   DeviceCounters* counters;
 };
@@ -268,9 +269,9 @@ inline cudaError_t fast_match_batch(fm_ctx* c, const FastBatchArgs& a) {
     rescore_kernel<<<a.blocks128, 128, 0, c->stream>>>(a.images, a.tasks, a.blk_off, a.n_tasks, a.segs,
                                                        c->d_cands.as<Cand>(), a.thr, a.ratio, a.rowres,
                                                        c->d_redo.as<uint2>(), &a.counters->rescore, a.rowdist,
-                                                       two_phase_ran ? c->d_rowstat.as<uint8_t>() : nullptr);
+                                                       two_phase_ran ? c->d_rowstat.as<uint8_t>() : nullptr, a.table);
     exact_rows_kernel<<<c->sm_count, kRedoThreads, 0, c->stream>>>(a.images, a.tasks, c->d_bands.as<uint2>(), c->d_redo.as<uint2>(),
-                                                             &a.counters->rescore, a.thr, a.ratio, a.rowres, a.rowdist);
+                                                             &a.counters->rescore, a.thr, a.ratio, a.rowres, a.rowdist, a.table);
     fold_redo_kernel<<<1, 1, 0, c->stream>>>(a.counters);
   }
   c->stats.kernel_launches += 5;

@@ -27,7 +27,8 @@ struct GenSmem {
   float scale[kGenCols], lap[kGenCols];
 };
 
-// kMode 0: nearest / second-nearest + acceptance -> rowres (match.cpp:303-330).
+// kMode 0: nearest / second-nearest + acceptance -> rowres (match.cpp:303-330), and the row's record -> rows
+// (FM_FLAG_ROW_TABLE; null otherwise).
 // kMode 1: -all count pass -> row_count / row_final.   kMode 2: -all emit pass (see fm_all.cuh).
 template <int kMode>
 __global__ void __launch_bounds__(kExactRows)
@@ -36,7 +37,7 @@ exact_generic_kernel(const ImageDev* __restrict__ images, const Task* __restrict
                      uint32_t require_flags, uint32_t* __restrict__ rowres, uint32_t* __restrict__ row_count,
                      uint32_t* __restrict__ row_final, const uint32_t* __restrict__ row_carry,
                      const unsigned long long* __restrict__ row_off, const unsigned long long* __restrict__ task_base,
-                     uint2* __restrict__ out, float* __restrict__ rowdist) {
+                     uint2* __restrict__ out, float* __restrict__ rowdist, fm_row* __restrict__ rows) {
   __shared__ GenSmem sm;
   const uint32_t t = find_segment(task_blk_off, n_tasks, blockIdx.x);
   const Task task = tasks[t];
@@ -113,6 +114,7 @@ exact_generic_kernel(const ImageDev* __restrict__ images, const Task* __restrict
   if (kMode == 0) {
     rowres[task.row_off + row] = accept_rule(d1, d2, thr, ratio) ? match : kNone;
     if (rowdist) rowdist[task.row_off + row] = d1;
+    if (rows) put_row(rows, task.row_off + row, d1, d2, match);
   }
   if (kMode == 1) {
     row_count[task.row_off + row] = count;

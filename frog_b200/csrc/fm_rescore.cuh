@@ -59,7 +59,7 @@ rescore_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ tas
                const uint32_t* __restrict__ task_blk_off, uint32_t n_tasks, uint32_t segs,
                const Cand* __restrict__ cands, float thr, float ratio, uint32_t* __restrict__ rowres,
                uint2* __restrict__ redo_list, RescoreCounters* __restrict__ counters, float* __restrict__ rowdist,
-               const uint8_t* __restrict__ rowstat) {
+               const uint8_t* __restrict__ rowstat, fm_row* __restrict__ rows) {
   const uint32_t t = find_segment_near(task_blk_off, n_tasks, blockIdx.x, gridDim.x);
   const Task task = tasks[t];
   if (task.flags & kTaskExact) return;
@@ -104,11 +104,15 @@ rescore_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ tas
   // Early rejection, certified (certified_reject, fm_score.cuh): the lists hold the row's two best approximate scores
   // a1 >= a2, and when the reference's ratio or threshold test must fail for them the row emits nothing and no exact
   // distance has to be gathered: with -d2 0.8 on unrelated images that is almost every row.
+  // A row table (rows != null, never with the two-phase path) records every row's exact (d1, d2): no row is rejected
+  // here.
   bool rejected = pre_rejected;
-  if (!pre_rejected && !overflow && a1 > -INFINITY) rejected = certified_reject(B.norm2_sorted[s], a1, a2, eps, thr, ratio);
+  if (!pre_rejected && !overflow && a1 > -INFINITY && !rows) rejected = certified_reject(B.norm2_sorted[s], a1, a2, eps, thr, ratio);
 
   uint32_t match = kNone;
   uint32_t n_eval = 0;
+  float d1 = FLT_MAX, d2 = FLT_MAX;
+  uint32_t best = 0;
   if (!overflow && !rejected && a1 > -INFINITY) {
     float r[kD];
     const float4* src = reinterpret_cast<const float4*>(B.desc + (size_t)row * kD);
@@ -117,8 +121,6 @@ rescore_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ tas
       float4 v = __ldg(src + q);
       r[4 * q] = v.x; r[4 * q + 1] = v.y; r[4 * q + 2] = v.z; r[4 * q + 3] = v.w;
     }
-    float d1 = FLT_MAX, d2 = FLT_MAX;
-    uint32_t best = 0;
     for (uint32_t e = 0; e < L; e++) {
       const Cand cd = c[e];
       if (!(cd.t > -INFINITY) || !(cd.t >= band)) continue;
@@ -135,6 +137,7 @@ rescore_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ tas
     if (rowdist) rowdist[task.row_off + row] = d1;
   }
   if (!pre_rejected) rowres[task.row_off + row] = match;
+  if (rows && !overflow) put_row(rows, task.row_off + row, d1, d2, best);  // (an overflowing row: exact_rows_kernel)
   if (overflow) {
     unsigned long long slot = atomicAdd(&counters->redo_rows, 1ull);
     redo_list[slot] = make_uint2(t, s);
@@ -163,7 +166,7 @@ __global__ void __launch_bounds__(kRedoThreads)
 exact_rows_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ tasks,
                   const uint2* __restrict__ bands, const uint2* __restrict__ redo_list,
                   const RescoreCounters* __restrict__ counters, float thr, float ratio,
-                  uint32_t* __restrict__ rowres, float* __restrict__ rowdist) {
+                  uint32_t* __restrict__ rowres, float* __restrict__ rowdist, fm_row* __restrict__ rows) {
   __shared__ float s_d1[kRedoThreads / 32], s_d2[kRedoThreads / 32];
   __shared__ uint32_t s_m[kRedoThreads / 32];
   const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -205,6 +208,7 @@ exact_rows_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ 
       for (int k = 1; k < kRedoThreads / 32; k++) top2_merge_sets(s_d1[k], s_d2[k], s_m[k], d1, d2, match);
       rowres[task.row_off + row] = accept_rule(d1, d2, thr, ratio) ? match : kNone;
       if (rowdist) rowdist[task.row_off + row] = d1;
+      if (rows) put_row(rows, task.row_off + row, d1, d2, match);
     }
     __syncthreads();
   }

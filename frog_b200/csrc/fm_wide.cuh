@@ -407,7 +407,7 @@ __global__ void __launch_bounds__(kWdRescoreThreads)
 wide_rescore_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ tasks,
                     const uint32_t* __restrict__ task_blk_off, uint32_t n_tasks, const Cand* __restrict__ cands, float thr,
                     float ratio, uint32_t* __restrict__ rowres, uint2* __restrict__ redo_list,
-                    RescoreCounters* __restrict__ counters, float* __restrict__ rowdist) {
+                    RescoreCounters* __restrict__ counters, float* __restrict__ rowdist, fm_row* __restrict__ rows) {
   const uint32_t t = find_segment_near(task_blk_off, n_tasks, blockIdx.x, gridDim.x);
   const Task task = tasks[t];
   if (task.flags & kTaskExact) return;  // CTA-uniform
@@ -436,8 +436,8 @@ wide_rescore_kernel(const ImageDev* __restrict__ images, const Task* __restrict_
     for (int k = 1; k < kTopK; k++) lowest = fminf(lowest, c[k].t);
     if (lowest >= band) overflow = true;
   }
-  bool rejected = false;
-  if (active && !overflow && a1 > -INFINITY) rejected = wide_certified_reject(B.norm2_sorted[s], a1, a2, eps, thr, ratio, d);
+  bool rejected = false;  // (never with a row table, as in rescore_kernel)
+  if (active && !overflow && a1 > -INFINITY && !rows) rejected = wide_certified_reject(B.norm2_sorted[s], a1, a2, eps, thr, ratio, d);
   const bool eval = active && !overflow && !rejected && a1 > -INFINITY;
   const uint32_t row = active ? B.perm[s] : 0u;
   float d1 = FLT_MAX, d2 = FLT_MAX;
@@ -461,6 +461,7 @@ wide_rescore_kernel(const ImageDev* __restrict__ images, const Task* __restrict_
   if (active && e == 0) {
     rowres[task.row_off + row] = eval && accept_rule(d1, d2, thr, ratio) ? best : kNone;
     if (eval && rowdist) rowdist[task.row_off + row] = d1;
+    if (rows && !overflow) put_row(rows, task.row_off + row, d1, d2, best);
     if (overflow) redo_list[atomicAdd(&counters->redo_rows, 1ull)] = make_uint2(t, s);
   }
   // statistics: one atomic per warp
@@ -481,7 +482,7 @@ wide_rescore_kernel(const ImageDev* __restrict__ images, const Task* __restrict_
 __global__ void __launch_bounds__(kRedoThreads)
 wide_exact_rows_kernel(const ImageDev* __restrict__ images, const Task* __restrict__ tasks, const uint2* __restrict__ bands,
                        const uint2* __restrict__ redo_list, const RescoreCounters* __restrict__ counters, float thr,
-                       float ratio, uint32_t* __restrict__ rowres, float* __restrict__ rowdist) {
+                       float ratio, uint32_t* __restrict__ rowres, float* __restrict__ rowdist, fm_row* __restrict__ rows) {
   __shared__ __align__(16) float s_row[kWideMaxD];
   __shared__ float s_d1[kRedoThreads / 32], s_d2[kRedoThreads / 32];
   __shared__ uint32_t s_m[kRedoThreads / 32];
@@ -536,6 +537,7 @@ wide_exact_rows_kernel(const ImageDev* __restrict__ images, const Task* __restri
       for (int k = 1; k < kRedoThreads / 32; k++) top2_merge_sets(s_d1[k], s_d2[k], s_m[k], d1, d2, match);
       rowres[task.row_off + row] = accept_rule(d1, d2, thr, ratio) ? match : kNone;
       if (rowdist) rowdist[task.row_off + row] = d1;
+      if (rows) put_row(rows, task.row_off + row, d1, d2, match);
     }
     __syncthreads();
   }
@@ -568,10 +570,10 @@ inline cudaError_t wide_match_batch(fm_ctx* c, const FastBatchArgs& a) {
     Span sp(&c->ev_match, c->stream, kPhRescore);
     wide_rescore_kernel<<<a.blocks128, kWdRescoreThreads, 0, c->stream>>>(
         a.images, a.tasks, a.blk_off, a.n_tasks, c->d_cands.as<Cand>(), a.thr, a.ratio, a.rowres, c->d_redo.as<uint2>(),
-        &a.counters->rescore, a.rowdist);
+        &a.counters->rescore, a.rowdist, a.table);
     // two CTAs per SM: a queued row is a long dependent chain per column, so the latency hiding comes from residency
     wide_exact_rows_kernel<<<2 * c->sm_count, kRedoThreads, 0, c->stream>>>(a.images, a.tasks, c->d_bands.as<uint2>(), c->d_redo.as<uint2>(),
-                                                                        &a.counters->rescore, a.thr, a.ratio, a.rowres, a.rowdist);
+                                                                        &a.counters->rescore, a.thr, a.ratio, a.rowres, a.rowdist, a.table);
     fold_redo_kernel<<<1, 1, 0, c->stream>>>(a.counters);
   }
   c->stats.kernel_launches += 5;

@@ -53,6 +53,27 @@ typedef enum fm_status {
                                  * completes the result.  Several results may be in flight on one context.  (Images
                                  * uploaded since the previous fm_match are prepared first, and the call waits for
                                  * that; FM_FLAG_MATCH_ALL sizes its lists on the host and is synchronous.) */
+#define FM_FLAG_ROW_TABLE 64u   /* also keep, in device memory owned by the result, one fm_row per outer-loop row of the
+                                 * call (below), so that fm_result_select() can re-decide the call at other thresholds
+                                 * without scoring again.  The lists at the call's own thresholds are unchanged.  Costs
+                                 * 12 bytes of device memory per row -- sum of N_second (+ N_first with FM_FLAG_SYM)
+                                 * over the pairs: 200 images x 20 000 keypoints, all ordered pairs, is 3.98e8 rows =
+                                 * 4.8 GB -- and scoring time: no row may be rejected from its approximate scores alone,
+                                 * because that test takes the thresholds, so the call scores in one pass and evaluates
+                                 * the exact distances of every row with a gated-in column.  FM_ERR_NOMEM (context
+                                 * still usable) when the table does not fit; FM_ERR_INVALID with FM_FLAG_MATCH_ALL. */
+
+/* One row of a row table (FM_FLAG_ROW_TABLE): the three values ComputeMatches' accept test reads (match.cpp:262-321),
+ * none of which depends on -d or -d2.  d1 and d2 are the exact nearest and second-nearest squared distances over the
+ * gated-in columns (FLT_MAX where the reference leaves them at FLT_MAX); nearest is the original index of the nearest
+ * column (the lowest one on ties), 0xFFFFFFFF when no column got below FLT_MAX -- in particular when none passes the
+ * gates.  The row is accepted at (dist, dist2second) iff
+ *   nearest != 0xFFFFFFFF && (sqrtf(d1 / d2) < dist2second || d2 == FLT_MAX) && sqrtf(d1) < dist. */
+typedef struct fm_row {
+  float d1;
+  float d2;
+  uint32_t nearest;
+} fm_row;
 
 /* ---- context --------------------------------------------------------------------------------- */
 
@@ -132,7 +153,34 @@ int fm_result_fetch(fm_result* r);
  * prefix sum of counts. */
 const uint32_t* fm_result_device_counts(const fm_result* r);
 const uint32_t* fm_result_device_pairs(const fm_result* r);
+/* Free a result.  A result with a row table waits for the work queued on its context's stream (fm_result_select calls
+ * on it included) before it releases the table. */
 void fm_result_free(fm_result* r);
+
+/* ---- re-deciding a call at other thresholds (FM_FLAG_ROW_TABLE) ---------------------------------------------------- */
+
+/*
+ * A new, independent result holding exactly the lists (and, with FM_FLAG_DISTANCES, distances) fm_match would return
+ * at (dist, dist2second) for the pairs and -sym choice of the call that produced `r`, in the same submission order --
+ * computed from r's row table (one pass over the table, then the same compaction fm_match runs), without scoring.
+ * `r` must hold a row table: a result of fm_match or fm_group_match with FM_FLAG_ROW_TABLE.  flags: any of
+ * FM_FLAG_DISTANCES, FM_FLAG_DEVICE_ONLY and FM_FLAG_ASYNC, with fm_match's meaning.  The work is queued on r's
+ * context stream(s) behind r's own work; r may be freed as soon as this returns.  The new result has no row table;
+ * fm_result_stats and fm_links_build (with the pair arrays of r's call) take it.  FM_ERR_INVALID for other flags, a
+ * result without a table or NaN thresholds; FM_ERR_UNSUPPORTED for dist >= 1.8e19, as fm_match.
+ */
+int fm_result_select(const fm_result* r, float dist, float dist2second, uint32_t flags, fm_result** out);
+/* The row table of r on its device: pair p's rows start at fm_result_row_offset(r, p) -- N_second rows in the original
+ * keypoint order of image `second`, then, with FM_FLAG_SYM, the reverse direction's N_first rows.  Valid in stream order
+ * (synchronise, or wait for the result, before reading it from another stream).  NULL without a table, and for a result
+ * of a group of several devices, whose table is split over the members (fm_result_rows_copy reads it). */
+const fm_row* fm_result_rows_device(const fm_result* r);
+/* First row of pair p in the table, in submission order over the whole call (also for group results); p == n_pairs gives
+ * the number of rows.  UINT64_MAX without a table or for p > n_pairs. */
+uint64_t fm_result_row_offset(const fm_result* r, size_t p);
+/* Copy pair p's rows (fm_result_row_offset(r, p + 1) - fm_result_row_offset(r, p) of them) to host memory `dst`; waits
+ * for the work that writes them. */
+int fm_result_rows_copy(fm_result* r, size_t p, fm_row* dst);
 
 /* ---- consumer hand-off ------------------------------------------------------------------------ */
 
@@ -230,7 +278,9 @@ int fm_group_upload_image(fm_group* g, uint32_t img, const float* desc, const fl
  * FM_FLAG_ASYNC, so a group never probes the first batch of a synchronous call to switch to two-phase scoring within
  * that call (see fm_match): the first call at dist2second < 1 runs single-pass where one context might not, and later
  * calls use each member's rejection rate of its previous call.  Results are exact either way.  The -all row limit
- * applies to the whole call, as for one context. */
+ * applies to the whole call, as for one context.  With FM_FLAG_ROW_TABLE each member keeps the table of its share;
+ * fm_result_select on the result selects on every member and gathers the lists on the lead the same way, and
+ * fm_result_row_offset / fm_result_rows_copy address the rows in submission order over the whole call. */
 int fm_group_match(fm_group* g, const uint32_t* pair_first, const uint32_t* pair_second, size_t n_pairs, float dist,
                    float dist2second, uint32_t flags, fm_result** out);
 
